@@ -2,11 +2,15 @@
 """Benchmark of the NGCF embedding-propagation hot path (BASELINE.json metric:
 "NGCF epoch time (fwd+bwd+BPR) at Gowalla shape; propagation SpMM HBM GB/s vs peak").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape gowalla]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape gowalla] [--dump-outputs DIR]
 
 A step is one reference training step (experiment.py:45-57): NGCF.forward over the full graph for one
 1024-triple batch with node_flag=True in training mode, BPR loss, backward to every parameter gradient
 (the optimizer step is not part of the metric).  One JSON line is printed by rank 0.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path returned in its last step (the loss and every
+parameter gradient) as DIR/<name>.npy.  Inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -45,7 +49,14 @@ def parse_args():
     ap.add_argument("--eager", action="store_true", help="time the eager drop-in path only (no CUDA graph)")
     ap.add_argument("--breakdown", action="store_true", help="print a per-entry-point time table to stderr")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra legs (other named shapes at the same N)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and parameter gradients of the last timed step as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 def log(*a):
@@ -99,6 +110,24 @@ def make_model(info, L, device, rng="device"):
     m = pkg.NGCF(info["emb"], [info["emb"]] * K, NODE_P, [MESS_P] * K, 1.0, [L, L],
                  synth.num_dict_for(info["n_user"], info["n_item"]), BATCH, device, rng=rng)
     return m
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, model):
+    """Writes what a caller of the timed step holds after it: the loss (float64) as loss.npy and every parameter
+    gradient (float32) as grad.<parameter>.npy.  Past DUMP_BYTES in all, each gradient keeps a fixed, seeded sample of
+    its rows: the same rows on every run of the same shape."""
+    grads = {k: p.grad.detach() for k, p in model.named_parameters() if p.grad is not None}
+    frac = min(1.0, DUMP_BYTES / (4 * sum(g.numel() for g in grads.values())))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([float(loss.detach())], dtype=np.float64))
+    for k, g in grads.items():
+        if frac < 1.0 and g.shape[0] > 1:
+            rows = np.sort(np.random.default_rng(0).choice(g.shape[0], max(1, int(g.shape[0] * frac)), replace=False))
+            g = g[torch.from_numpy(rows).to(g.device)]
+        np.save(os.path.join(out_dir, f"grad.{k}.npy"), g.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -333,18 +362,21 @@ def run_ours(args):
     sampler.start()
     windows = []
 
-    def timed_resident(fn):
-        """K steps on device-resident batches, per-step CUDA events, L2 flushed between steps; max over ranks."""
+    def timed_resident(fn, dump=False):
+        """K steps on device-resident batches, per-step CUDA events, L2 flushed between steps; max over ranks.  With
+        ``dump``, rank 0 writes the last step's outputs to --dump-outputs afterwards."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
         fence()
         w0 = time.time()
         for j in range(args.steps):
             flush.zero_()
             ev[j][0].record()
-            fn(dbatches[j % len(dbatches)])
+            loss = fn(dbatches[j % len(dbatches)])
             ev[j][1].record()
         fence()
         windows.append((w0, time.time()))
+        if dump and args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, loss, model)
         return max_over_ranks(sum(a.elapsed_time(b) for a, b in ev)) / args.steps
 
     def timed_e2e(fn, to_dev):
@@ -369,7 +401,7 @@ def run_ours(args):
     # ---- the eager drop-in path first (before any graph capture touches the allocator) ---------------------------
     h2d = sum(v.numel() * v.element_size() for k, v in hbatches[0].items() if k != "year")
     launches0 = lib.ngcf_launch_count()
-    ms_eager = timed_resident(step)
+    ms_eager = timed_resident(step, dump=args.eager)
     launches_eager = (lib.ngcf_launch_count() - launches0) / args.steps
     ms_e2e_eager, loss_eager = timed_e2e(step, to_dev=True)
 
@@ -389,7 +421,8 @@ def run_ours(args):
     run = gstep if gstep is not None else step
 
     # ---- value: device-resident inputs ------------------------------------------------------------------------
-    ms_per_step = timed_resident(run) if gstep is not None else ms_eager
+    # (a failed capture times the eager step again here: its first timed window's outputs are gone by now)
+    ms_per_step = ms_eager if args.eager else timed_resident(run, dump=True)
     launches = gstep.launches_per_step if gstep is not None else launches_eager
 
     # ---- warm variant (no flush, back-to-back) — reported as context only -------------------------------------
@@ -533,7 +566,7 @@ def run_ours(args):
         # the exact-fp32 FFMA dense kernels and the row-per-warp SpMM) with the reference's CPU step beside it
         for shp in ("amazon-book", "yelp2018") + (("seoul",) if world == 1 else ()):
             try:
-                extra[shp] = time_shape(pkg, shp, dev, world, rank)
+                extra[shp] = time_shape(pkg, shp, dev, world, rank, steps=args.steps)
                 log(f"[bench] extra {shp}: {extra[shp]['ms_per_step']} ms/step")
             except Exception as e:
                 extra[shp] = {"error": f"{type(e).__name__}: {e}"}
@@ -622,7 +655,7 @@ def run_pl(args):
     n_user, n_item, n_edges, emb, K = synth.SHAPES[args.shape]
     N = n_user + n_item
     nd = synth.num_dict_for(n_user, n_item)
-    steps = min(args.steps, 10)
+    steps = args.steps
     warm = max(min(args.warmup, 3), 3)
 
     def fence():
@@ -702,12 +735,16 @@ def run_pl(args):
     db = [{k: (v if k == "year" else v.to(dev)) for k, v in b.items()} for b in hb]
     for j in range(steps):
         ev[j][0].record()
-        gstep(db[j % len(db)])
+        loss = gstep(db[j % len(db)])
         ev[j][1].record()
     fence()
+    windows = [(w0, time.time())]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model)
     ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in ev)) / steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     fence()
+    w0 = time.time()
     e0.record()
     last = 0.0
     for j in range(steps):
@@ -715,7 +752,7 @@ def run_pl(args):
     e1.record()
     fence()
     ms_e2e = max_over_ranks(e0.elapsed_time(e1)) / steps
-    windows = [(w0, time.time())]
+    windows.append((w0, time.time()))
     # roofline: layer 0's product on this rank's shard, exactly as the step runs it
     plan = model._last.plan
     r0 = model._shard.r0 if model._shard else 0
@@ -920,7 +957,7 @@ def time_cpu_reference(L, batches, info, max_steps, warmup, budget_s):
         torch.set_num_threads(cores)
         single = {"ms_per_step": round(s1 * 1e3, 2), "cores": 1, "sample": "mean of 2 steps"}
     return {"value": round(s * info["steps_per_epoch"], 3), "unit": "s/epoch", "ms_per_step": round(s * 1e3, 2),
-            "cores": cores, "kind": "reference", "single_thread": single,
+            "cores": cores, "kind": "reference", "steps": n, "single_thread": single,
             "sample": f"{n} full training steps (of {info['steps_per_epoch']} per epoch) of the same workload, {warmup} "
                       f"warm-up; the reference's unmodified NGCF.py / bprloss.py (baseline/_ref) on device='cpu': "
                       f"torch.sparse COO mm + host float64 node-dropout mask + autograd"}
@@ -1002,7 +1039,7 @@ def time_oracle(L, batches, info, max_steps, warmup, budget_s):
         torch.set_num_threads(cores)
         single = {"ms_per_step": round(min(t1) * 1e3, 2), "cores": 1, "sample": "best of 2 steps"}
     return {"value": round(s * info["steps_per_epoch"], 3), "unit": "s/epoch", "ms_per_step": round(s * 1e3, 2),
-            "cores": cores, "kind": "port", "single_thread": single,
+            "cores": cores, "kind": "port", "steps": len(ts), "single_thread": single,
             "sample": f"{len(ts)} full training steps (of {info['steps_per_epoch']} per epoch) of the same workload, "
                       f"{warmup} warm-up; oracle/ngcf_oracle.py = the reference's torch.sparse CPU path incl. its host "
                       f"float64 node-dropout mask"}
@@ -1016,10 +1053,11 @@ def run_reference(args):
               "(matrix.py:55-62) and cannot hold this graph; no CPU run exists for the device-generated pl-* shapes"})
         return
     L, batches, info = make_workload(args.shape)
-    res = time_cpu_reference(L, batches, info, max_steps=args.steps, warmup=min(args.warmup, 2), budget_s=200.0)
+    warmup = min(args.warmup, 2)
+    res = time_cpu_reference(L, batches, info, max_steps=args.steps, warmup=warmup, budget_s=float("inf"))
     spe = info["steps_per_epoch"]
     out = {"impl": "reference", "metric": METRIC, "value": res["value"], "unit": "s/epoch", "n_gpus": args.gpus,
-           "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": False,
+           "steps": res["steps"], "warmup": warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": False,
            "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
            "config": {"workload": info["workload"], "steps_per_epoch": spe},
            "run": {"device": "cpu", "kind": res["kind"], "cores": res["cores"]},

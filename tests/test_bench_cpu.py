@@ -26,7 +26,7 @@ def _json_lines(stdout):
 @pytest.fixture(scope="module")
 def reference_line():
     # the reference's own shape (BASELINE.json configs[0]): small enough for a CPU test
-    r = _run(["--impl", "reference", "--shape", "seoul", "--steps", "1", "--warmup", "1"])
+    r = _run(["--impl", "reference", "--shape", "seoul", "--steps", "2", "--warmup", "1"])
     assert r.returncode == 0, r.stderr[-2000:]
     lines = _json_lines(r.stdout)
     assert len(lines) == 1, "the reference arm prints exactly one JSON line on stdout"
@@ -42,6 +42,7 @@ def test_reference_arm_prints_the_contract_line(reference_line):
     assert d["vs_baseline"] is None                                  # BASELINE.json publishes no number for this metric
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
+    assert d["steps"] == cb["steps"] == 2 and d["warmup"] == 1                   # the steps it ran, no time budget
     assert d["e2e"] == {"value": d["value"], "unit": "s/epoch", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
@@ -73,6 +74,41 @@ def test_device_generated_shapes_have_no_reference_run():
     assert r.returncode == 0
     (d,) = _json_lines(r.stdout)
     assert d["impl"] == "reference" and "unavailable" in d
+
+
+def test_bad_arguments_are_refused():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = _run(args, timeout=120)
+        assert r.returncode == 2 and _json_lines(r.stdout) == [], args
+
+
+def test_dump_outputs_writes_the_loss_and_every_gradient(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    torch.manual_seed(0)
+    m = torch.nn.Sequential(torch.nn.Embedding(5000, 16), torch.nn.Linear(16, 8))
+    loss = m(torch.randint(0, 5000, (64,))).square().sum()
+    loss.backward()
+    bench.dump_outputs(str(tmp_path / "full"), loss, m)
+    names = {"loss.npy", "grad.0.weight.npy", "grad.1.weight.npy", "grad.1.bias.npy"}
+    assert set(os.listdir(tmp_path / "full")) == names
+    got = np.load(tmp_path / "full" / "loss.npy")
+    assert got.dtype == np.float64 and got.tolist() == [float(loss)]
+    for k, p in m.named_parameters():
+        g = np.load(tmp_path / "full" / f"grad.{k}.npy")
+        assert g.dtype == np.float32 and np.array_equal(g, p.grad.numpy()), k
+    # past the size limit: a seeded sample of every gradient's rows, the same rows on every call
+    monkeypatch.setattr(bench, "DUMP_BYTES", 64 << 10)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), loss, m)
+    assert sum(np.load(tmp_path / "s1" / f).nbytes for f in names - {"loss.npy"}) <= 64 << 10
+    for f in names:
+        a, b = np.load(tmp_path / "s1" / f), np.load(tmp_path / "s2" / f)
+        assert np.array_equal(a, b), f
+    full = {r.tobytes() for r in np.load(tmp_path / "full" / "grad.0.weight.npy")}
+    part = np.load(tmp_path / "s1" / "grad.0.weight.npy")
+    assert 0 < len(part) < 5000 and all(r.tobytes() in full for r in part)
 
 
 def test_product_arm_refuses_to_run_without_a_gpu():
