@@ -298,6 +298,28 @@ int ngcf_score_topk_workspace(int64_t n_users, int64_t n_items, int D, int k, si
 int ngcf_score_topk(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
                     float* out_val /*[n_users,k]*/, int64_t* out_idx /*[n_users,k]*/,
                     void* workspace, size_t workspace_bytes, void* stream);
+/* The same ranking with items removed per user (full-ranking evaluation: a user's training items are never
+ * recommended).  Row u's items excl_idx[excl_ptr[u] .. excl_ptr[u+1]) must be ascending and unique (excl_idx may be
+ * NULL when every row is empty); n_items < 2^31.  A row with fewer than k items left ends in slots of idx = -1,
+ * val = -FLT_MAX.  workspace: ngcf_score_topk_workspace bytes.  k <= 32 with n_items >= 1024 and D % 4 == 0 runs on
+ * the tensor cores like ngcf_score_topk; other shapes (k > 32 among them) run the much slower CUDA-core kernel. */
+int ngcf_score_topk_excluding(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
+                              const int64_t* excl_ptr /*[n_users+1]*/, const int32_t* excl_idx,
+                              float* out_val /*[n_users,k]*/, int64_t* out_idx /*[n_users,k]*/,
+                              void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- full-ranking metrics against held-out items ------------------------------------------------------------------
+ * topk_idx [n_users,k]: ranked item ids per user (-1 = empty slot), e.g. from ngcf_score_topk_excluding; truth_ptr
+ * [n_users+1] / truth_idx: per user the ascending unique held-out item ids.  For each of the n_K cut-offs Ks_host
+ * (strictly ascending, 1 <= K <= k <= 128, n_K <= 8), with hits = how many of the first K ids are held out:
+ *   recall = hits / |T|,  precision = hits / K,  hit = hits > 0,
+ *   ndcg = sum over hit positions p < K of 1/log2(p+2)  /  sum over p < min(|T|, K) of 1/log2(p+2).
+ * per_user [n_users, n_K, 4] = (recall, precision, ndcg, hit) per K; users with an empty T get zeros and are not
+ * counted.  totals [n_K*4 + 1]: the means over the counted users (double sums in a fixed order: bit-reproducible;
+ * 0 when none is counted), then the counted users' number. */
+int ngcf_rank_metrics(const int64_t* topk_idx, int64_t n_users, int k, const int64_t* truth_ptr,
+                      const int32_t* truth_idx, const int* Ks_host, int n_K, float* per_user, float* totals,
+                      void* stream);
 
 /* ---- optimizer step: torch.optim.Adam(model.parameters(), lr) of main.py:74, stepped at experiment.py:58 -----------
  * One launch over up to NGCF_ADAM_MAX_TENSORS parameter tensors (host arrays of device pointers, sizes in elements):

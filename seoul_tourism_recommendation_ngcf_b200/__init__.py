@@ -5,7 +5,7 @@ from .experiment import Experiment, eval_groups
 from .graph import GraphedStep
 from .optim import Adam
 from .sampler import TourDataset, sample_negatives
-from .scoring import score_topk
+from .scoring import Interactions, full_rank_eval, rank_metrics, score_topk
 
 __all__ = ["NGCF", "BPR", "GraphedStep", "Adam", "score_topk", "Experiment", "eval_groups", "TourDataset",
-           "sample_negatives"]
+           "sample_negatives", "Interactions", "full_rank_eval", "rank_metrics"]

@@ -81,6 +81,8 @@ SIGNATURES = {
     "ngcf_push_selected_rows": [C.POINTER(_vp), C.POINTER(_vp), _vp, C.c_int, C.c_int, _i64, _i64, C.c_int, C.POINTER(_vp),
                                 C.POINTER(_i64), C.POINTER(_i64), C.c_int, _vp, _vp],
     "ngcf_score_topk": [_vp, _i64, _vp, _i64, C.c_int, C.c_int, _vp, _vp, _vp, _sz, _vp],
+    "ngcf_score_topk_excluding": [_vp, _i64, _vp, _i64, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _sz, _vp],
+    "ngcf_rank_metrics": [_vp, _i64, C.c_int, _vp, _vp, C.POINTER(C.c_int), C.c_int, _vp, _vp, _vp],
 }
 
 _lib = None

@@ -80,6 +80,15 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
+// first position in [lo, hi) of the ascending list a whose value is >= v (hi if there is none)
+__device__ __forceinline__ int64_t lower_bound_i32(const int32_t* __restrict__ a, int64_t lo, int64_t hi, int v) {
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (a[mid] < v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
 __device__ __forceinline__ float4 ld_f4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st_f4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 

@@ -5,6 +5,7 @@
 // (coalesced, one dot product per warp via shuffle reduction) and keep a sorted per-warp top-k list in
 // shared memory; the lists are merged per CTA, then per user by a second kernel.
 #include <float.h>
+#include <limits.h>
 
 #include "common.cuh"
 
@@ -41,9 +42,12 @@ __device__ __forceinline__ void warp_insert(float* lv, int* li, int k, float s, 
     __syncwarp();
 }
 
+// kExclude: the items of the user's ascending exclusion list [excl_ptr[user], excl_ptr[user+1]) of excl_idx are skipped
+template <bool kExclude>
 __global__ void __launch_bounds__(TK_WARPS * 32)
 score_partial_kernel(const float* __restrict__ U, const float* __restrict__ I, int64_t n_items, int D, int k,
-                     int n_split, float* __restrict__ pv, int* __restrict__ pi) {
+                     int n_split, float* __restrict__ pv, int* __restrict__ pi, const int64_t* __restrict__ excl_ptr,
+                     const int32_t* __restrict__ excl_idx) {
     extern __shared__ __align__(16) float smem[];
     float* us = smem;                                  // [D]
     float* lv = us + ((D + 3) & ~3);                   // [TK_WARPS][k]
@@ -57,7 +61,20 @@ score_partial_kernel(const float* __restrict__ U, const float* __restrict__ I, i
     const int64_t i0 = split * per, i1 = min(n_items, i0 + per);
     float* mylv = lv + warp * k;
     int* myli = li + warp * k;
+    // exclusion cursor of the warp (warp-uniform): it visits its items in ascending order
+    const int32_t *xp = nullptr, *xe = nullptr;
+    int xnext = INT_MAX;
+    if (kExclude) {
+        const int64_t e = excl_ptr[user + 1];
+        xp = excl_idx + lower_bound_i32(excl_idx, excl_ptr[user], e, (int)(i0 + warp));
+        xe = excl_idx + e;
+        xnext = xp < xe ? *xp : INT_MAX;
+    }
     for (int64_t it = i0 + warp; it < i1; it += TK_WARPS) {
+        if (kExclude) {
+            while (xnext < it) xnext = ++xp < xe ? *xp : INT_MAX;
+            if (xnext == it) continue;
+        }
         const float* ir = I + it * D;
         float s = 0.f;
         for (int c = lane; c < D; c += 32) s = fmaf(us[c], ir[c], s);
@@ -121,7 +138,8 @@ bool ngcf_score_topk_tc_eligible(int64_t n_users, int64_t n_items, int D, int k)
 int ngcf_score_topk_tc_splits(int64_t n_users, int64_t n_items);
 size_t ngcf_score_topk_tc_pack_bytes(int64_t n_users, int64_t n_items, int D);
 int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k, int n_split,
-                       float* pv, int* pi, uint8_t* pack, cudaStream_t st);
+                       float* pv, int* pi, uint8_t* pack, const int64_t* excl_ptr, const int32_t* excl_idx,
+                       cudaStream_t st);
 bool ngcf_use_tensor_cores();
 
 extern "C" int ngcf_score_topk_workspace(int64_t n_users, int64_t n_items, int D, int k, size_t* bytes_host) {
@@ -134,9 +152,10 @@ extern "C" int ngcf_score_topk_workspace(int64_t n_users, int64_t n_items, int D
     return NGCF_OK;
 }
 
-extern "C" int ngcf_score_topk(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
-                               float* out_val, int64_t* out_idx, void* workspace, size_t workspace_bytes,
-                               void* stream) {
+// ngcf_score_topk and ngcf_score_topk_excluding; excl_ptr == NULL: no exclusion (the kernels that read no list)
+static int score_topk_impl(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
+                           const int64_t* excl_ptr, const int32_t* excl_idx, float* out_val, int64_t* out_idx,
+                           void* workspace, size_t workspace_bytes, void* stream) {
     NGCF_REQUIRE(U && I && out_val && out_idx, "score_topk: null pointer");
     NGCF_REQUIRE(k > 0 && k <= TK_MAXK, "score_topk: k %d not in [1,%d]", k, TK_MAXK);
     NGCF_REQUIRE(k <= n_items, "score_topk: k %d > number of items %lld (torch.topk raises too)", k, (long long)n_items);
@@ -157,7 +176,8 @@ extern "C" int ngcf_score_topk(const float* U, int64_t n_users, const float* I, 
         float* pv = reinterpret_cast<float*>(workspace);
         int* pi = reinterpret_cast<int*>(pv + (size_t)n_users * ns * k);
         uint8_t* pack = reinterpret_cast<uint8_t*>(pi + (size_t)n_users * ns * k);
-        if ((rc = ngcf_score_topk_tc(U, n_users, I, n_items, D, k, ns, pv, pi, pack, st)) != NGCF_OK) return rc;
+        if ((rc = ngcf_score_topk_tc(U, n_users, I, n_items, D, k, ns, pv, pi, pack, excl_ptr, excl_idx, st)) != NGCF_OK)
+            return rc;
         score_merge_kernel<<<(unsigned)n_users, 32, sizeof(float) * 2 * k, st>>>(pv, pi, ns, k, out_val, out_idx);
         NGCF_LAUNCH_OK("score_merge_kernel");
         return NGCF_OK;
@@ -169,9 +189,28 @@ extern "C" int ngcf_score_topk(const float* U, int64_t n_users, const float* I, 
     NGCF_REQUIRE(smem1 <= 48 * 1024, "score_topk: D %d too wide for the v1 kernel", D);
     NGCF_REQUIRE(n_users <= 0x7fffffffLL, "score_topk: too many users");
     dim3 grid((unsigned)n_users, (unsigned)ns);
-    score_partial_kernel<<<grid, TK_WARPS * 32, smem1, st>>>(U, I, n_items, D, k, ns, pv, pi);
+    if (excl_ptr)
+        score_partial_kernel<true><<<grid, TK_WARPS * 32, smem1, st>>>(U, I, n_items, D, k, ns, pv, pi, excl_ptr, excl_idx);
+    else
+        score_partial_kernel<false><<<grid, TK_WARPS * 32, smem1, st>>>(U, I, n_items, D, k, ns, pv, pi, nullptr, nullptr);
     NGCF_LAUNCH_OK("score_partial_kernel");
     score_merge_kernel<<<(unsigned)n_users, 32, sizeof(float) * 2 * k, st>>>(pv, pi, ns, k, out_val, out_idx);
     NGCF_LAUNCH_OK("score_merge_kernel");
     return NGCF_OK;
+}
+
+extern "C" int ngcf_score_topk(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
+                               float* out_val, int64_t* out_idx, void* workspace, size_t workspace_bytes,
+                               void* stream) {
+    return score_topk_impl(U, n_users, I, n_items, D, k, nullptr, nullptr, out_val, out_idx, workspace, workspace_bytes,
+                           stream);
+}
+
+extern "C" int ngcf_score_topk_excluding(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k,
+                                         const int64_t* excl_ptr, const int32_t* excl_idx, float* out_val,
+                                         int64_t* out_idx, void* workspace, size_t workspace_bytes, void* stream) {
+    NGCF_REQUIRE(excl_ptr, "score_topk_excluding: null exclusion row pointer");
+    NGCF_REQUIRE(n_items <= 0x7fffffffLL, "score_topk_excluding: more than 2^31-1 items");
+    return score_topk_impl(U, n_users, I, n_items, D, k, excl_ptr, excl_idx, out_val, out_idx, workspace,
+                           workspace_bytes, stream);
 }

@@ -10,7 +10,12 @@
 // tcgen05.mma chain into a double-buffered 128 x 128 fp32 accumulator in TMEM, and the epilogue threads (TMEM lane = user) filter the 128 scores of their user
 // against that user's current k-th best and put the few survivors into that user's list in shared memory.  The score
 // matrix never exists; partial lists per (user, item range) are merged by score_merge_kernel (topk.cu).
+// Full-ranking evaluation drops each user's training items (kExclude): an epilogue thread visits its user's items in
+// ascending order, so a cursor into the user's ascending exclusion list plus the next excluded id in a register turn
+// each 32-item chunk into one compare (a 32-bit mask is built only when that id falls inside the chunk); no shared
+// memory is added.
 #include <float.h>
+#include <limits.h>
 #include <stdlib.h>
 
 #include "tc.cuh"
@@ -36,6 +41,8 @@ struct ScoreTcArgs {
     int tiles_per_split;       // item tiles per split
     float* pv;                 // [n_users][n_split][k]
     int* pi;
+    const int64_t* excl_ptr;   // kExclude: per user [excl_ptr[u], excl_ptr[u+1]) of excl_idx, ascending unique item ids
+    const int32_t* excl_idx;
     int dbg_skip_epilogue;     // timing experiments only (NGCF_B200_TOPK_SKIP_EPI=1): accumulators are read and dropped
 };
 
@@ -44,6 +51,8 @@ struct ScoreBars {
     uint32_t tmem_base;
 };
 
+// kExclude: items on the user's exclusion list never enter its lists (the false instantiation reads no list at all)
+template <bool kExclude>
 __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArgs a) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -92,6 +101,15 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
         const int k = a.k;
         float thr = -FLT_MAX;                                             // k-th best as of the last merge
         int cnt = k;                                                      // next free slot
+        // exclusion cursor: the thread walks its items in ascending order, so one pointer into the user's ascending
+        // list suffices; xnext is the next excluded id at or after the current chunk (INT_MAX: none left)
+        int64_t xp = 0, xe = 0;
+        int xnext = INT_MAX;
+        if (kExclude && live) {
+            xe = a.excl_ptr[u0 + row + 1];
+            xp = lower_bound_i32(a.excl_idx, a.excl_ptr[u0 + row], xe, t0 * ST_ROWS);
+            xnext = xp < xe ? a.excl_idx[xp] : INT_MAX;
+        }
         auto merge = [&]() {
             const int extras = __reduce_max_sync(FULL_MASK, cnt) - k;
             for (int x = 0; x < extras; ++x) {
@@ -132,12 +150,20 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
                 }
                 if (__any_sync(FULL_MASK, cnt > k + ST_EXTRA - 32)) merge();   // room for a whole chunk of survivors
                 if (!live) continue;
+                uint32_t xmask = 0;                                       // bit j: item i0 + c*32 + j is excluded
+                if (kExclude) {
+                    const int cb = (int)(i0 + c * 32);
+                    while (xnext < cb + 32) {                             // usually one compare per chunk
+                        xmask |= 1u << (xnext - cb);
+                        xnext = ++xp < xe ? a.excl_idx[xp] : INT_MAX;
+                    }
+                }
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     const float s = v[j];
                     const int64_t item = i0 + c * 32 + j;
                     // NaN fails the comparison and is never ranked
-                    if (s > thr && item < a.n_items) {
+                    if (s > thr && item < a.n_items && !(xmask >> j & 1u)) {
                         lv[cnt * ST_ROWS + row] = s;
                         li[cnt * ST_ROWS + row] = (int)item;
                         ++cnt;
@@ -257,8 +283,10 @@ size_t ngcf_score_topk_tc_pack_bytes(int64_t n_users, int64_t n_items, int D) {
     return (ut + it) * KB * 2 * ST_BLOCK + 1024;
 }
 
+// excl_ptr / excl_idx: NULL for plain ranking, else per user the ascending unique item ids that are never ranked
 int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k, int n_split,
-                       float* pv, int* pi, uint8_t* pack, cudaStream_t st) {
+                       float* pv, int* pi, uint8_t* pack, const int64_t* excl_ptr, const int32_t* excl_idx,
+                       cudaStream_t st) {
     const int KB = (D + 31) / 32;
     const int64_t ut = (n_users + ST_ROWS - 1) / ST_ROWS, itiles = (n_items + ST_ROWS - 1) / ST_ROWS;
     uint8_t* Up = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(pack) + 1023) & ~(uintptr_t)1023);
@@ -272,11 +300,13 @@ int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t 
     }
     static int skip = -1;
     if (skip < 0) { const char* e = getenv("NGCF_B200_TOPK_SKIP_EPI"); skip = (e && e[0] == '1') ? 1 : 0; }
-    ScoreTcArgs a{Up, Ip, n_users, n_items, D, k, n_split, (int)((itiles + n_split - 1) / n_split), pv, pi, skip};
+    ScoreTcArgs a{Up, Ip, n_users, n_items, D, k, n_split, (int)((itiles + n_split - 1) / n_split), pv, pi, excl_ptr,
+                  excl_idx, skip};
     const size_t smem = 1024 + (size_t)ST_STAGES * ST_STAGE_BYTES + (size_t)(k + ST_EXTRA) * ST_ROWS * 8 + sizeof(ScoreBars);
-    NGCF_CUDA(cudaFuncSetAttribute(score_topk_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));   // per device
+    auto kern = excl_ptr ? score_topk_tc_kernel<true> : score_topk_tc_kernel<false>;
+    NGCF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));   // per device
     dim3 grid((unsigned)ut, (unsigned)n_split);
-    score_topk_tc_kernel<<<grid, ST_THREADS, smem, st>>>(a);
+    kern<<<grid, ST_THREADS, smem, st>>>(a);
     NGCF_LAUNCH_OK("score_topk_tc_kernel");
     return NGCF_OK;
 }
