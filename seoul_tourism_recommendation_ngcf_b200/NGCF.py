@@ -30,8 +30,7 @@ def _stream() -> int:
 class _Ctx:
     """Per-forward state shared by the autograd node and the module (layer activations, plan, masks)."""
     __slots__ = ("plan", "E", "S", "dims", "vals_f", "vals_b", "mess_mult", "mess_p", "seed", "seed_dev", "masked", "drop_p", "bits_f", "bits_b", "comp_f", "comp_b", "mess_bits",
-                 "rows", "offsets", "W1", "W2", "fresh_key", "node_mode", "last_partial", "comp_b_stream", "needs_grad", "comp_b_late",
-                 "fm_stream")
+                 "rows", "offsets", "W1", "W2", "fresh_key", "node_mode", "last_partial", "fm_stream")
 
 
 def _capturing() -> bool:
@@ -72,9 +71,6 @@ class _Propagate(torch.autograd.Function):
         st.bits_f = st.bits_b = st.comp_f = st.comp_b = None
         st.node_mode = mod._node_mode
         st.last_partial = None
-        st.comp_b_stream = None
-        st.comp_b_late = False
-        needs_grad = st.needs_grad
         if st.drop_p > 0:
             # this step's node-dropout decisions for all K layers, drawn once instead of a hash evaluation per entry in
             # each of the 2K products; a symmetric L serves both directions from one pass.  "compact" (default) also
@@ -85,27 +81,10 @@ class _Propagate(torch.autograd.Function):
             # (every width, the last one too: the batch-row gradient rows of the final backward product are D_total wide)
             node_mode = mod._node_mode if all(d % 4 == 0 for d in st.dims) or mod._node_mode == "inkernel" else "bits"
             st.node_mode = node_mode
-            if node_mode == "compact" and shared and needs_grad and mod._compact_overlap == "late" and sh is None:
-                # the forward needs L's survivors now; L^T's are first read by the backward's first product: that half of
-                # the pass is queued on a second stream BEHIND the last layer (below), where the small launches between
-                # the two passes (row gather, BPR, row-gradient scatter: a few CTAs each) leave the GPU nearly idle
-                st.comp_f, _ = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=True, as_Lt=False)
-                st.comp_b_late = True
-            elif node_mode == "compact" and shared and needs_grad and mod._compact_overlap == "1":
-                # the same split with L^T's half forked right here, beside the forward's first kernels (measured slower
-                # than one combined pass: it takes SM time from the critical path)
-                st.comp_f, _ = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=True, as_Lt=False)
-                main = torch.cuda.current_stream()
-                if mod._side_stream2 is None:
-                    mod._side_stream2 = torch.cuda.Stream(device=dev)
-                mod._side_stream2.wait_stream(main)
-                with torch.cuda.stream(mod._side_stream2):
-                    _, st.comp_b = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=False, as_Lt=True)
-                for e_, c_ in st.comp_b:                                # allocated under the side stream, used on main
-                    e_.record_stream(main)
-                    c_.record_stream(main)
-                st.comp_b_stream = mod._side_stream2
-            elif node_mode == "compact":
+            if node_mode == "compact":
+                # L's and (symmetric L) L^T's survivor lists in one pass: L^T's half on a second stream, beside the
+                # forward or behind its last layer, measured slower on one B200 (0.518 / 0.509-0.513 vs 0.502-0.510 ms
+                # per step: two more launches and the entries read twice cost more than the overlap hides)
                 st.comp_f, ct = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=True, as_Lt=shared)
                 if shared:
                     st.comp_b = ct
@@ -156,7 +135,7 @@ class _Propagate(torch.autograd.Function):
                                           _lib.ptr(st.mess_bits[k]), float(st.mess_p[k]), st.seed, _lib.ptr(st.seed_dev), k, r0, En.data_ptr(),
                                           _stream()),
                        "dense_fwd")                                                          # NGCF.py:131-142
-            if xkey is not None and k == K - 1 and mod._sparse_last:
+            if xkey is not None and k == K - 1:
                 # nothing downstream gathers from the LAST layer's output: other ranks need it for the <= 3 B batch rows only
                 # (NGCF.py:151-155); all_users_emb / all_items_emb complete it on first read (_materialize)
                 mod._xchg.push_selected(xkey, r0, nloc, st.rows[:n_sets], st.offsets[:n_sets])
@@ -167,17 +146,6 @@ class _Propagate(torch.autograd.Function):
                 all_gather_rows(Xn, En, mod._group)
             st.S.append(S)
             st.E.append(Xn)
-        if st.comp_b_late:
-            main = torch.cuda.current_stream()
-            if mod._side_stream2 is None:
-                mod._side_stream2 = torch.cuda.Stream(device=dev)
-            mod._side_stream2.wait_stream(main)
-            with torch.cuda.stream(mod._side_stream2):
-                _, st.comp_b = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=False, as_Lt=True)
-            for e_, c_ in st.comp_b:                                    # allocated under the side stream, used on main
-                e_.record_stream(main)
-                c_.record_stream(main)
-            st.comp_b_stream = mod._side_stream2
         D = sum(st.dims)
         layers, dims = _lib.ptr_array(st.E), _lib.int_array(st.dims)
         outs = [torch.empty(st.rows[j].numel(), D, dtype=torch.float32, device=dev) for j in range(n_sets)]
@@ -239,12 +207,12 @@ class _Propagate(torch.autograd.Function):
             _, st.bits_b = node_dropout_bits(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=False, as_Lt=True)
         gE_next = None
         col_off = D
-        # the weight-gradient kernels need gM only: with the gS exchange queued behind the backward kernel (row-sharded
-        # runs) they run beside it on a second stream; each layer then keeps its own gM until the join below
+        # the weight-gradient kernels need gM only: beside the transposed product (and the gS exchange queued behind the
+        # backward kernel in row-sharded runs) they run on a second stream; each layer then keeps its own gM until the
+        # join below.  0.508 -> 0.494 ms per step on one B200 (GraphedStep), 0.611 -> 0.594 ms at 2 ranks.
         # (second streams cost the HOST two event calls per fork and join: they pay under CUDA-graph capture, where the
         # step is replayed without host work, and in row-sharded runs; the eager single-GPU step is host-bound already)
-        overlap = mod._wgrad_overlap != "0" and (mod._wgrad_overlap == "force" or _capturing() or
-                                                  (sh is not None and mod._xchg is not None))
+        overlap = _capturing() or (sh is not None and mod._xchg is not None)
         if overlap:
             if mod._side_stream is None:
                 mod._side_stream = torch.cuda.Stream(device=dev)
@@ -290,9 +258,6 @@ class _Propagate(torch.autograd.Function):
                 gS_all = gS
             vals = st.vals_b[k] if st.vals_b is not None else None
             last = (k == 0)
-            if st.comp_b_stream is not None:                          # L^T's survivor lists were compacted on a second stream
-                torch.cuda.current_stream().wait_stream(st.comp_b_stream)
-                st.comp_b_stream = None
             gE_next = spmm(side, vals, gS_all, d_in, addend=gEl, slot=slot_loc if last else None,
                            gsum=gsum if last else None, drop_p=st.drop_p, seed=st.seed, seed_dev=st.seed_dev, layer=k,
                            transposed=True, row_offset=r0, keep_bits=st.bits_b,
@@ -394,24 +359,8 @@ class NGCF(nn.Module):
         self._shard = None       # sharded.RowShards once shard() was called
         self._group = None
         self._xchg = None        # sharded.PeerExchange (peer-memory exchange) when available
-        self._sparse_last = os.environ.get("NGCF_B200_SPARSE_LAST", "1") == "1"
-        # weight-gradient kernels on a second stream beside the transposed product (and the gS exchange of a row-sharded
-        # run): 0.508 -> 0.494 ms per step on one B200 (GraphedStep), 0.611 -> 0.594 ms at 2 ranks; "0" switches it off,
-        # "force" also uses it in the eager single-GPU step (slower there: the eager step is bound by host issue)
-        self._wgrad_overlap = os.environ.get("NGCF_B200_WGRAD_OVERLAP", "1")
-        self._side_stream = None
-        self._side_stream2 = None
-        # L^T's survivor lists on a second stream beside the forward: measured slower on one B200 (0.518 vs 0.510 ms per
-        # step: the compaction is issue-bound and takes SM time from the forward's first kernels), so opt-in only
-        # L^T's half of the node-dropout compaction on a second stream: "1" = forked at the start of the forward, "late" =
-        # behind the last layer (beside the small launches between the passes).  Both measured SLOWER than the one combined
-        # pass on one B200 (0.518 / 0.509-0.513 vs 0.502-0.510 ms per step: two more launches and the entries read twice
-        # cost more than the overlap hides), so the default is "0"; profiles/r02_overlap_experiments.txt
-        self._compact_overlap = os.environ.get("NGCF_B200_COMPACT_OVERLAP", "0")          # "0" | "1" | "late"
-        # the feature mix (two small launches that rewrite <= B user rows) on a second stream beside the node-dropout
-        # compaction, which does not touch the table; joined before the first product (0.502 -> 0.499 ms per step)
-        self._featmix_overlap = os.environ.get("NGCF_B200_FEATMIX_OVERLAP", "1") == "1"
-        self._side_stream3 = None
+        self._side_stream = None     # weight gradients beside the transposed product (_Propagate.backward)
+        self._side_stream3 = None    # feature mix beside the node-dropout compaction (forward)
         self._trace = None       # debugging aid: set to a list to record the backward's per-layer tensors
         self._inject = None      # tests only: dict(edge_keep=[K x uint8[nnz]], mess_mult=[K x [N,d]])
 
@@ -543,7 +492,7 @@ class NGCF(nn.Module):
         K, N = self.n_layer, self.n_user + self.n_item
         if (self._side_stream is None or self._side_stream.device != dev) and not _capturing():
             # second streams of the capture-time overlaps, handed out of torch's pool BEFORE any capture begins
-            self._side_stream, self._side_stream2, self._side_stream3 = (torch.cuda.Stream(device=dev) for _ in range(3))
+            self._side_stream, self._side_stream3 = (torch.cuda.Stream(device=dev) for _ in range(2))
 
         def ix(t):
             return t.to(device=dev, dtype=torch.int64).contiguous()
@@ -564,8 +513,10 @@ class NGCF(nn.Module):
                                             u_id.numel(), float(self.emb_ratio), self._winner.data_ptr(), _stream()),
                        "feature_mix")                                        # NGCF.py:103-115
 
+        # the feature mix (two small launches that rewrite <= B user rows) on a second stream beside the node-dropout
+        # compaction, which does not touch the table; joined before the first product (0.502 -> 0.499 ms per step)
         fm_stream = None
-        if self._featmix_overlap and self._shard is None and _capturing() and bool(node_flag) and \
+        if self._shard is None and _capturing() and bool(node_flag) and \
                 (self.node_dropout or 0) > 0 and self.rng == "device":
             main = torch.cuda.current_stream()
             if self._side_stream3 is None:
@@ -627,8 +578,6 @@ class NGCF(nn.Module):
         st.rows = [u_id, pos_item] + ([neg_item] if has_neg else [])
         st.offsets = [0, self.n_user] + ([self.n_user] if has_neg else [])
 
-        # (autograd.Function.forward runs with grad mode off: whether a backward will follow is decided here)
-        st.needs_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
         wb = [l.weight for l in self.w1_list] + [l.bias for l in self.w1_list] + \
              [l.weight for l in self.w2_list] + [l.bias for l in self.w2_list]
         outs = _Propagate.apply(self, st, len(st.rows), self.user_embedding.weight, self.item_embedding.weight, *wb)

@@ -49,8 +49,7 @@ int ngcf_num_sms();   // cached cudaDevAttrMultiProcessorCount of the current de
 // launch_dependents at its top, so the NEXT kernel's CTAs become resident while this one drains and run their
 // prologue (barriers, TMEM allocation, tile descriptors, weight tiles); they stop at pdl_wait() — which returns once
 // the preceding kernel has completed and its writes are visible — before touching anything a predecessor produced and
-// before writing anything at all.  NGCF_B200_PDL=0 launches everything fully serialised (A/B timing).
-bool ngcf_pdl_enabled();
+// before writing anything at all.
 
 template <typename... KArgs, typename... Args>
 static inline cudaError_t ngcf_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
@@ -62,7 +61,7 @@ static inline cudaError_t ngcf_launch_pdl(void (*kernel)(KArgs...), dim3 grid, d
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = ngcf_pdl_enabled() ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);

@@ -3,8 +3,6 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <stdarg.h>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tmap.h"
 
@@ -18,15 +16,6 @@ void ngcf_set_error(const char* fmt, ...) {
     va_start(ap, fmt);
     vsnprintf(g_err, sizeof(g_err), fmt, ap);
     va_end(ap);
-}
-
-bool ngcf_pdl_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NGCF_B200_PDL");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
 }
 
 int ngcf_num_sms() {

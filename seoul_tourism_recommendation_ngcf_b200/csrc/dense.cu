@@ -3,9 +3,6 @@
 //
 // v1 arithmetic: exact fp32 FFMA register-tiled micro-kernels (4x4 per thread, operands in shared memory,
 // LDS.128).  Every width 1..128 is accepted (the reference's own width is 65).
-#include <stdlib.h>
-#include <string.h>
-
 #include "common.cuh"
 
 namespace {
@@ -469,12 +466,6 @@ int ngcf_dense_bwd_tc(const float* gE_next, const int32_t* slot, const float* gs
                       uint64_t seed, const uint64_t* seed_dev, int layer, int64_t row_offset, int gh_normalized, float* gS, float* gEl,
                       float* gW1, float* gb1, float* gW2, float* gb2, float* gM_scratch, cudaStream_t st);
 
-// NGCF_B200_DENSE=ffma forces the exact-fp32 FFMA kernels (A/B comparisons); default: tensor cores where eligible
-bool ngcf_use_tensor_cores() {
-    const char* e = getenv("NGCF_B200_DENSE");
-    return !(e && strcmp(e, "ffma") == 0);
-}
-
 extern "C" int ngcf_pack_weights(const float* W1, const float* b1, const float* W2, const float* b2, int d_in,
                                  int d_out, float* wcat, float* bias_eff, void* stream) {
     NGCF_REQUIRE(W1 && b1 && W2 && b2 && wcat && bias_eff, "pack_weights: null pointer");
@@ -515,7 +506,7 @@ extern "C" int ngcf_dense_fwd(const float* S, const float* E, int64_t n_rows, in
     NGCF_REQUIRE(mess_p >= 0.f && mess_p < 1.f, "dense_fwd: mess_p %f not in [0,1)", mess_p);
     NGCF_REQUIRE(n_rows >= 0 && n_rows < ((int64_t)1 << 31), "dense_fwd: n_rows %lld", (long long)n_rows);
     if (n_rows == 0) return NGCF_OK;
-    if (ngcf_use_tensor_cores() && ngcf_dense_fwd_tc_eligible(d_in, d_out) && aligned16(S) && aligned16(E) &&
+    if (ngcf_dense_fwd_tc_eligible(d_in, d_out) && aligned16(S) && aligned16(E) &&
         aligned16(E_out) && (!mess_mult || aligned16(mess_mult)))
         return ngcf_dense_fwd_tc(S, E, n_rows, d_in, d_out, wcat, bias_eff, slope, mess_mult, mess_bits, mess_p, seed, seed_dev,
                                  layer, row_offset, E_out, as_stream(stream));
@@ -550,7 +541,7 @@ extern "C" int ngcf_dense_bwd(const float* gE_next, const int32_t* slot, const f
     NGCF_REQUIRE(mess_p >= 0.f && mess_p < 1.f, "dense_bwd: mess_p %f not in [0,1)", mess_p);
     NGCF_REQUIRE(n_rows >= 0 && n_rows < ((int64_t)1 << 31), "dense_bwd: n_rows %lld", (long long)n_rows);
     if (n_rows == 0) return NGCF_OK;
-    if (ngcf_use_tensor_cores() && gM_scratch && ngcf_dense_bwd_tc_eligible(d_in, d_out, gh_normalized) && aligned16(S) &&
+    if (gM_scratch && ngcf_dense_bwd_tc_eligible(d_in, d_out, gh_normalized) && aligned16(S) &&
         aligned16(E) && aligned16(gS) && aligned16(gEl) && aligned16(gM_scratch))
         return ngcf_dense_bwd_tc(gE_next, slot, gsum, ld_gsum, col_off, E_out, S, E, n_rows, d_in, d_out, W1, W2,
                                  slope, mess_mult, mess_bits, mess_p, seed, seed_dev, layer, row_offset, gh_normalized, gS,

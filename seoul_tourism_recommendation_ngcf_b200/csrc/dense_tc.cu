@@ -2,17 +2,9 @@
 //     E_out = Dropout(LeakyReLU((S+E)·W1^T + (S*E)·W2^T + 2 b1 + b2))
 // as ONE GEMM per 128-row tile:  [128 x 2d] · [2d x d_out], A = [S+E | S*E] built on the fly, B = [W1 | W2]
 // resident in shared memory for the whole (persistent) kernel, fp32 accumulator in TMEM, 3xTF32 (tc.cuh).
-//
-// Warp roles (416 threads, one CTA per SM):
-//   warps 0-7   epilogue: tcgen05.ld the accumulator (TMEM lane = tile row), bias + LeakyReLU + dropout, store
-//   warp  8     TMEM allocation; lane 0 issues every tcgen05.mma / tcgen05.commit
-//   warps 9-12  loaders: coalesced 128-bit reads of S and E, split into TF32 hi/lo, written straight into the
-//               128-byte-swizzled K-major operand layout
-// A is pipelined per 32-wide K block: block kb of the next tile is refilled as soon as the MMAs that read it have
-// completed (tcgen05.commit -> empty[kb]); the accumulator is double buffered in TMEM so the epilogue of tile t
-// overlaps the loads and MMAs of tile t+1.
+// The accumulator is double buffered in TMEM so the epilogue of tile t overlaps the loads and MMAs of tile t+1
+// (warp roles: dense_fwd_tma_kernel).
 #include <stdlib.h>
-#include <string.h>
 
 #include "tc.cuh"
 #include "tmap.h"
@@ -63,21 +55,11 @@ struct FwdTcArgs {
 };
 enum { FW_SINGLE = 0, FW_PARTIAL = 1, FW_FINAL = 2 };
 
-struct Bars {
-    uint64_t full[TC_MAX_KB];
-    uint64_t empty[TC_MAX_KB];
-    uint64_t tmem_full[2];
-    uint64_t tmem_empty[2];
-    uint32_t tmem_base;
-};
-
-// Forward roles: warps 0-7 epilogue (warp w: TMEM lane quarter w & 3, 32-column chunk w >> 2), warp 8 MMA issuer,
-// warps 9-12 loaders.  (ncu, first version with 4 epilogue + 8 loader warps: the loaders sat idle 59 % of the time
-// waiting for the epilogue — bias/LeakyReLU/dropout RNG for 128 x 64 outputs per tile in 4 warps was the critical path.)
+// Forward roles: warps 0-7 epilogue (warp w: TMEM lane quarter w & 3, 32-column chunk w >> 2), warp 8 MMA issuer.
+// (ncu, first version with 4 epilogue + 8 loader warps: the loaders sat idle 59 % of the time waiting for the
+// epilogue — bias/LeakyReLU/dropout RNG for 128 x 64 outputs per tile in 4 warps was the critical path.)
 constexpr int FW_EPI_WARPS = 8;
-constexpr int FW_LOAD_WARPS = 4;
 constexpr int FW_MMA_WARP = FW_EPI_WARPS;
-static_assert((FW_EPI_WARPS + 1 + FW_LOAD_WARPS) * 32 == TC_THREADS, "forward roles must fill the CTA");
 
 // 32 x 32 fp32 transposition buffer without padding: 16-byte chunk c of row r lives at chunk position c ^ (r & 7)
 __device__ __forceinline__ int stage_off(int r, int c) { return r * 32 + ((c ^ (r & 7)) << 2); }
@@ -178,190 +160,13 @@ __device__ __forceinline__ void fwd_epilogue_role(const FwdTcArgs& a, float* sta
     }
 }
 
-template <int MM>
-__global__ void __launch_bounds__(TC_THREADS, 1) dense_fwd_tc_kernel(FwdTcArgs a) {
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;          // operand tiles need 1024-byte alignment
-    uint8_t* smem = smem_raw + (base - smem_u32(smem_raw));
-    const int d_in = a.d_in, d_out = a.d_out;
-    const int KBH = d_in / 32, KB = 2 * KBH;                              // K blocks per half / in total
-    const int b_block = d_out * 128;                                      // bytes of one K block of B (hi or lo)
-    uint8_t* A_hi = smem;
-    uint8_t* A_lo = A_hi + KB * TC_A_BLOCK;
-    uint8_t* B_hi = A_lo + KB * TC_A_BLOCK;
-    uint8_t* B_lo = B_hi + KB * b_block;
-    float* bias_s = reinterpret_cast<float*>(B_lo + KB * b_block);
-    float* stage = bias_s + 64;                                           // [8 warps][32 x 32]
-    Bars* bars = reinterpret_cast<Bars*>(stage + FW_EPI_WARPS * 32 * 32);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    pdl_launch_dependents();
-
-    // ---- one-off setup: barriers, TMEM, weights ----------------------------------------------------------------
-    if (tid == 0) {
-        for (int i = 0; i < TC_MAX_KB; ++i) {
-            mbar_init(&bars->full[i], FW_LOAD_WARPS);
-            mbar_init(&bars->empty[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&bars->tmem_full[i], 1);
-            mbar_init(&bars->tmem_empty[i], FW_EPI_WARPS);
-        }
-        fence_mbar_init();
-    }
-    if (warp == FW_MMA_WARP) tmem_alloc(&bars->tmem_base, 128);           // 2 accumulators x 64 fp32 columns
-    pdl_wait();      // wcat / bias_eff may come from the launch right before this one (ngcf_pack_weights); S, E do
-    // B[n][k] = wcat[k][n], split and swizzled (row n of K block kb: 32 values of k)
-    // (consecutive threads take consecutive n: the four loads below are then coalesced rows of wcat; with c fastest
-    // every lane touched its own cache line and this set-up was ~30 % of the kernel's warp time in ncu)
-    for (int i = tid; i < d_out * KB * 8; i += TC_THREADS) {
-        const int n = i % d_out, c = (i / d_out) & 7, kb = i / (d_out * 8);
-        float4 w;
-        const int k = kb * 32 + c * 4;                                    // 4 consecutive k stay inside the W1 or the W2 part
-        const int wrow = k < d_in ? a.w_row1 + k : a.w_row2 + (k - d_in);
-        const float* src = a.wcat + (int64_t)wrow * a.d_out_full + a.out_off + n;
-        w.x = src[0]; w.y = src[a.d_out_full]; w.z = src[2 * a.d_out_full]; w.w = src[3 * a.d_out_full];
-        float4 hi, lo;
-        split_tf32(w, hi, lo);
-        const uint32_t off = kb * b_block + sw128_offset(n, c);
-        *reinterpret_cast<float4*>(B_hi + off) = hi;
-        *reinterpret_cast<float4*>(B_lo + off) = lo;
-    }
-    for (int i = tid; i < 64; i += TC_THREADS) bias_s[i] = i < d_out ? a.bias_eff[a.out_off + i] : 0.f;
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem_base = bars->tmem_base;
-
-    const int n_my = (a.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // tiles of this CTA
-    const bool dbg = g_bwd_dbg_on == 1 && blockIdx.x == 0 && (warp == 0 || warp == FW_MMA_WARP || warp == FW_MMA_WARP + 1);
-    if (dbg && lane == 0 && warp == 0) g_bwd_dbg[0][7][7] = clock64();
-
-    if (warp < FW_EPI_WARPS) {
-        fwd_epilogue_role<MM>(a, stage, bias_s, bars->tmem_full, bars->tmem_empty, tmem_base, n_my, warp, lane, dbg);
-    } else if (warp == FW_MMA_WARP) {
-        // ======================= MMA issuer =====================================================================
-        const uint32_t idesc = umma_idesc_tf32(TC_ROWS, d_out, 0, 0);
-        for (int it = 0; it < n_my; ++it) {
-            const int buf = it & 1;
-            mbar_wait(&bars->tmem_empty[buf], ((it >> 1) & 1) ^ 1);       // epilogue has drained this accumulator
-            tc_fence_after_sync();
-            const uint32_t tmem_d = tmem_base + buf * 64;
-            uint32_t accumulate = 0;
-            for (int hh = 0; hh < KBH; ++hh) {
-                for (int part = 0; part < 2; ++part) {
-                    const int kb = part * KBH + hh;
-                    mbar_wait(&bars->full[kb], it & 1);
-                    tc_fence_after_sync();
-                    if (lane == 0) {
-                        const uint32_t a_hi = smem_u32(A_hi + kb * TC_A_BLOCK), a_lo = smem_u32(A_lo + kb * TC_A_BLOCK);
-                        const uint32_t b_hi = smem_u32(B_hi + kb * b_block), b_lo = smem_u32(B_lo + kb * b_block);
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {                     // 4 x (K = 8 TF32 = 32 bytes) per block
-                            const uint64_t dah = umma_desc_sw128(a_hi + k * 32, 16, 1024);
-                            const uint64_t dal = umma_desc_sw128(a_lo + k * 32, 16, 1024);
-                            const uint64_t dbh = umma_desc_sw128(b_hi + k * 32, 16, 1024);
-                            const uint64_t dbl = umma_desc_sw128(b_lo + k * 32, 16, 1024);
-                            umma_tf32(tmem_d, dah, dbh, idesc, accumulate);
-                            umma_tf32(tmem_d, dal, dbh, idesc, 1);
-                            umma_tf32(tmem_d, dah, dbl, idesc, 1);
-                            accumulate = 1;
-                        }
-                        umma_commit(&bars->empty[kb]);                    // A block kb may be refilled
-                    }
-                    __syncwarp();
-                }
-            }
-            if (lane == 0) umma_commit(&bars->tmem_full[buf]);            // accumulator complete
-            __syncwarp();
-        }
-    } else {
-        // ======================= loaders ========================================================================
-        // Software-pipelined by quarter steps (64 rows x 32 columns of S and of E = 4 + 4 float4 per thread): the loads
-        // of the next quarter are in flight while this one is split and stored (first version: load a half, wait,
-        // convert — the loaders were the critical path at ~7000 cycles per tile, two exposed round trips each).
-        const int lt = tid - (FW_EPI_WARPS + 1) * 32;                     // 0 .. 127
-        constexpr int LT = FW_LOAD_WARPS * 32;
-        constexpr int QQ = (TC_ROWS / 2) * 8 / LT;                        // 16-byte chunks per thread per quarter step
-        struct Stage {
-            float4 s[QQ], e[QQ];
-        };
-        const int total_q = n_my * KBH * 2;
-        auto issue = [&](Stage& g, int i) {
-            const int it = i / (2 * KBH), hh = (i >> 1) % KBH, half_rows = (i & 1) * (TC_ROWS / 2);
-            const int64_t row0 = (int64_t)(blockIdx.x + it * gridDim.x) * TC_ROWS + half_rows;
-#pragma unroll
-            for (int q = 0; q < QQ; ++q) {
-                const int idx = q * LT + lt, r = idx >> 3, c = idx & 7;
-                const int64_t row = row0 + r;
-                g.s[q] = g.e[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (row < a.n_rows) {
-                    g.s[q] = ld_stream_f4(a.S + row * a.ld_in + a.in_off + hh * 32 + c * 4);
-                    g.e[q] = ld_stream_f4(a.E + row * a.ld_in + a.in_off + hh * 32 + c * 4);
-                }
-            }
-        };
-        auto convert = [&](const Stage& g, int i) {
-            const int hh = (i >> 1) % KBH, half_rows = (i & 1) * (TC_ROWS / 2);
-            const int kb1 = hh, kb2 = KBH + hh;
-#pragma unroll
-            for (int q = 0; q < QQ; ++q) {
-                const int idx = q * LT + lt, r = (idx >> 3) + half_rows, c = idx & 7;
-                const uint32_t off = sw128_offset(r, c);
-                const float4 sv = g.s[q], ev = g.e[q];
-                const float4 x1 = make_float4(sv.x + ev.x, sv.y + ev.y, sv.z + ev.z, sv.w + ev.w);
-                const float4 x2 = make_float4(sv.x * ev.x, sv.y * ev.y, sv.z * ev.z, sv.w * ev.w);
-                float4 hi, lo;
-                split_tf32_trunc(x1, hi, lo);
-                *reinterpret_cast<float4*>(A_hi + kb1 * TC_A_BLOCK + off) = hi;
-                *reinterpret_cast<float4*>(A_lo + kb1 * TC_A_BLOCK + off) = lo;
-                split_tf32_trunc(x2, hi, lo);
-                *reinterpret_cast<float4*>(A_hi + kb2 * TC_A_BLOCK + off) = hi;
-                *reinterpret_cast<float4*>(A_lo + kb2 * TC_A_BLOCK + off) = lo;
-            }
-        };
-        Stage g0, g1;
-        if (total_q > 0) issue(g0, 0);
-        for (int i = 0; i < total_q; i += 2) {                            // quarter i: rows 0..63 (g0), i + 1: rows 64..127 (g1)
-            const int it = i / (2 * KBH), hh = (i >> 1) % KBH;
-            const int kb1 = hh, kb2 = KBH + hh;
-            issue(g1, i + 1);
-            BWD_STAMP(2, it, hh * 3 + 0);
-            mbar_wait(&bars->empty[kb1], (it & 1) ^ 1);
-            mbar_wait(&bars->empty[kb2], (it & 1) ^ 1);
-            BWD_STAMP(2, it, hh * 3 + 1);
-            convert(g0, i);
-            if (i + 2 < total_q) issue(g0, i + 2);
-            convert(g1, i + 1);
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (lane == 0) {
-                mbar_arrive(&bars->full[kb1]);
-                mbar_arrive(&bars->full[kb2]);
-            }
-            BWD_STAMP(2, it, hh * 3 + 2);
-        }
-    }
-
-    tc_fence_before_sync();
-    __syncthreads();
-    if (dbg && lane == 0 && warp == 0) g_bwd_dbg[1][7][7] = clock64();
-    if (warp == FW_MMA_WARP) {
-        tc_fence_after_sync();
-        tmem_dealloc(tmem_base, 128);
-    }
-}
-
-
 // ====================================================================================================================
-// Round 2: the same forward with its S / E traffic on TMA.  ncu on the kernel above: 30 % of the HBM peak with nothing
-// saturated — four loader warps holding their loads in registers keep ~16 KB in flight per SM, a third of what Little's
-// law asks for.  Here ONE thread streams the tile's S and E blocks (128 rows x 32 columns, 16 KB each, 128-byte
-// swizzled by the tensor map = already in the UMMA K-major operand layout) into a raw shared-memory ring with
-// cp.async.bulk.tensor; four converter warps read a raw stage at the very byte offsets they then write (S+E and S*E,
-// split into TF32 hi / lo) in a two-slot operand ring; the MMA issuer and the epilogue are unchanged.  Up to 64 KB of
-// loads are in flight per SM whatever the converters do.
+// The forward with its S / E traffic on TMA.  ncu on round 1's version, whose four loader warps held their loads in
+// registers: 30 % of the HBM peak with nothing saturated — ~16 KB in flight per SM, a third of what Little's law asks
+// for.  Here ONE thread streams the tile's S and E blocks (128 rows x 32 columns, 16 KB each, 128-byte swizzled by the
+// tensor map = already in the UMMA K-major operand layout) into a raw shared-memory ring with cp.async.bulk.tensor;
+// four converter warps read a raw stage at the very byte offsets they then write (S+E and S*E, split into TF32 hi / lo)
+// in a two-slot operand ring.  Up to 64 KB of loads are in flight per SM whatever the converters do.
 //
 // Warp roles (448 threads): 0-7 epilogue, 8 MMA issuer + TMEM, 9 TMA producer (one lane), 10-13 converters.
 // ====================================================================================================================
@@ -1230,16 +1035,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) wgrad_tc_kernel(WgradArgs a) {
 
 }  // namespace
 
-// NGCF_B200_DENSE=tc_v1 selects the register-staged loaders of round 1 (A/B comparisons); default: TMA loaders
-static bool fwd_use_tma() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NGCF_B200_DENSE");
-        v = !(e && strcmp(e, "tc_v1") == 0);
-    }
-    return v == 1;
-}
-
 // widths up to 64 are one block; 128 is decomposed into 64-wide blocks of the same kernel (K halves accumulate through
 // the partial sums parked in E_out, N halves are independent)
 bool ngcf_dense_fwd_tc_eligible(int d_in, int d_out) {
@@ -1262,10 +1057,6 @@ int ngcf_dense_fwd_tc(const float* S, const float* E, int64_t n_rows, int d_in, 
         NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tma_kernel<MM_MULT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tma_kernel<MM_BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tma_kernel<MM_HASH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tc_kernel<MM_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tc_kernel<MM_MULT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tc_kernel<MM_BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-        NGCF_CUDA(cudaFuncSetAttribute(dense_fwd_tc_kernel<MM_HASH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         attr_set = true;
     }
     const int bk = d_in > 64 ? 64 : d_in, bn = d_out > 64 ? 64 : d_out;   // block widths
@@ -1273,22 +1064,17 @@ int ngcf_dense_fwd_tc(const float* S, const float* E, int64_t n_rows, int d_in, 
     const int n_tiles = (int)ceil_div64(n_rows, TC_ROWS);
     const int grid = (int)min((int64_t)n_tiles, (int64_t)ngcf_num_sms());
     const int KB = 2 * bk / 32;
-    const bool use_tma = fwd_use_tma();
-    const size_t smem_v1 = 1024 + (size_t)KB * (2 * TC_A_BLOCK + 2 * bn * 128) + 64 * sizeof(float) +
-                           FW_EPI_WARPS * 32 * 32 * sizeof(float) + sizeof(Bars);
-    const size_t smem_v2 = 1024 + (size_t)F2_RAW_STAGES * F2_RAW_BYTES + (size_t)F2_A_SLOTS * 2 * TC_A_BLOCK +
-                           (size_t)KB * 2 * bn * 128 + 64 * sizeof(float) + FW_EPI_WARPS * 32 * 32 * sizeof(float) +
-                           sizeof(Bars2);
+    const size_t smem = 1024 + (size_t)F2_RAW_STAGES * F2_RAW_BYTES + (size_t)F2_A_SLOTS * 2 * TC_A_BLOCK +
+                        (size_t)KB * 2 * bn * 128 + 64 * sizeof(float) + FW_EPI_WARPS * 32 * 32 * sizeof(float) +
+                        sizeof(Bars2);
     FwdTmaArgs p{};
-    if (use_tma) {
-        // S / E as [n_rows, d_in] fp32 with boxes of 128 rows x 32 columns, 128-byte swizzle; rows past the end read as 0
-        int rc = ngcf_encode_tmap_2d(&p.tmS, S, (uint64_t)n_rows, (uint64_t)d_in, (uint64_t)d_in, 32, TC_ROWS,
-                                     CU_TENSOR_MAP_SWIZZLE_128B);
-        if (rc == 0)
-            rc = ngcf_encode_tmap_2d(&p.tmE, E, (uint64_t)n_rows, (uint64_t)d_in, (uint64_t)d_in, 32, TC_ROWS,
-                                     CU_TENSOR_MAP_SWIZZLE_128B);
-        NGCF_REQUIRE(rc == 0, "dense_fwd: cuTensorMapEncodeTiled failed (%d)", rc);
-    }
+    // S / E as [n_rows, d_in] fp32 with boxes of 128 rows x 32 columns, 128-byte swizzle; rows past the end read as 0
+    int rc = ngcf_encode_tmap_2d(&p.tmS, S, (uint64_t)n_rows, (uint64_t)d_in, (uint64_t)d_in, 32, TC_ROWS,
+                                 CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc == 0)
+        rc = ngcf_encode_tmap_2d(&p.tmE, E, (uint64_t)n_rows, (uint64_t)d_in, (uint64_t)d_in, 32, TC_ROWS,
+                                 CU_TENSOR_MAP_SWIZZLE_128B);
+    NGCF_REQUIRE(rc == 0, "dense_fwd: cuTensorMapEncodeTiled failed (%d)", rc);
     for (int nh = 0; nh < NH; ++nh)
         for (int kh = 0; kh < KH; ++kh) {
             FwdTcArgs a{S, E, n_rows, bk, bn, wcat, bias_eff, slope, mess_mult, mess_bits, mess_p, seed, seed_dev, layer,
@@ -1298,24 +1084,14 @@ int ngcf_dense_fwd_tc(const float* S, const float* E, int64_t n_rows, int d_in, 
             a.out_off = nh * bn; a.d_out_full = d_out;
             a.mode = KH == 1 ? FW_SINGLE : (kh == 0 ? FW_PARTIAL : FW_FINAL);
             const int mm = a.mode == FW_PARTIAL ? MM_NONE : mess_mode(mess_mult, mess_bits, mess_p);
-            if (use_tma) {
-                p.b = a;
-                switch (mm) {
-                    case MM_NONE: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_NONE>, dim3(grid), dim3(F2_THREADS), smem_v2, st, p)); break;
-                    case MM_MULT: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_MULT>, dim3(grid), dim3(F2_THREADS), smem_v2, st, p)); break;
-                    case MM_BITS: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_BITS>, dim3(grid), dim3(F2_THREADS), smem_v2, st, p)); break;
-                    default: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_HASH>, dim3(grid), dim3(F2_THREADS), smem_v2, st, p)); break;
-                }
-                NGCF_LAUNCH_OK("dense_fwd_tma_kernel");
-                continue;
-            }
+            p.b = a;
             switch (mm) {
-                case MM_NONE: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tc_kernel<MM_NONE>, dim3(grid), dim3(TC_THREADS), smem_v1, st, a)); break;
-                case MM_MULT: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tc_kernel<MM_MULT>, dim3(grid), dim3(TC_THREADS), smem_v1, st, a)); break;
-                case MM_BITS: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tc_kernel<MM_BITS>, dim3(grid), dim3(TC_THREADS), smem_v1, st, a)); break;
-                default: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tc_kernel<MM_HASH>, dim3(grid), dim3(TC_THREADS), smem_v1, st, a)); break;
+                case MM_NONE: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_NONE>, dim3(grid), dim3(F2_THREADS), smem, st, p)); break;
+                case MM_MULT: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_MULT>, dim3(grid), dim3(F2_THREADS), smem, st, p)); break;
+                case MM_BITS: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_BITS>, dim3(grid), dim3(F2_THREADS), smem, st, p)); break;
+                default: NGCF_CUDA(ngcf_launch_pdl(dense_fwd_tma_kernel<MM_HASH>, dim3(grid), dim3(F2_THREADS), smem, st, p)); break;
             }
-            NGCF_LAUNCH_OK("dense_fwd_tc_kernel");
+            NGCF_LAUNCH_OK("dense_fwd_tma_kernel");
         }
     return NGCF_OK;
 }

@@ -9,9 +9,6 @@
 // that row (fence + counter).  (First version: hub pass and row pass as two launches, the row pass reading
 // hub_of_row[row] before every row - tools/spmm_timeline.py showed that dependent load plus the narrow tail batches as
 // 4-8 exposed round trips per 16-row tile, and the two launches each paid their own tail.)
-#include <stdlib.h>
-#include <string.h>
-
 #include "spmm_core.cuh"
 
 namespace {
@@ -608,16 +605,6 @@ __global__ void __launch_bounds__(CW_WARPS * 32) compact_kernel(CompactArgs a, i
     }
 }
 
-// NGCF_B200_SPMM=rows selects the row-per-warp kernel (A/B comparisons); default: the streaming kernel
-bool spmm_use_stream() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NGCF_B200_SPMM");
-        v = !(e && strcmp(e, "rows") == 0);
-    }
-    return v == 1;
-}
-
 template <int G>
 int launch(const SpmmArgs& a, int n_ctas, bool stream, cudaStream_t st) {
     if (n_ctas <= 0) return NGCF_OK;
@@ -693,8 +680,8 @@ extern "C" int ngcf_spmm(const ngcf_csr* g, const float* X, int64_t ldx, int d, 
                      (!addend || (aligned16(addend) && ld_add % 4 == 0)) &&
                      (!slot || (aligned16(gsum) && ld_gsum % 4 == 0)) && (g->n_hub == 0 || aligned16(hub_partial));
     const bool hubs = g->n_hub > 0 && g->n_chunks > 0;
-    // vector widths: the streaming kernel; NGCF_B200_SPMM=rows or any other width: the row-per-warp kernel
-    const bool stream_k = vec && spmm_use_stream() && (!hubs || (g->tile_hubmask && g->hub_rows));
+    // vector widths: the streaming kernel; any other width: the row-per-warp kernel
+    const bool stream_k = vec && (!hubs || (g->tile_hubmask && g->hub_rows));
     NGCF_REQUIRE(stream_k || !c_ent, "spmm: compacted survivor lists need the streaming kernel (width %% 4 == 0)");
     NGCF_REQUIRE(stream_k || !hubs || g->hub_done, "spmm: hub_done counters missing");
     SpmmArgs a{};

@@ -140,7 +140,6 @@ size_t ngcf_score_topk_tc_pack_bytes(int64_t n_users, int64_t n_items, int D);
 int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t n_items, int D, int k, int n_split,
                        float* pv, int* pi, uint8_t* pack, const int64_t* excl_ptr, const int32_t* excl_idx,
                        cudaStream_t st);
-bool ngcf_use_tensor_cores();
 
 extern "C" int ngcf_score_topk_workspace(int64_t n_users, int64_t n_items, int D, int k, size_t* bytes_host) {
     NGCF_REQUIRE(bytes_host, "score_topk_workspace: null pointer");
@@ -169,7 +168,7 @@ static int score_topk_impl(const float* U, int64_t n_users, const float* I, int6
         return NGCF_ERR_WORKSPACE;
     }
     cudaStream_t st = as_stream(stream);
-    if (ngcf_use_tensor_cores() && ngcf_score_topk_tc_eligible(n_users, n_items, D, k) &&
+    if (ngcf_score_topk_tc_eligible(n_users, n_items, D, k) &&
         (reinterpret_cast<uintptr_t>(U) & 15) == 0 && (reinterpret_cast<uintptr_t>(I) & 15) == 0) {
         // GEMM-shaped path on the tensor cores (topk_tc.cu); partial lists per item range, merged below
         const int ns = ngcf_score_topk_tc_splits(n_users, n_items);

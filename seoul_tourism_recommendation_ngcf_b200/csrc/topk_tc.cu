@@ -16,7 +16,6 @@
 // memory is added.
 #include <float.h>
 #include <limits.h>
-#include <stdlib.h>
 
 #include "tc.cuh"
 
@@ -43,7 +42,6 @@ struct ScoreTcArgs {
     int* pi;
     const int64_t* excl_ptr;   // kExclude: per user [excl_ptr[u], excl_ptr[u+1]) of excl_idx, ascending unique item ids
     const int32_t* excl_idx;
-    int dbg_skip_epilogue;     // timing experiments only (NGCF_B200_TOPK_SKIP_EPI=1): accumulators are read and dropped
 };
 
 struct ScoreBars {
@@ -97,7 +95,7 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
         // cost of a merge is paid once per warp, not once per user.  (First version: every survivor was merged at once —
         // 32 independent users per warp made nearly every score column an event: 11 of the kernel's 14 ms.)
         const int row = warp * 32 + lane;                                 // TMEM lane = user row of the tile
-        const bool live = u0 + row < a.n_users && !a.dbg_skip_epilogue;
+        const bool live = u0 + row < a.n_users;
         const int k = a.k;
         float thr = -FLT_MAX;                                             // k-th best as of the last merge
         int cnt = k;                                                      // next free slot
@@ -298,10 +296,8 @@ int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t 
         score_pack_kernel<<<(unsigned)ceil_div64(ci, 256), 256, 0, st>>>(I, n_items, D, KB, Ip, ci);
         NGCF_LAUNCH_OK("score_pack_kernel(I)");
     }
-    static int skip = -1;
-    if (skip < 0) { const char* e = getenv("NGCF_B200_TOPK_SKIP_EPI"); skip = (e && e[0] == '1') ? 1 : 0; }
     ScoreTcArgs a{Up, Ip, n_users, n_items, D, k, n_split, (int)((itiles + n_split - 1) / n_split), pv, pi, excl_ptr,
-                  excl_idx, skip};
+                  excl_idx};
     const size_t smem = 1024 + (size_t)ST_STAGES * ST_STAGE_BYTES + (size_t)(k + ST_EXTRA) * ST_ROWS * 8 + sizeof(ScoreBars);
     auto kern = excl_ptr ? score_topk_tc_kernel<true> : score_topk_tc_kernel<false>;
     NGCF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));   // per device

@@ -1,4 +1,4 @@
-"""Protocol timeline of CTA 0 of dense_fwd_tc_kernel (SM clocks), Gowalla-sized layer.  python tools/fwd_timeline.py [mess_p]"""
+"""Protocol timeline of CTA 0 of dense_fwd_tma_kernel (SM clocks), Gowalla-sized layer.  python tools/fwd_timeline.py [mess_p]"""
 import ctypes as C, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -26,19 +26,11 @@ flush.zero_(); run(); torch.cuda.synchronize()
 out = np.zeros(4 * 8 * 8, dtype=np.int64)
 raw.ngcf_debug_bwd_timeline(0, out.ctypes.data)
 t = out.reshape(4, 8, 8); t0 = t[0, 7, 7]
-if os.environ.get("NGCF_B200_DENSE") != "tc_v1":
-    print("dense_fwd_tma_kernel, CTA 0, SM cycles after the set-up barrier; kernel end =", t[1, 7, 7] - t0)
-    print(f"pdl_wait returned {t[0, 7, 6] - t0}; weights staged {t[0, 7, 5] - t0}")
-    for it in range(4):
-        print(f"tile {it}: producer got raw_empty " + " ".join(str(int(t[3, it, k] - t0)) for k in range(2)) +
-              " | converter " + " ".join(f"{n}={int(t[2, it, k] - t0)}" for k, n in enumerate(
-                  ["q0 raw_full", "q0 a_empty", "q0 done", "q1 raw_full", "q1 a_empty", "q1 done"])) +
-              " | mma tmem_empty=" + str(int(t[1, it, 0] - t0)) + " a_full " + " ".join(str(int(t[1, it, 1 + k] - t0)) for k in range(4)) +
-              " | epilogue " + " ".join(f"{n}={int(t[0, it, k] - t0)}" for k, n in enumerate(["wait", "tmem_full", "stored", "tmem read", "transposed"])))
-    sys.exit(0)
-
-print("cycles after the CTA's setup; total =", t[1, 7, 7] - t0)
+print("dense_fwd_tma_kernel, CTA 0, SM cycles after the set-up barrier; kernel end =", t[1, 7, 7] - t0)
+print(f"pdl_wait returned {t[0, 7, 6] - t0}; weights staged {t[0, 7, 5] - t0}")
 for it in range(4):
-    print(f"loader tile {it}: " + "  ".join(f"{n}={int(t[2, it, k] - t0)}" for k, n in enumerate(["h0 loaded", "h0 got empty", "h0 stored", "h1 loaded", "h1 got empty", "h1 stored"])))
-for it in range(4):
-    print(f"epilogue tile {it}: " + "  ".join(f"{n}={int(t[0, it, k] - t0)}" for k, n in enumerate(["wait", "got tmem_full", "stored"])))
+    print(f"tile {it}: producer got raw_empty " + " ".join(str(int(t[3, it, k] - t0)) for k in range(2)) +
+          " | converter " + " ".join(f"{n}={int(t[2, it, k] - t0)}" for k, n in enumerate(
+              ["q0 raw_full", "q0 a_empty", "q0 done", "q1 raw_full", "q1 a_empty", "q1 done"])) +
+          " | mma tmem_empty=" + str(int(t[1, it, 0] - t0)) + " a_full " + " ".join(str(int(t[1, it, 1 + k] - t0)) for k in range(4)) +
+          " | epilogue " + " ".join(f"{n}={int(t[0, it, k] - t0)}" for k, n in enumerate(["wait", "tmem_full", "stored", "tmem read", "transposed"])))

@@ -1,6 +1,6 @@
 """Accuracy audit at full Gowalla shape: every gradient of one training step (dropout off) from (a) this library,
 (b) the fp32 CPU oracle (= the reference's torch path), both measured against the float64 restatement.
-  python tools/grad_accuracy.py [shape]      (NGCF_B200_DENSE=ffma to audit the FFMA kernels)"""
+  python tools/grad_accuracy.py [shape]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np

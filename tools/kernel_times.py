@@ -54,6 +54,15 @@ t("node_dropout_bits (L and L^T)", lambda: node_dropout_bits(plan.fwd, 0.3, 1, N
 t("dense_fwd (mess_p 0.1)", lambda: lib.ngcf_dense_fwd(S.data_ptr(), X.data_ptr(), N, d, d, wcat.data_ptr(), bias.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, Y.data_ptr(), st))
 t("dense_fwd (no dropout)", lambda: lib.ngcf_dense_fwd(S.data_ptr(), X.data_ptr(), N, d, d, wcat.data_ptr(), bias.data_ptr(), 0.2, None, None, 0.0, 1, None, 0, 0, Y.data_ptr(), st))
 t("dense_bwd + wgrad (mess_p 0.1)", lambda: lib.ngcf_dense_bwd(gE.data_ptr(), slot.data_ptr(), gsum.data_ptr(), 4 * d, d, E_out.data_ptr(), S.data_ptr(), X.data_ptr(), N, d, d, W1.data_ptr(), W2.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, 1, gS.data_ptr(), gEl.data_ptr(), gW1.data_ptr(), gb1.data_ptr(), gW2.data_ptr(), gb2.data_ptr(), gM.data_ptr(), st))
-os.environ["NGCF_B200_DENSE"] = "ffma"
-t("dense_fwd FFMA (mess_p 0.1)", lambda: lib.ngcf_dense_fwd(S.data_ptr(), X.data_ptr(), N, d, d, wcat.data_ptr(), bias.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, Y.data_ptr(), st))
-t("dense_bwd FFMA (mess_p 0.1)", lambda: lib.ngcf_dense_bwd(gE.data_ptr(), slot.data_ptr(), gsum.data_ptr(), 4 * d, d, E_out.data_ptr(), S.data_ptr(), X.data_ptr(), N, d, d, W1.data_ptr(), W2.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, 1, gS.data_ptr(), gEl.data_ptr(), gW1.data_ptr(), gb1.data_ptr(), gW2.data_ptr(), gb2.data_ptr(), gM.data_ptr(), st))
+# the FFMA kernels: what runs at widths the tensor-core kernels do not take, such as the reference's own 65
+w = 65
+S6, X6, E6, gE6 = (torch.randn(N, w, device=dev) for _ in range(4))
+Y6, gS6, gEl6, gM6 = (torch.empty(N, w, device=dev) for _ in range(4))
+W1_6 = torch.randn(w, w, device=dev) * 0.1; W2_6 = torch.randn(w, w, device=dev) * 0.1
+b1_6 = torch.randn(w, device=dev); b2_6 = torch.randn(w, device=dev)
+wcat6 = torch.empty(2 * w * w, device=dev); bias6 = torch.empty(w, device=dev)
+lib.ngcf_pack_weights(W1_6.data_ptr(), b1_6.data_ptr(), W2_6.data_ptr(), b2_6.data_ptr(), w, w, wcat6.data_ptr(), bias6.data_ptr(), st)
+gW1_6 = torch.zeros(w, w, device=dev); gW2_6 = torch.zeros(w, w, device=dev); gb1_6 = torch.zeros(w, device=dev); gb2_6 = torch.zeros(w, device=dev)
+gsum6 = torch.randn(3000, 4 * w, device=dev)
+t("dense_fwd FFMA, width 65 (mess_p 0.1)", lambda: lib.ngcf_dense_fwd(S6.data_ptr(), X6.data_ptr(), N, w, w, wcat6.data_ptr(), bias6.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, Y6.data_ptr(), st))
+t("dense_bwd FFMA, width 65 (mess_p 0.1)", lambda: lib.ngcf_dense_bwd(gE6.data_ptr(), slot.data_ptr(), gsum6.data_ptr(), 4 * w, w, E6.data_ptr(), S6.data_ptr(), X6.data_ptr(), N, w, w, W1_6.data_ptr(), W2_6.data_ptr(), 0.2, None, None, 0.1, 1, None, 0, 0, 1, gS6.data_ptr(), gEl6.data_ptr(), gW1_6.data_ptr(), gb1_6.data_ptr(), gW2_6.data_ptr(), gb2_6.data_ptr(), gM6.data_ptr(), st))

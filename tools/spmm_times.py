@@ -28,7 +28,7 @@ def t(name, fn, reps=30):
         out[mode] = statistics.median(a.elapsed_time(b) for a, b in ev) * 1e3
     print(f"{name:44s} warm {out['warm']:8.1f} us   cold {out['cold']:8.1f} us", flush=True)
 
-tag = os.environ.get("NGCF_B200_LIB", "default").split("libngcf_")[-1] + " " + os.environ.get("NGCF_B200_SPMM", "stream")
+tag = os.environ.get("NGCF_B200_LIB", "default").split("libngcf_")[-1]
 print(f"== {tag}: tiles {plan.fwd.tiles.shape[0]} + {0 if plan.fwd.chunk_tiles is None else plan.fwd.chunk_tiles.shape[0]} chunk tiles, "
       f"tile {lib.ngcf_spmm_tile_rows()} rows / {lib.ngcf_spmm_tile_entries()} entries")
 t("spmm (no dropout)", lambda: spmm(plan.fwd, None, X, d, out=Y))
