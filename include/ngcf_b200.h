@@ -116,6 +116,8 @@ int ngcf_feature_mix(float* user_w, int64_t n_user, int d,
  * streaming kernel: it ADDS its row sums to Y after Y := addend (pass addend == Y to accumulate in place and
  * save the copy); other widths run the row-per-warp kernel.  The column word of an entry carries, above its 27-bit
  * column id, the index of the entry's row inside its tile (see plan.py).
+ *   ldx, ldy, ld_add, ld_gsum: row pitches in floats, ldx and ldy >= d; ldx < 2^30 (the gathers address rows of X
+ *               with a 32-bit byte stride).  An in-place addend (addend == Y) needs ld_add == ldy.
  *   slot/gsum : optional sparse row addend — if slot[i] >= 0, Y[i,:] += gsum[slot[i]*ld_gsum + 0..d)
  *               (the IndexBackward scatter of NGCF.py:151-155 folded into the last backward SpMM).
  *   drop_p > 0: device-RNG node dropout (NGCF.py:93-100,124-126) evaluated in-kernel: entry (r,c) of L survives

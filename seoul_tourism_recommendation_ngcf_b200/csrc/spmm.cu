@@ -665,7 +665,13 @@ extern "C" int ngcf_spmm(const ngcf_csr* g, const float* X, int64_t ldx, int d, 
     if (rc != NGCF_OK) return rc;
     NGCF_REQUIRE(X && Y, "spmm: null pointer");
     NGCF_REQUIRE(d > 0 && d <= NGCF_MAX_WIDTH, "spmm: width %d not in [1,%d]", d, NGCF_MAX_WIDTH);
-    NGCF_REQUIRE(ldx >= d && ldy >= d && ldx < ((int64_t)1 << 31), "spmm: bad leading dimension");
+    NGCF_REQUIRE(ldx >= d && ldy >= d, "spmm: leading dimension below the width %d (ldx %lld, ldy %lld)", d,
+                 (long long)ldx, (long long)ldy);
+    // the vector gathers address X rows with a 32-bit byte stride (one IMAD.WIDE.U32 per gathered row)
+    NGCF_REQUIRE(ldx < ((int64_t)1 << 30), "spmm: ldx %lld must be below 2^30 (byte stride ldx * 4 < 2^32)",
+                 (long long)ldx);
+    NGCF_REQUIRE(addend != Y || ld_add == ldy, "spmm: an in-place addend (addend == Y) needs ld_add == ldy (%lld != %lld)",
+                 (long long)ld_add, (long long)ldy);
     NGCF_REQUIRE(drop_p >= 0.f && drop_p < 1.f, "spmm: drop_p %f not in [0,1)", drop_p);
     NGCF_REQUIRE(layer >= 0 && layer < NGCF_MAX_LAYERS, "spmm: layer %d", layer);
     NGCF_REQUIRE(row_offset >= 0 && row_offset < ((int64_t)1 << 31), "spmm: row_offset %lld", (long long)row_offset);
