@@ -364,6 +364,23 @@ int ngcf_sample_negatives(const int32_t* pos_ptr, const int32_t* pos_idx, const 
                           const int64_t* candidates, int n_candidates, int ng_ratio, uint64_t seed, int64_t* out,
                           int32_t* n_short, void* stream);
 
+/* ---- dynamic hard-negative sampling (DNS): the negative of each training row chosen on the device ----------------------
+ * Layers / dims / n_layers_plus1 as ngcf_gather_concat takes them (E_0..E_K, [N, d_k] each, N = n_user + n_items).  For
+ * batch row b of user u = u_id[b]: the user's final row is built as ngcf_gather_concat builds it (E_0 raw, blocks k >= 1
+ * divided by max(||E_k row||, 1e-12)); then M candidates j = 0..M-1 are drawn with replacement, uniformly over the items
+ * outside u's exclusion list excl_idx[excl_ptr[u] .. excl_ptr[u+1]) (ascending, unique item ids; excl_idx may be NULL
+ * when every list is empty):  h = hash64(seed + *seed_dev, b, b >> 32, j, 'HNEG'),  r = (h.x * n_free) >> 32,
+ * item = the r-th item not in the list.  Each candidate is scored as the dot product of the two final rows, and
+ * chosen[b] = the candidate of largest |score| (ties: lowest j), an item id without the n_user offset.  |score| because
+ * the BPR loss compares |u.p| with |u.n| (ngcf_bpr_fwd_bwd).  Every user in u_id must have a free item (n_free >= 1);
+ * the caller checks that once (a row without one gets chosen = -1).  cand [batch, M] (int64) and score [batch, M]
+ * (fp32) are optional debug outputs.  1 <= M <= 64, n_items < 2^31.  Allocates nothing, never synchronises
+ * (capturable; seed_dev optional, as for dropout). */
+int ngcf_hard_negatives(const float* const* layers_host, const int* dims_host, int n_layers_plus1, int64_t n_user,
+                        const int64_t* u_id, int64_t batch, const int64_t* excl_ptr /*[n_user+1]*/,
+                        const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
+                        int64_t* chosen /*[batch]*/, int64_t* cand, float* score, void* stream);
+
 /* ---- Laplacian builder on the device: matrix.py:41-62 restricted to the non-zeros (SURVEY.md section 8(f) #2) ----------
  * From n_pairs DISTINCT (user, item, rating != 0) pairs: deg[N] = number of non-zeros per row of A = [[0,R],[R^T,0]]
  * (matrix.py:55), then the 2*n_pairs entries of L = D^-1/2 A D^-1/2 (matrix.py:56-62): entry e -> (user, n_user+item),

@@ -18,6 +18,7 @@ import torch.distributed as dist
 
 from . import _lib
 from .plan import LaplacianPlan, node_dropout_bits, node_dropout_compact, spmm
+from .sampler import HardNegatives
 from .sharded import RowShards, all_gather_rows
 
 LEAKY_SLOPE = 0.2   # NGCF.py:140
@@ -30,7 +31,7 @@ def _stream() -> int:
 class _Ctx:
     """Per-forward state shared by the autograd node and the module (layer activations, plan, masks)."""
     __slots__ = ("plan", "E", "S", "dims", "vals_f", "vals_b", "mess_mult", "mess_p", "seed", "seed_dev", "masked", "drop_p", "bits_f", "bits_b", "comp_f", "comp_b", "mess_bits",
-                 "rows", "offsets", "W1", "W2", "fresh_key", "node_mode", "last_partial", "fm_stream")
+                 "rows", "offsets", "W1", "W2", "fresh_key", "node_mode", "last_partial", "fm_stream", "hneg")
 
 
 def _capturing() -> bool:
@@ -148,7 +149,14 @@ class _Propagate(torch.autograd.Function):
             st.E.append(Xn)
         D = sum(st.dims)
         layers, dims = _lib.ptr_array(st.E), _lib.int_array(st.dims)
-        outs = [torch.empty(st.rows[j].numel(), D, dtype=torch.float32, device=dev) for j in range(n_sets)]
+        if st.hneg is not None:                                        # dynamic hard negatives: fills st.rows[2]
+            hn, train, chosen, cand, score = st.hneg
+            _lib.check(lib.ngcf_hard_negatives(layers, dims, K + 1, mod.n_user, st.rows[0].data_ptr(),
+                                               st.rows[0].numel(), train.ptr.data_ptr(), _lib.ptr(train.idx),
+                                               mod.n_item, hn.n_candidates, st.seed, _lib.ptr(st.seed_dev),
+                                               chosen.data_ptr(), _lib.ptr(cand), _lib.ptr(score), _stream()),
+                       "hard_negatives")
+        outs =[torch.empty(st.rows[j].numel(), D, dtype=torch.float32, device=dev) for j in range(n_sets)]
         _lib.check(lib.ngcf_gather_concat_sets(layers, dims, K + 1, _lib.ptr_array(st.rows[:n_sets]),
                                                _lib.i64_array(st.offsets[:n_sets]),
                                                _lib.i64_array([r.numel() for r in st.rows[:n_sets]]), _lib.ptr_array(outs),
@@ -303,6 +311,9 @@ class NGCF(nn.Module):
     snapshot : False (default) keeps E_0 = the live parameter table (zero copy); a second forward or an optimizer step
           before ``backward()`` / before reading ``all_users_emb`` then raises.  True copies the table per forward, which
           is what the reference's ``torch.cat`` (NGCF.py:120) does, and lifts that restriction.
+
+    ``forward(..., neg_item=HardNegatives(...), ...)`` chooses each row's negative on the device from that forward's
+    own layer outputs (sampler.HardNegatives); the picks are then ``neg_item.chosen``.
     """
 
     def __init__(self, embed_size: int, layer_size: list, node_dropout: float, mess_dropout: list,
@@ -499,8 +510,19 @@ class NGCF(nn.Module):
 
         u_id, pos_item = ix(u_id), ix(pos_item)
         feats_idx = [ix(age), ix(sex), ix(month), ix(day), ix(dow)]          # concat order, NGCF.py:110
-        has_neg = len(neg_item) > 0                                          # NGCF.py:154
-        neg_item = ix(neg_item) if has_neg else None
+        hneg = neg_item if isinstance(neg_item, HardNegatives) else None
+        if hneg is not None:
+            if self._shard is not None:
+                raise ValueError("HardNegatives: not available on a row-sharded model (the candidates' rows of the "
+                                 "last layer are spread over the ranks)")
+            if hneg.train.n_rows != self.n_user or hneg.train.n_items != self.n_item:
+                raise ValueError(f"HardNegatives: train has {hneg.train.n_rows} rows over {hneg.train.n_items} items; "
+                                 f"the model has {self.n_user} users and {self.n_item} items")
+            has_neg = True
+            neg_item = torch.empty(u_id.numel(), dtype=torch.int64, device=dev)   # written by ngcf_hard_negatives
+        else:
+            has_neg = len(neg_item) > 0                                      # NGCF.py:154
+            neg_item = ix(neg_item) if has_neg else None
         year_idx = int(year.min()) % 18                                      # == year.unique()[0] % 18, NGCF.py:117
 
         table = self._packed_table()
@@ -561,7 +583,9 @@ class NGCF(nn.Module):
             st.mess_p = [float(p) for p in self.mess_dropout[:K]]
         # per-forward RNG key from torch's CPU generator (reproducible under torch.manual_seed); drawn only when
         # a device-RNG stream is live and only after the reference-mode mask draws, whose RNG stream it must not shift
-        need_seed = st.drop_p > 0 or any(p > 0 for p in st.mess_p)
+        # (the hard-negative draws take the same seed: with dropout on, a forward with HardNegatives and one without draw
+        # the same key from the generator and so the same dropout masks)
+        need_seed = st.drop_p > 0 or any(p > 0 for p in st.mess_p) or hneg is not None
         if not need_seed:
             st.seed = 0
         elif self.rng == "reference":
@@ -577,6 +601,13 @@ class NGCF(nn.Module):
             st.vals_b = [plan.entries(plan.bwd, masks[k]) for k in range(K)]
         st.rows = [u_id, pos_item] + ([neg_item] if has_neg else [])
         st.offsets = [0, self.n_user] + ([self.n_user] if has_neg else [])
+        st.hneg = None
+        if hneg is not None:
+            M = hneg.n_candidates
+            st.hneg = (hneg, hneg._on(dev), neg_item,
+                       torch.empty(u_id.numel(), M, dtype=torch.int64, device=dev) if hneg.debug else None,
+                       torch.empty(u_id.numel(), M, dtype=torch.float32, device=dev) if hneg.debug else None)
+            hneg.chosen, hneg.cand, hneg.score = st.hneg[2:]
 
         wb = [l.weight for l in self.w1_list] + [l.bias for l in self.w1_list] + \
              [l.weight for l in self.w2_list] + [l.bias for l in self.w2_list]

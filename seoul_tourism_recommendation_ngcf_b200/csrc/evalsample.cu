@@ -5,6 +5,8 @@
 //                           distinct items the user has no positive feedback for, uniformly, without replacement.
 //   * ngcf_laplacian_entries — the non-zeros of L = D^-1/2 A D^-1/2 from the rating pairs (matrix.py:41-62),
 //                           section 8(f) #2.
+//   * ngcf_hard_negatives  — dynamic hard-negative sampling inside a training step: per batch row, M free items
+//                           scored against the user with the current layer outputs, the hardest one kept.
 // All are small latency/HBM-bound integer + dot-product kernels; no tensor cores.
 #include <limits.h>
 
@@ -170,6 +172,126 @@ sample_negatives_kernel(const int32_t* __restrict__ pos_ptr, const int32_t* __re
     }
 }
 
+// ---- dynamic hard negatives (DNS) -------------------------------------------------------------------------------------
+constexpr int HN_WARPS = 4;                              // rows per CTA
+constexpr int HN_MAX_M = 64;                             // candidates per row
+constexpr int HN_GROUP = 4;                              // candidates scored together (loads in flight per lane)
+constexpr int HN_Q = NGCF_MAX_WIDTH / 32;                // columns per lane of one layer block
+#define NGCF_STREAM_HNEG 0x484e4547u                     // 'HNEG'
+
+struct HardNegArgs {
+    const float* layer[NGCF_MAX_LAYERS + 1];
+    int dim[NGCF_MAX_LAYERS + 1];
+    int n;
+    int64_t n_user;
+    const int64_t* u_id;
+    int64_t batch;
+    const int64_t* excl_ptr;
+    const int32_t* excl_idx;
+    int n_items;
+    int M;
+    uint64_t seed;
+    const uint64_t* seed_dev;
+    int64_t* chosen;
+    int64_t* cand;
+    float* score;
+};
+
+// One warp per batch row.  The user's final row (gather_row's formula: E_0 raw, E_k / max(||E_k||, 1e-12)) stays in
+// registers; M candidates are drawn with replacement, uniformly over the items outside the user's exclusion list (lane
+// l draws j = l and l + 32), and scored HN_GROUP at a time against the candidates' final rows, whose layer blocks are
+// normalised on the fly.  Only the B*M candidate rows of E_0..E_K are read.
+__global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegArgs a) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t row = (int64_t)blockIdx.x * HN_WARPS + warp;
+    if (row >= a.batch) return;
+    const int64_t usr = a.u_id[row];
+    float ur[NGCF_MAX_LAYERS + 1][HN_Q];
+#pragma unroll
+    for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+        if (k < a.n) {
+            const int d = a.dim[k];
+            const float* src = a.layer[k] + usr * (int64_t)d;
+            float ss = 0.f;
+#pragma unroll
+            for (int q = 0; q < HN_Q; ++q) {
+                const int c = lane + 32 * q;
+                ur[k][q] = c < d ? src[c] : 0.f;
+                ss = fmaf(ur[k][q], ur[k][q], ss);
+            }
+            if (k > 0) {
+                const float scale = 1.f / fmaxf(sqrtf(warp_sum(ss)), 1e-12f);   // F.normalize, NGCF.py:144
+#pragma unroll
+                for (int q = 0; q < HN_Q; ++q) ur[k][q] *= scale;
+            }
+        }
+    }
+    const int64_t p0 = a.excl_ptr[usr];
+    const int deg = (int)(a.excl_ptr[usr + 1] - p0);
+    const int n_free = a.n_items - deg;                  // >= 1: checked by the caller (HardNegatives)
+    const uint64_t seed = ngcf_seed(a.seed, a.seed_dev);
+    int item[2] = {-1, -1};
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int j = lane + 32 * h;
+        if (j < a.M && n_free > 0) {
+            const uint2 x = ngcf_hash64(seed, (uint32_t)row, (uint32_t)(row >> 32), (uint32_t)j, NGCF_STREAM_HNEG);
+            const int r = (int)(((uint64_t)x.x * (uint64_t)n_free) >> 32);              // uniform in [0, n_free)
+            item[h] = nth_free(a.excl_idx + p0, deg, r);
+        }
+    }
+    // The loss is logsigmoid(|u.p| - |u.n|) (bprloss.py:18, bpr_kernel): a negative is hardest when its score is
+    // largest in ABSOLUTE value, so the pick is the candidate of largest |score|, ties to the lowest j.
+    float best = -1.f;
+    int best_item = __shfl_sync(FULL_MASK, item[0], 0);
+    for (int j0 = 0; j0 < a.M; j0 += HN_GROUP) {
+        int it[HN_GROUP];
+#pragma unroll
+        for (int g = 0; g < HN_GROUP; ++g) {
+            const int j = j0 + g < a.M ? j0 + g : j0;   // a short last group repeats its first candidate
+            it[g] = __shfl_sync(FULL_MASK, j < 32 ? item[0] : item[1], j & 31);
+        }
+        float sc[HN_GROUP] = {};
+#pragma unroll
+        for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+            if (k < a.n) {
+                const int d = a.dim[k];
+                float v[HN_GROUP][HN_Q];
+#pragma unroll
+                for (int g = 0; g < HN_GROUP; ++g) {
+                    const float* src = a.layer[k] + (a.n_user + it[g]) * (int64_t)d;
+#pragma unroll
+                    for (int q = 0; q < HN_Q; ++q) {
+                        const int c = lane + 32 * q;
+                        v[g][q] = c < d ? src[c] : 0.f;
+                    }
+                }
+#pragma unroll
+                for (int g = 0; g < HN_GROUP; ++g) {
+                    float dot = 0.f, ss = 0.f;
+#pragma unroll
+                    for (int q = 0; q < HN_Q; ++q) {
+                        dot = fmaf(ur[k][q], v[g][q], dot);
+                        ss = fmaf(v[g][q], v[g][q], ss);
+                    }
+                    dot = warp_sum(dot);
+                    sc[g] += k > 0 ? dot / fmaxf(sqrtf(warp_sum(ss)), 1e-12f) : dot;
+                }
+            }
+        }
+#pragma unroll
+        for (int g = 0; g < HN_GROUP; ++g) {
+            const int j = j0 + g;
+            if (j < a.M) {
+                if (fabsf(sc[g]) > best) { best = fabsf(sc[g]); best_item = it[g]; }
+                if (lane == 0 && a.cand) a.cand[row * a.M + j] = it[g];
+                if (lane == 0 && a.score) a.score[row * a.M + j] = sc[g];
+            }
+        }
+    }
+    if (lane == 0) a.chosen[row] = best_item;
+}
+
 // ---- Laplacian entries from the rating pairs (matrix.py:41-62, restricted to the non-zeros) ------------------------
 __global__ void lap_degree_kernel(const int64_t* __restrict__ user, const int64_t* __restrict__ item, int64_t n_pairs,
                                   int64_t n_user, int32_t* __restrict__ deg) {
@@ -256,5 +378,35 @@ extern "C" int ngcf_sample_negatives(const int32_t* pos_ptr, const int32_t* pos_
     sample_negatives_kernel<<<(unsigned)ceil_div64(n_rows, 128), 128, 0, as_stream(stream)>>>(
         pos_ptr, pos_idx, row_user, n_rows, candidates, n_candidates, ng_ratio, seed, out, n_short);
     NGCF_LAUNCH_OK("sample_negatives_kernel");
+    return NGCF_OK;
+}
+
+extern "C" int ngcf_hard_negatives(const float* const* layers_host, const int* dims_host, int n_layers_plus1,
+                                   int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                                   const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
+                                   const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
+                                   void* stream) {
+    NGCF_REQUIRE(layers_host && dims_host, "hard_negatives: null layer array");
+    NGCF_REQUIRE(n_layers_plus1 >= 1 && n_layers_plus1 <= NGCF_MAX_LAYERS + 1, "hard_negatives: %d blocks",
+                 n_layers_plus1);
+    HardNegArgs a{};
+    for (int k = 0; k < n_layers_plus1; ++k) {
+        NGCF_REQUIRE(layers_host[k] && dims_host[k] > 0 && dims_host[k] <= NGCF_MAX_WIDTH, "hard_negatives: bad block %d",
+                     k);
+        a.layer[k] = layers_host[k];
+        a.dim[k] = dims_host[k];
+    }
+    NGCF_REQUIRE(n_user > 0, "hard_negatives: n_user %lld", (long long)n_user);
+    NGCF_REQUIRE(n_items >= 1 && n_items <= INT_MAX, "hard_negatives: n_items %lld not in [1, 2^31-1]",
+                 (long long)n_items);
+    NGCF_REQUIRE(M >= 1 && M <= HN_MAX_M, "hard_negatives: M %d outside [1, %d]", M, HN_MAX_M);
+    NGCF_REQUIRE(batch >= 0, "hard_negatives: batch %lld", (long long)batch);
+    NGCF_REQUIRE(batch == 0 || (u_id && excl_ptr && chosen), "hard_negatives: null pointer");
+    a.n = n_layers_plus1; a.n_user = n_user; a.u_id = u_id; a.batch = batch; a.excl_ptr = excl_ptr;
+    a.excl_idx = excl_idx; a.n_items = (int)n_items; a.M = M; a.seed = seed; a.seed_dev = seed_dev;
+    a.chosen = chosen; a.cand = cand; a.score = score;
+    if (batch == 0) return NGCF_OK;
+    hard_negatives_kernel<<<(unsigned)ceil_div64(batch, HN_WARPS), HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    NGCF_LAUNCH_OK("hard_negatives_kernel");
     return NGCF_OK;
 }

@@ -20,22 +20,28 @@ class GraphedStep:
     """``step = GraphedStep(model, criterion, batch_size); loss = step(batch)`` with ``batch`` a dict of int64
     tensors (host or device) holding ``year`` plus the eight index fields of ``TourDataset`` (utils.py:167-275).
     ``year`` must be a host tensor (it selects ``lap_list[year.min() % 18]`` on the host, NGCF.py:117); one graph is
-    kept per selected Laplacian.  ``node_flag`` / train-vs-eval mode are frozen at capture time."""
+    kept per selected Laplacian.  ``node_flag`` / train-vs-eval mode are frozen at capture time.
 
-    def __init__(self, model, criterion, batch_size: int, node_flag: bool = True, warmup: int = 1, optimizer=None):
+    ``negatives``: a ``HardNegatives``; each replay then chooses every row's negative on the device, from fresh
+    candidates, and batches carry no ``neg_item``.  After each call ``negatives.chosen`` holds that step's picks."""
+
+    def __init__(self, model, criterion, batch_size: int, node_flag: bool = True, warmup: int = 1, optimizer=None,
+                 negatives=None):
         dev = model.user_embedding.weight.device
         if dev.type != "cuda":
             raise RuntimeError("GraphedStep needs the model on a CUDA device")
         self.model, self.criterion, self.node_flag, self.warmup = model, criterion, bool(node_flag), int(warmup)
         self.B = int(batch_size)
+        self.negatives = negatives
+        self.fields = FIELDS[:-1] if negatives is not None else FIELDS
         # optional ngcf_b200.Adam: its step (and the zeroing of the gradients for the next batch, experiment.py:55,58)
         # joins the graph, so a replay is the reference's whole training iteration
         self.optimizer = optimizer
-        self.static_idx = torch.zeros(len(FIELDS), self.B, dtype=torch.int64, device=dev)
+        self.static_idx = torch.zeros(len(self.fields), self.B, dtype=torch.int64, device=dev)
         # pinned staging buffers for host batches, rotated: the H2D copy below is asynchronous, so a buffer may only be
         # rewritten once the copy that read it has run (its event); with one buffer a host running ahead of the GPU
         # would overwrite a batch that is still waiting to be copied
-        self.stages = [torch.zeros(len(FIELDS), self.B, dtype=torch.int64).pin_memory() for _ in range(3)]
+        self.stages = [torch.zeros(len(self.fields), self.B, dtype=torch.int64).pin_memory() for _ in range(3)]
         self.stage_events = [None] * len(self.stages)
         self._stage_i = 0
         self.seed_dev = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -44,9 +50,10 @@ class GraphedStep:
 
     def _run(self, year, with_optimizer: bool = True):
         m = self.model
-        f = {k: self.static_idx[i] for i, k in enumerate(FIELDS)}
+        f = {k: self.static_idx[i] for i, k in enumerate(self.fields)}
+        neg = self.negatives if self.negatives is not None else f["neg_item"]
         u, p, n = m(year=year, u_id=f["u_id"], age=f["age"], sex=f["sex"], month=f["month"], day=f["day"], dow=f["dow"],
-                    pos_item=f["pos_item"], neg_item=f["neg_item"], node_flag=self.node_flag)
+                    pos_item=f["pos_item"], neg_item=neg, node_flag=self.node_flag)
         loss = self.criterion(u, p, n)
         loss.backward()
         if self.optimizer is not None and with_optimizer:
@@ -84,7 +91,9 @@ class GraphedStep:
         year = batch["year"]
         if year.device.type != "cpu":
             raise ValueError("GraphedStep: pass `year` as a host tensor (it is only used to pick lap_list[year % 18])")
-        on_host = [batch[k].device.type == "cpu" for k in FIELDS]
+        if self.negatives is not None and "neg_item" in batch:
+            raise ValueError("GraphedStep: built with negatives=, so the batch must not carry neg_item")
+        on_host = [batch[k].device.type == "cpu" for k in self.fields]
         stage = None
         if any(on_host):
             j = self._stage_i
@@ -92,7 +101,7 @@ class GraphedStep:
             if self.stage_events[j] is not None:
                 self.stage_events[j].synchronize()                    # the copy that last read this buffer has run
             stage = self.stages[j]
-        for i, k in enumerate(FIELDS):
+        for i, k in enumerate(self.fields):
             t = batch[k]
             if t.numel() != self.B:
                 raise ValueError(f"GraphedStep was built for batches of {self.B} rows, got {t.numel()} for {k}")
@@ -101,7 +110,7 @@ class GraphedStep:
         if all(on_host):
             self.static_idx.copy_(stage, non_blocking=True)           # one pinned H2D copy for the whole batch
         else:
-            for i, k in enumerate(FIELDS):
+            for i, k in enumerate(self.fields):
                 self.static_idx[i].copy_(stage[i] if on_host[i] else batch[k], non_blocking=True)
         if stage is not None:
             if self.stage_events[j] is None:
@@ -114,6 +123,8 @@ class GraphedStep:
         g, loss, grads, last = entry
         g.replay()
         self.model._last, self.model._all_E = last, None              # all_users_emb / all_items_emb: rebuild on read
+        if last.hneg is not None:                                     # this graph's output buffers of the picks
+            last.hneg[0].chosen, last.hneg[0].cand, last.hneg[0].score = last.hneg[2:]
         if self.optimizer is not None:
             from . import _lib
             _lib.bump_param_epoch()                                   # the replay stepped the parameters

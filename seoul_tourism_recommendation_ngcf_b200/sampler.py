@@ -113,3 +113,41 @@ class TourDataset(torch.utils.data.Dataset):
             users = np.repeat(users, ng_ratio + 1, axis=0)                       # [R*25, 8] (utils.py:249-266)
             items = torch.cat((pos[:, None], neg), dim=1).reshape(-1)            # [R*25]: positive, then its negatives
         return torch.from_numpy(users).reshape(-1, 7 if self.train else 8), items
+
+
+class HardNegatives:
+    """Dynamic hard-negative sampling (DNS): pass as ``neg_item=`` to ``NGCF.forward`` (or ``negatives=`` to
+    ``GraphedStep``) and each batch row's negative is chosen on the device, inside the step, from ``n_candidates``
+    items drawn uniformly (with replacement) among those the user has no ``train`` interaction with: the candidate
+    whose final embedding row has the largest |dot product| with the user's, under the layer outputs of that same
+    forward.  ``train``: an :class:`Interactions` with one row per user, e.g. ``Interactions.from_pairs(users, items,
+    n_item, rows=torch.arange(n_user))``.  After each forward ``chosen`` (int64 [B], item ids) holds the picks; with
+    ``debug=True`` also ``cand`` (int64 [B, n_candidates]) and ``score`` (fp32 [B, n_candidates])."""
+
+    MAX_CANDIDATES = 64                  # ngcf_hard_negatives: M <= 64
+
+    def __init__(self, train, n_candidates: int = 32, *, debug: bool = False):
+        from .scoring import Interactions
+        if not isinstance(train, Interactions):
+            raise TypeError("HardNegatives: train must be an Interactions (Interactions.from_pairs)")
+        n_candidates = int(n_candidates)
+        if not 1 <= n_candidates <= self.MAX_CANDIDATES:
+            raise ValueError(f"HardNegatives: n_candidates {n_candidates} not in [1, {self.MAX_CANDIDATES}]")
+        deg = train.ptr.detach().cpu().diff()
+        if deg.numel() and int(deg.max()) >= train.n_items:
+            # the kernel draws from the items outside the row's list and has no way to report an empty set
+            u = int(torch.nonzero(deg >= train.n_items)[0])
+            raise ValueError(f"HardNegatives: row {u} lists all {train.n_items} items; it has no negative to draw")
+        self.train, self.n_candidates, self.debug = train, n_candidates, bool(debug)
+        self.chosen = self.cand = self.score = None
+        self._dev = {}
+
+    def _on(self, device):
+        """``train`` on ``device``, copied once (a forward under CUDA-graph capture must not copy from the host)."""
+        t = self._dev.get(device)
+        if t is None:
+            t = self._dev[device] = self.train.to(device)
+        return t
+
+    def __repr__(self):
+        return f"HardNegatives({self.train!r}, n_candidates={self.n_candidates})"
