@@ -381,6 +381,30 @@ int ngcf_hard_negatives(const float* const* layers_host, const int* dims_host, i
                         const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
                         int64_t* chosen /*[batch]*/, int64_t* cand, float* score, void* stream);
 
+/* Same draws, but chosen[b] = the candidate of largest SIGNED score (ties: lowest j): the hard negative of a softmax
+ * loss (ngcf_softmax_loss), where a large negative score is an easy negative.  Same arguments and rules. */
+int ngcf_hard_negatives_signed(const float* const* layers_host, const int* dims_host, int n_layers_plus1,
+                               int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                               const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
+                               int64_t* chosen, int64_t* cand, float* score, void* stream);
+
+/* ---- in-batch sampled-softmax (InfoNCE) loss with its row gradients ---------------------------------------------------
+ * u, p: [batch, D] fp32; n: [batch, D] or NULL (no explicit negatives).  Columns c_j = p_j (j < batch), then
+ * c_{batch+j} = n_j; logits s_ij = u_i.c_j / temperature.  With item ids (pos_ids [batch], and neg_ids [batch] when n is
+ * given; both NULL: no masking) column j is masked for row i iff j != i and id(c_j) == pos_ids[i]; repeated items
+ * are not de-duplicated.
+ *   loss[0] = (1/batch_size) sum_i [ logsumexp_{unmasked j} s_ij - s_ii + weight_decay (|u_i|^2 + |p_i|^2 + |n_i|^2) ]
+ * and, when gu / gp (/ gn with n) are given, its gradients with respect to u, p and n (all NULL: forward only).
+ * 1 <= batch <= 4096, 1 <= D <= 1152, temperature > 0, weight_decay >= 0, batch_size > 0.  The three products run on
+ * the tensor cores (3xTF32); no atomics, the loss is summed in a fixed order in double: two calls on the same inputs
+ * give the same bits.  workspace: ngcf_softmax_loss_workspace bytes for n_cols = batch (no n) or 2 * batch (a short
+ * one: NGCF_ERR_WORKSPACE).  Allocates nothing, never synchronises (capturable). */
+int ngcf_softmax_loss_workspace(int64_t batch, int n_cols, int D, size_t* bytes_host);
+int ngcf_softmax_loss(const float* u, const float* p, const float* n, int64_t batch, int D, const int64_t* pos_ids,
+                      const int64_t* neg_ids, float temperature, float weight_decay, float batch_size,
+                      float* loss /*[1]*/, float* gu, float* gp, float* gn, void* workspace, size_t workspace_bytes,
+                      void* stream);
+
 /* ---- Laplacian builder on the device: matrix.py:41-62 restricted to the non-zeros (SURVEY.md section 8(f) #2) ----------
  * From n_pairs DISTINCT (user, item, rating != 0) pairs: deg[N] = number of non-zeros per row of A = [[0,R],[R^T,0]]
  * (matrix.py:55), then the 2*n_pairs entries of L = D^-1/2 A D^-1/2 (matrix.py:56-62): entry e -> (user, n_user+item),

@@ -151,10 +151,11 @@ class _Propagate(torch.autograd.Function):
         layers, dims = _lib.ptr_array(st.E), _lib.int_array(st.dims)
         if st.hneg is not None:                                        # dynamic hard negatives: fills st.rows[2]
             hn, train, chosen, cand, score = st.hneg
-            _lib.check(lib.ngcf_hard_negatives(layers, dims, K + 1, mod.n_user, st.rows[0].data_ptr(),
-                                               st.rows[0].numel(), train.ptr.data_ptr(), _lib.ptr(train.idx),
-                                               mod.n_item, hn.n_candidates, st.seed, _lib.ptr(st.seed_dev),
-                                               chosen.data_ptr(), _lib.ptr(cand), _lib.ptr(score), _stream()),
+            pick = lib.ngcf_hard_negatives_signed if hn.signed else lib.ngcf_hard_negatives
+            _lib.check(pick(layers, dims, K + 1, mod.n_user, st.rows[0].data_ptr(),
+                            st.rows[0].numel(), train.ptr.data_ptr(), _lib.ptr(train.idx),
+                            mod.n_item, hn.n_candidates, st.seed, _lib.ptr(st.seed_dev),
+                            chosen.data_ptr(), _lib.ptr(cand), _lib.ptr(score), _stream()),
                        "hard_negatives")
         outs =[torch.empty(st.rows[j].numel(), D, dtype=torch.float32, device=dev) for j in range(n_sets)]
         _lib.check(lib.ngcf_gather_concat_sets(layers, dims, K + 1, _lib.ptr_array(st.rows[:n_sets]),

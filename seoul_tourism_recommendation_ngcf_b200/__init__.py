@@ -6,6 +6,8 @@ from .graph import GraphedStep
 from .optim import Adam
 from .sampler import HardNegatives, TourDataset, sample_negatives
 from .scoring import Interactions, full_rank_eval, rank_metrics, score_topk
+from .softmax_loss import SoftmaxLoss
 
 __all__ = ["NGCF", "BPR", "GraphedStep", "Adam", "score_topk", "Experiment", "eval_groups", "TourDataset",
-           "sample_negatives", "Interactions", "full_rank_eval", "rank_metrics", "HardNegatives"]
+           "sample_negatives", "Interactions", "full_rank_eval", "rank_metrics", "HardNegatives",
+           "SoftmaxLoss"]

@@ -75,6 +75,10 @@ SIGNATURES = {
     "ngcf_sample_negatives": [_vp, _vp, _vp, _i64, _vp, C.c_int, C.c_int, _u64, _vp, _vp, _vp],
     "ngcf_hard_negatives": [C.POINTER(_vp), C.POINTER(C.c_int), C.c_int, _i64, _vp, _i64, _vp, _vp, _i64, C.c_int, _u64,
                             _vp, _vp, _vp, _vp, _vp],
+    "ngcf_hard_negatives_signed": [C.POINTER(_vp), C.POINTER(C.c_int), C.c_int, _i64, _vp, _i64, _vp, _vp, _i64, C.c_int,
+                                   _u64, _vp, _vp, _vp, _vp, _vp],
+    "ngcf_softmax_loss_workspace": [_i64, C.c_int, C.c_int, C.POINTER(_sz)],
+    "ngcf_softmax_loss": [_vp, _vp, _vp, _i64, C.c_int, _vp, _vp, _f32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _sz, _vp],
     "ngcf_laplacian_entries": [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp],
     "ngcf_plgraph_entries": [_i64, _i64, _i64, C.c_double, _u64, _i64, _i64, _vp, _vp, _i64, _vp],
     "ngcf_build_tiles": [_vp, _i64, C.c_int, C.c_int, _vp, _vp, _i64, _vp, _vp],

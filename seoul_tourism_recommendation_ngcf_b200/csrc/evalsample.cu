@@ -201,6 +201,8 @@ struct HardNegArgs {
 // registers; M candidates are drawn with replacement, uniformly over the items outside the user's exclusion list (lane
 // l draws j = l and l + 32), and scored HN_GROUP at a time against the candidates' final rows, whose layer blocks are
 // normalised on the fly.  Only the B*M candidate rows of E_0..E_K are read.
+// kSigned: the pick is the largest signed score instead (the hard negative of a softmax loss).
+template <bool kSigned>
 __global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegArgs a) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * HN_WARPS + warp;
@@ -242,7 +244,7 @@ __global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegAr
     }
     // The loss is logsigmoid(|u.p| - |u.n|) (bprloss.py:18, bpr_kernel): a negative is hardest when its score is
     // largest in ABSOLUTE value, so the pick is the candidate of largest |score|, ties to the lowest j.
-    float best = -1.f;
+    float best = kSigned ? -INFINITY : -1.f;
     int best_item = __shfl_sync(FULL_MASK, item[0], 0);
     for (int j0 = 0; j0 < a.M; j0 += HN_GROUP) {
         int it[HN_GROUP];
@@ -283,7 +285,8 @@ __global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegAr
         for (int g = 0; g < HN_GROUP; ++g) {
             const int j = j0 + g;
             if (j < a.M) {
-                if (fabsf(sc[g]) > best) { best = fabsf(sc[g]); best_item = it[g]; }
+                const float key = kSigned ? sc[g] : fabsf(sc[g]);
+                if (key > best) { best = key; best_item = it[g]; }
                 if (lane == 0 && a.cand) a.cand[row * a.M + j] = it[g];
                 if (lane == 0 && a.score) a.score[row * a.M + j] = sc[g];
             }
@@ -381,11 +384,10 @@ extern "C" int ngcf_sample_negatives(const int32_t* pos_ptr, const int32_t* pos_
     return NGCF_OK;
 }
 
-extern "C" int ngcf_hard_negatives(const float* const* layers_host, const int* dims_host, int n_layers_plus1,
-                                   int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
-                                   const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
-                                   const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
-                                   void* stream) {
+static int hard_negatives(bool is_signed, const float* const* layers_host, const int* dims_host, int n_layers_plus1,
+                          int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                          const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
+                          int64_t* chosen, int64_t* cand, float* score, void* stream) {
     NGCF_REQUIRE(layers_host && dims_host, "hard_negatives: null layer array");
     NGCF_REQUIRE(n_layers_plus1 >= 1 && n_layers_plus1 <= NGCF_MAX_LAYERS + 1, "hard_negatives: %d blocks",
                  n_layers_plus1);
@@ -406,7 +408,29 @@ extern "C" int ngcf_hard_negatives(const float* const* layers_host, const int* d
     a.excl_idx = excl_idx; a.n_items = (int)n_items; a.M = M; a.seed = seed; a.seed_dev = seed_dev;
     a.chosen = chosen; a.cand = cand; a.score = score;
     if (batch == 0) return NGCF_OK;
-    hard_negatives_kernel<<<(unsigned)ceil_div64(batch, HN_WARPS), HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    const unsigned grid = (unsigned)ceil_div64(batch, HN_WARPS);
+    if (is_signed)
+        hard_negatives_kernel<true><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    else
+        hard_negatives_kernel<false><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
     NGCF_LAUNCH_OK("hard_negatives_kernel");
     return NGCF_OK;
+}
+
+extern "C" int ngcf_hard_negatives(const float* const* layers_host, const int* dims_host, int n_layers_plus1,
+                                   int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                                   const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
+                                   const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
+                                   void* stream) {
+    return hard_negatives(false, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
+                          n_items, M, seed, seed_dev, chosen, cand, score, stream);
+}
+
+extern "C" int ngcf_hard_negatives_signed(const float* const* layers_host, const int* dims_host, int n_layers_plus1,
+                                          int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                                          const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
+                                          const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
+                                          void* stream) {
+    return hard_negatives(true, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
+                          n_items, M, seed, seed_dev, chosen, cand, score, stream);
 }

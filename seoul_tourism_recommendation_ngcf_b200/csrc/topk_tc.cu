@@ -17,19 +17,11 @@
 #include <float.h>
 #include <limits.h>
 
-#include "tc.cuh"
+#include "tc_gemm.cuh"
 
 namespace {
 
-using namespace tc;
-
-constexpr int ST_ROWS = 128;                   // users per tile (UMMA M) and items per tile (UMMA N)
-constexpr int ST_EPI_WARPS = 4;
-constexpr int ST_THREADS = (ST_EPI_WARPS + 2) * 32;                       // + MMA warp + producer warp
-constexpr int ST_STAGES = 2;
 constexpr int ST_EXTRA = 64;                    // appended-but-not-yet-merged entries a user's list can hold
-constexpr int ST_BLOCK = ST_ROWS * 128;        // bytes of one 32-column K block of A or B (hi or lo)
-constexpr int ST_STAGE_BYTES = 4 * ST_BLOCK;   // A hi, A lo, B hi, B lo
 constexpr int ST_MAXK = 32;
 
 struct ScoreTcArgs {
@@ -44,11 +36,6 @@ struct ScoreTcArgs {
     const int32_t* excl_idx;
 };
 
-struct ScoreBars {
-    uint64_t full[ST_STAGES], empty[ST_STAGES], tmem_full[2], tmem_empty[2];
-    uint32_t tmem_base;
-};
-
 // kExclude: items on the user's exclusion list never enter its lists (the false instantiation reads no list at all)
 template <bool kExclude>
 __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArgs a) {
@@ -59,7 +46,7 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
     float* lv = reinterpret_cast<float*>(ring + ST_STAGES * ST_STAGE_BYTES);   // [k + ST_EXTRA][128]: user lists, slot-major
     const int cap = a.k + ST_EXTRA;
     int* li = reinterpret_cast<int*>(lv + cap * ST_ROWS);
-    ScoreBars* bars = reinterpret_cast<ScoreBars*>(li + cap * ST_ROWS);
+    GemmBars* bars = reinterpret_cast<GemmBars*>(li + cap * ST_ROWS);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int ut = blockIdx.x, sp = blockIdx.y;
@@ -69,23 +56,8 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
     const int n_t = max(0, t1 - t0);
     const int KB = (a.D + 31) / 32;
 
-    if (tid == 0) {
-        for (int i = 0; i < ST_STAGES; ++i) {
-            mbar_init(&bars->full[i], 1);                               // the producer's arrive.expect_tx; TMA completes the bytes
-            mbar_init(&bars->empty[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&bars->tmem_full[i], 1);
-            mbar_init(&bars->tmem_empty[i], ST_EPI_WARPS);
-        }
-        fence_mbar_init();
-    }
-    if (warp == ST_EPI_WARPS) tmem_alloc(&bars->tmem_base, 256);          // 2 accumulators x 128 fp32 columns
     for (int i = tid; i < a.k * ST_ROWS; i += ST_THREADS) { lv[i] = -FLT_MAX; li[i] = 0x7fffffff; }   // the k kept slots
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem_base = bars->tmem_base;
+    const uint32_t tmem_base = gemm_setup(bars, warp);
 
     if (warp < ST_EPI_WARPS) {
         // ======================= epilogue: per-user top-k ==========================================================
@@ -176,86 +148,11 @@ __global__ void __launch_bounds__(ST_THREADS, 1) score_topk_tc_kernel(ScoreTcArg
             for (int j = 0; j < k; ++j) { ov[j] = lv[j * ST_ROWS + row]; oi[j] = li[j * ST_ROWS + row]; }
         }
     } else if (warp == ST_EPI_WARPS) {
-        // ======================= MMA issuer =====================================================================
-        const uint32_t idesc = umma_idesc_tf32(ST_ROWS, ST_ROWS, 0, 0);
-        int step = 0;
-        for (int it = 0; it < n_t; ++it) {
-            const int buf = it & 1;
-            mbar_wait(&bars->tmem_empty[buf], ((it >> 1) & 1) ^ 1);
-            tc_fence_after_sync();
-            const uint32_t tmem_d = tmem_base + buf * ST_ROWS;
-            for (int kb = 0; kb < KB; ++kb, ++step) {
-                const int stg = step % ST_STAGES;
-                mbar_wait(&bars->full[stg], (step / ST_STAGES) & 1);
-                tc_fence_after_sync();
-                if (lane == 0) {
-                    const uint32_t a_hi = smem_u32(ring + stg * ST_STAGE_BYTES), a_lo = a_hi + ST_BLOCK;
-                    const uint32_t b_hi = a_lo + ST_BLOCK, b_lo = b_hi + ST_BLOCK;
-#pragma unroll
-                    for (int k8 = 0; k8 < 4; ++k8) {                      // 4 x (K = 8 TF32 = 32 bytes) per block
-                        const uint64_t dah = umma_desc_sw128(a_hi + k8 * 32, 16, 1024);
-                        const uint64_t dal = umma_desc_sw128(a_lo + k8 * 32, 16, 1024);
-                        const uint64_t dbh = umma_desc_sw128(b_hi + k8 * 32, 16, 1024);
-                        const uint64_t dbl = umma_desc_sw128(b_lo + k8 * 32, 16, 1024);
-                        umma_tf32(tmem_d, dah, dbh, idesc, (kb | k8) ? 1u : 0u);
-                        umma_tf32(tmem_d, dal, dbh, idesc, 1);
-                        umma_tf32(tmem_d, dah, dbl, idesc, 1);
-                    }
-                    umma_commit(&bars->empty[stg]);                       // the stage may be refilled
-                }
-                __syncwarp();
-            }
-            if (lane == 0) umma_commit(&bars->tmem_full[buf]);            // accumulator complete
-            __syncwarp();
-        }
-    } else {
-        // ======================= producer: two 32-KB bulk copies per K step ========================================
-        if (lane == 0) {
-            const int total = n_t * KB;
-            for (int s = 0; s < total; ++s) {
-                const int it = s / KB, kb = s - it * KB, stg = s % ST_STAGES;
-                mbar_wait(&bars->empty[stg], ((s / ST_STAGES) & 1) ^ 1);  // the MMAs that read this stage are done
-                const uint32_t dst = smem_u32(ring + stg * ST_STAGE_BYTES), bar = smem_u32(&bars->full[stg]);
-                const uint8_t* srcA = a.Up + ((size_t)ut * KB + kb) * (2 * ST_BLOCK);
-                const uint8_t* srcB = a.Ip + ((size_t)(t0 + it) * KB + kb) * (2 * ST_BLOCK);
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(ST_STAGE_BYTES) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(dst), "l"(srcA), "r"(2 * ST_BLOCK), "r"(bar) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             ::"r"(dst + 2 * ST_BLOCK), "l"(srcB), "r"(2 * ST_BLOCK), "r"(bar) : "memory");
-            }
-        }
+        gemm_issue(n_t, KB, ring, bars, tmem_base, lane);
+    } else if (lane == 0) {
+        gemm_produce(a.Up, a.Ip, ut, t0, n_t, KB, ring, bars);
     }
-
-    tc_fence_before_sync();
-    __syncthreads();
-    if (warp == ST_EPI_WARPS) {
-        tc_fence_after_sync();
-        tmem_dealloc(tmem_base, 256);
-    }
-}
-
-// X [n, D] row-major fp32 -> operand blocks: for row tile t and K block kb, a 16-KB hi image followed by a 16-KB lo image
-// of the 128-byte-swizzled K-major layout (rows / columns past the end are zero).  hi = x (the tensor core truncates to
-// TF32), lo = x - trunc(x).
-__global__ void __launch_bounds__(256) score_pack_kernel(const float* __restrict__ X, int64_t n, int D, int KB,
-                                                         uint8_t* __restrict__ out, int64_t n_chunks) {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;     // one 16-byte chunk each
-    if (i >= n_chunks) return;
-    const int c = (int)(i & 7);
-    const int64_t rk = i >> 3;                                            // (tile, kb, row) with row fastest ... no: row-major source
-    const int kb = (int)(rk % KB);
-    const int64_t row = rk / KB;
-    const int col = kb * 32 + c * 4;
-    float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (row < n && col < D) x = ld_f4(X + row * D + col);
-    float4 hi, lo;
-    split_tf32_trunc(x, hi, lo);
-    const int64_t t = row / ST_ROWS;
-    const uint32_t off = sw128_offset((uint32_t)(row % ST_ROWS), (uint32_t)c);
-    uint8_t* blk = out + ((size_t)t * KB + kb) * (2 * ST_BLOCK);
-    *reinterpret_cast<float4*>(blk + off) = hi;
-    *reinterpret_cast<float4*>(blk + ST_BLOCK + off) = lo;
+    gemm_teardown(tmem_base, warp);
 }
 
 }  // namespace
@@ -289,16 +186,12 @@ int ngcf_score_topk_tc(const float* U, int64_t n_users, const float* I, int64_t 
     const int64_t ut = (n_users + ST_ROWS - 1) / ST_ROWS, itiles = (n_items + ST_ROWS - 1) / ST_ROWS;
     uint8_t* Up = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(pack) + 1023) & ~(uintptr_t)1023);
     uint8_t* Ip = Up + (size_t)ut * KB * 2 * ST_BLOCK;
-    {
-        const int64_t cu = ut * ST_ROWS * KB * 8, ci = itiles * ST_ROWS * KB * 8;
-        score_pack_kernel<<<(unsigned)ceil_div64(cu, 256), 256, 0, st>>>(U, n_users, D, KB, Up, cu);
-        NGCF_LAUNCH_OK("score_pack_kernel(U)");
-        score_pack_kernel<<<(unsigned)ceil_div64(ci, 256), 256, 0, st>>>(I, n_items, D, KB, Ip, ci);
-        NGCF_LAUNCH_OK("score_pack_kernel(I)");
-    }
+    int rc = gemm_pack<false>(false, U, n_users, D, D, KB, 0, KB, Up, st);
+    if (rc == NGCF_OK) rc = gemm_pack<false>(false, I, n_items, D, D, KB, 0, KB, Ip, st);
+    if (rc != NGCF_OK) return rc;
     ScoreTcArgs a{Up, Ip, n_users, n_items, D, k, n_split, (int)((itiles + n_split - 1) / n_split), pv, pi, excl_ptr,
                   excl_idx};
-    const size_t smem = 1024 + (size_t)ST_STAGES * ST_STAGE_BYTES + (size_t)(k + ST_EXTRA) * ST_ROWS * 8 + sizeof(ScoreBars);
+    const size_t smem = 1024 + (size_t)ST_STAGES * ST_STAGE_BYTES + (size_t)(k + ST_EXTRA) * ST_ROWS * 8 + sizeof(GemmBars);
     auto kern = excl_ptr ? score_topk_tc_kernel<true> : score_topk_tc_kernel<false>;
     NGCF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));   // per device
     dim3 grid((unsigned)ut, (unsigned)n_split);

@@ -18,6 +18,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
+from .softmax_loss import SoftmaxLoss
 
 
 @_lib.on_device
@@ -103,7 +104,12 @@ class Experiment(nn.Module):
                     u, p, n = self.model(year=year, u_id=u_id, age=age, sex=sex, month=month, day=day, dow=dow,
                                          pos_item=pos_item, neg_item=neg_item, node_flag=True)
                     self.optimizer.zero_grad()
-                    loss = self.criterion(u, p, n)
+                    if isinstance(self.criterion, SoftmaxLoss):         # item ids mask the batch's false negatives
+                        dev = u.device
+                        neg_ids = neg_item.to(dev, torch.int64) if n.numel() else None
+                        loss = self.criterion(u, p, n, pos_item.to(dev, torch.int64), neg_ids)
+                    else:
+                        loss = self.criterion(u, p, n)
                     loss.backward()
                     self.optimizer.step()
                 total_loss += loss.detach()

@@ -13,6 +13,8 @@ from __future__ import annotations
 
 import torch
 
+from .softmax_loss import SoftmaxLoss
+
 FIELDS = ("u_id", "age", "sex", "month", "day", "dow", "pos_item", "neg_item")
 
 
@@ -54,7 +56,13 @@ class GraphedStep:
         neg = self.negatives if self.negatives is not None else f["neg_item"]
         u, p, n = m(year=year, u_id=f["u_id"], age=f["age"], sex=f["sex"], month=f["month"], day=f["day"], dow=f["dow"],
                     pos_item=f["pos_item"], neg_item=neg, node_flag=self.node_flag)
-        loss = self.criterion(u, p, n)
+        if isinstance(self.criterion, SoftmaxLoss):
+            # the batch's item ids mask false negatives; under capture these are the static index rows (or the
+            # HardNegatives picks), so every replay masks with its own batch's ids
+            rows = m._last.rows
+            loss = self.criterion(u, p, n, rows[1], rows[2] if len(rows) > 2 else None)
+        else:
+            loss = self.criterion(u, p, n)
         loss.backward()
         if self.optimizer is not None and with_optimizer:
             self.optimizer.step()         # (a replay overwrites every gradient buffer, so nothing needs zeroing)

@@ -122,11 +122,14 @@ class HardNegatives:
     whose final embedding row has the largest |dot product| with the user's, under the layer outputs of that same
     forward.  ``train``: an :class:`Interactions` with one row per user, e.g. ``Interactions.from_pairs(users, items,
     n_item, rows=torch.arange(n_user))``.  After each forward ``chosen`` (int64 [B], item ids) holds the picks; with
-    ``debug=True`` also ``cand`` (int64 [B, n_candidates]) and ``score`` (fp32 [B, n_candidates])."""
+    ``debug=True`` also ``cand`` (int64 [B, n_candidates]) and ``score`` (fp32 [B, n_candidates]).
+
+    ``signed=True`` picks the candidate of largest signed score instead, for :class:`SoftmaxLoss`: there a large
+    negative score is an easy negative, while BPR's loss compares |u.p| with |u.n|."""
 
     MAX_CANDIDATES = 64                  # ngcf_hard_negatives: M <= 64
 
-    def __init__(self, train, n_candidates: int = 32, *, debug: bool = False):
+    def __init__(self, train, n_candidates: int = 32, *, signed: bool = False, debug: bool = False):
         from .scoring import Interactions
         if not isinstance(train, Interactions):
             raise TypeError("HardNegatives: train must be an Interactions (Interactions.from_pairs)")
@@ -138,7 +141,7 @@ class HardNegatives:
             # the kernel draws from the items outside the row's list and has no way to report an empty set
             u = int(torch.nonzero(deg >= train.n_items)[0])
             raise ValueError(f"HardNegatives: row {u} lists all {train.n_items} items; it has no negative to draw")
-        self.train, self.n_candidates, self.debug = train, n_candidates, bool(debug)
+        self.train, self.n_candidates, self.signed, self.debug = train, n_candidates, bool(signed), bool(debug)
         self.chosen = self.cand = self.score = None
         self._dev = {}
 
