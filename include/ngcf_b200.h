@@ -236,6 +236,25 @@ int ngcf_gather_concat_sets(const float* const* layers_host, const int* dims_hos
                             const int64_t* const* rows_host, const int64_t* offsets_host, const int64_t* sizes_host,
                             float* const* outs_host, int n_sets, int64_t ld_out, void* stream);
 
+/* ---- LightGCN readout and its backward (lightgcn.py) -----------------------------------------------------------------
+ * ngcf_layer_mean: out[b, :] = (E_0[r, :] + E_1[r, :] + ... + E_K[r, :]) * (1/(K+1)), summed in that order in fp32,
+ * r = rows[b] + row_offset (rows == NULL: r = b + row_offset, i.e. all_users_emb / all_items_emb).  layers_host: K+1
+ * device pointers to contiguous [N, d] layers, 1 <= d <= NGCF_MAX_WIDTH; out is [n_out, ld_out], ld_out >= d.
+ * ngcf_layer_mean_sets: the same for up to four row sets at once (users / positives / negatives of a batch): set j
+ * gathers rows rows_host[j][i] + offsets_host[j] into outs_host[j] ([sizes_host[j], ld_out]). */
+int ngcf_layer_mean(const float* const* layers_host, int n_layers_plus1, int d, const int64_t* rows, int64_t row_offset,
+                    int64_t n_out, float* out, int64_t ld_out, void* stream);
+int ngcf_layer_mean_sets(const float* const* layers_host, int n_layers_plus1, int d, const int64_t* const* rows_host,
+                         const int64_t* offsets_host, const int64_t* sizes_host, float* const* outs_host, int n_sets,
+                         int64_t ld_out, void* stream);
+/* The dense gradient of the last layer from a slot map (ngcf_rowgrad_scatter's slot / gsum):
+ *   out[i, :] = slot[i] >= 0 ? scale * gsum[slot[i], :] : 0      for i < n_rows, and gsum[slot[i], :] *= scale in place,
+ * so that ngcf_spmm's slot/gsum addend then adds the same scaled rows (LightGCN: scale = 1/(K+1), the readout's
+ * weight).  Every slot must belong to one row only, as ngcf_rowgrad_scatter leaves them.  n_rows < 2^31,
+ * 1 <= d <= NGCF_MAX_WIDTH, ld_gsum and ld_out >= d (row pitches in floats). */
+int ngcf_rowgrad_expand(const int32_t* slot, int64_t n_rows, float* gsum, int64_t ld_gsum, int d, float scale,
+                        float* out, int64_t ld_out, void* stream);
+
 /* ---- BPR loss: bprloss.py:15-22, forward and row gradients in one kernel ------------------------------
  * loss = (-sum_b logsigmoid(|u_b.p_b| - |u_b.n_b|)
  *         + wd (reg_w_u sum|u_b|^2 + reg_w_p sum|p_b|^2 + reg_w_n sum|n_b|^2)) / batch_size_ctor  -> *loss (device)
@@ -387,6 +406,14 @@ int ngcf_hard_negatives_signed(const float* const* layers_host, const int* dims_
                                int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
                                const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
                                int64_t* chosen, int64_t* cand, float* score, void* stream);
+
+/* Same draws and picks (signed_pick != 0: the largest signed score, else the largest |score|) on LightGCN's final rows:
+ * the layer mean (E_0 + ... + E_K) / (K+1) of n_layers_plus1 layers of width d each, summed in ngcf_layer_mean's order,
+ * for the user and for every candidate.  Other arguments and rules as ngcf_hard_negatives; 1 <= d <= NGCF_MAX_WIDTH. */
+int ngcf_hard_negatives_mean(const float* const* layers_host, int d, int n_layers_plus1, int64_t n_user,
+                             const int64_t* u_id, int64_t batch, const int64_t* excl_ptr, const int32_t* excl_idx,
+                             int64_t n_items, int M, int signed_pick, uint64_t seed, const uint64_t* seed_dev,
+                             int64_t* chosen, int64_t* cand, float* score, void* stream);
 
 /* ---- in-batch sampled-softmax (InfoNCE) loss with its row gradients ---------------------------------------------------
  * u, p: [batch, D] fp32; n: [batch, D] or NULL (no explicit negatives).  Columns c_j = p_j (j < batch), then

@@ -303,7 +303,66 @@ class _Propagate(torch.autograd.Function):
         return (None, None, None, gU, gI, *gW1, *gb1, *gW2, *gb2)
 
 
-class NGCF(nn.Module):
+def draw_seed(generator=None) -> int:
+    """A per-forward device-RNG key from ``generator`` (default: torch's CPU generator, so ``torch.manual_seed``
+    reproduces it)."""
+    return int(torch.randint(0, 2 ** 62, (1,), generator=generator).item())
+
+
+class _TableModel(nn.Module):
+    """What NGCF and LightGCN share: E_0 of a forward is the live packed [N, d] table behind ``user_embedding`` and
+    ``item_embedding`` (no copy), one execution plan per ``lap_list`` element, the row-gradient slot map, and the rule
+    that refuses to use a forward's E_0 once the table changed under it.  Subclasses set n_user, n_item, emb_size,
+    lap_list, _plans, _table, _slot, _shard, _snapshot and _mix_count, and name themselves in _NAME."""
+    _STALE_ADVICE = "Run the forward again."
+
+    def _packed_table(self) -> torch.Tensor:
+        """[N, d] view over user_embedding.weight and item_embedding.weight laid out back to back, so that
+        ``cat(user, item)`` (NGCF.py:120) costs nothing.  Re-packs (and rebinds both ``.data``) whenever the
+        two parameters are not adjacent, e.g. after ``model.to(device)`` or ``load_state_dict``."""
+        u, i = self.user_embedding.weight, self.item_embedding.weight
+        d = self.emb_size
+        adjacent = (u.is_contiguous() and i.is_contiguous() and u.dtype == torch.float32 and
+                    u.data_ptr() + self.n_user * d * 4 == i.data_ptr() and
+                    getattr(self, "_table", None) is not None and self._table.data_ptr() == u.data_ptr())
+        if not adjacent:
+            n_rows = self._shard.N_pad if self._shard is not None else self.n_user + self.n_item
+            table = torch.zeros(n_rows, d, dtype=torch.float32, device=u.device)   # rows past N: shard padding
+            table[:self.n_user].copy_(u.data)
+            table[self.n_user:self.n_user + self.n_item].copy_(i.data)
+            u.data = table[:self.n_user]
+            i.data = table[self.n_user:self.n_user + self.n_item]
+            self._table = table
+        return self._table if self._shard is None else self._table   # [N_pad, d] when sharded (pad rows are zero)
+
+    def _slot_map(self, N, dev):
+        if self._slot is None or self._slot.device != dev or self._slot.numel() != N:
+            self._slot = torch.full((N,), -1, dtype=torch.int32, device=dev)
+        return self._slot
+
+    def _plan(self, year_idx: int, dev) -> LaplacianPlan:
+        L = self.lap_list[year_idx]
+        p = self._plans.get(year_idx)
+        if p is None or p.src is not L or p.coo_val.device != dev:
+            p = LaplacianPlan(L, dev, shard=self._shard)
+            self._plans[year_idx] = p
+        return p
+
+    def _fresh_key(self):
+        return (self._mix_count, _lib.param_epoch(), self.user_embedding.weight._version,
+                self.item_embedding.weight._version)
+
+    def _check_fresh(self, st, what: str):
+        """E_0 of a forward is the live table (see __init__): refuse to use it once something changed the table."""
+        if self._snapshot or st.fresh_key == self._fresh_key():
+            return
+        why = "the step that produced it also ran the optimizer" if st.fresh_key is None else \
+            "another forward (feature mix) or an optimizer step ran since"
+        raise RuntimeError(f"{self._NAME} (B200): {what} needs the embedding table as the forward left it, but {why}. "
+                           + self._STALE_ADVICE)
+
+
+class NGCF(_TableModel):
     """Same surface as the reference ``NGCF`` (NGCF.py:8-17).  Extra keyword-only knobs:
 
     rng : "device" (default) draws node- and message-dropout decisions in-kernel from a counter-based hash stream keyed
@@ -316,6 +375,9 @@ class NGCF(nn.Module):
     ``forward(..., neg_item=HardNegatives(...), ...)`` chooses each row's negative on the device from that forward's
     own layer outputs (sampler.HardNegatives); the picks are then ``neg_item.chosen``.
     """
+    _NAME = "NGCF"
+    _STALE_ADVICE = ("Run the forward again, or construct the module with snapshot=True to keep a per-forward copy like "
+                     "the reference's torch.cat (NGCF.py:120).")
 
     def __init__(self, embed_size: int, layer_size: list, node_dropout: float, mess_dropout: list,
                  emb_ratio: float, lap_list: list, num_dict: dict, batch_size: int, device, *, rng: str = "device",
@@ -448,38 +510,6 @@ class NGCF(nn.Module):
         return "equal row blocks, per-layer NCCL all-gather of E / gS, all-reduce of W/b grads"
 
     # ---- internal buffers ---------------------------------------------------------------------------
-    def _packed_table(self) -> torch.Tensor:
-        """[N, d] view over user_embedding.weight and item_embedding.weight laid out back to back, so that
-        ``cat(user, item)`` (NGCF.py:120) costs nothing.  Re-packs (and rebinds both ``.data``) whenever the
-        two parameters are not adjacent, e.g. after ``model.to(device)`` or ``load_state_dict``."""
-        u, i = self.user_embedding.weight, self.item_embedding.weight
-        d = self.emb_size
-        adjacent = (u.is_contiguous() and i.is_contiguous() and u.dtype == torch.float32 and
-                    u.data_ptr() + self.n_user * d * 4 == i.data_ptr() and
-                    getattr(self, "_table", None) is not None and self._table.data_ptr() == u.data_ptr())
-        if not adjacent:
-            n_rows = self._shard.N_pad if self._shard is not None else self.n_user + self.n_item
-            table = torch.zeros(n_rows, d, dtype=torch.float32, device=u.device)   # rows past N: shard padding
-            table[:self.n_user].copy_(u.data)
-            table[self.n_user:self.n_user + self.n_item].copy_(i.data)
-            u.data = table[:self.n_user]
-            i.data = table[self.n_user:self.n_user + self.n_item]
-            self._table = table
-        return self._table if self._shard is None else self._table   # [N_pad, d] when sharded (pad rows are zero)
-
-    def _slot_map(self, N, dev):
-        if self._slot is None or self._slot.device != dev or self._slot.numel() != N:
-            self._slot = torch.full((N,), -1, dtype=torch.int32, device=dev)
-        return self._slot
-
-    def _plan(self, year_idx: int, dev) -> LaplacianPlan:
-        L = self.lap_list[year_idx]
-        p = self._plans.get(year_idx)
-        if p is None or p.src is not L or p.coo_val.device != dev:
-            p = LaplacianPlan(L, dev, shard=self._shard)
-            self._plans[year_idx] = p
-        return p
-
     def _reference_node_masks(self, nnz: int, dev):
         """Bit-exact reproduction of NGCF.sparse_dropout's host RNG stream (NGCF.py:94): float64 ones through a
         fresh (always-training) nn.Dropout on the CPU generator, over the surviving entries only."""
@@ -592,9 +622,9 @@ class NGCF(nn.Module):
         elif self.rng == "reference":
             if self._seed_gen is None:
                 self._seed_gen = torch.Generator().manual_seed(torch.initial_seed() & (2 ** 63 - 1))
-            st.seed = int(torch.randint(0, 2 ** 62, (1,), generator=self._seed_gen).item())
+            st.seed = draw_seed(self._seed_gen)
         else:
-            st.seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+            st.seed = draw_seed()
         # CUDA-graph mode (graph.GraphedStep): the launches are frozen, so the per-step key comes from a device counter
         st.seed_dev = self._seed_dev if need_seed else None
         if masks is not None:
@@ -619,20 +649,6 @@ class NGCF(nn.Module):
         return u_embeddings, pos_i_embeddings, neg_i_embeddings
 
     # ---- attributes the reference sets in forward (NGCF.py:147-149), materialised on first read ---------
-    def _fresh_key(self):
-        return (self._mix_count, _lib.param_epoch(), self.user_embedding.weight._version,
-                self.item_embedding.weight._version)
-
-    def _check_fresh(self, st, what: str):
-        """E_0 of a forward is the live table (see __init__): refuse to use it once something changed the table."""
-        if self._snapshot or st.fresh_key == self._fresh_key():
-            return
-        why = "the step that produced it also ran the optimizer" if st.fresh_key is None else \
-            "another forward (feature mix) or an optimizer step ran since"
-        raise RuntimeError(f"NGCF (B200): {what} needs the embedding table as the forward left it, but {why}. "
-                           "Run the forward again, or construct the module with snapshot=True to keep a per-forward "
-                           "copy like the reference's torch.cat (NGCF.py:120).")
-
     @_lib.on_device
     def _materialize(self):
         if self._last is None:

@@ -77,6 +77,12 @@ SIGNATURES = {
                             _vp, _vp, _vp, _vp, _vp],
     "ngcf_hard_negatives_signed": [C.POINTER(_vp), C.POINTER(C.c_int), C.c_int, _i64, _vp, _i64, _vp, _vp, _i64, C.c_int,
                                    _u64, _vp, _vp, _vp, _vp, _vp],
+    "ngcf_hard_negatives_mean": [C.POINTER(_vp), C.c_int, C.c_int, _i64, _vp, _i64, _vp, _vp, _i64, C.c_int, C.c_int,
+                                 _u64, _vp, _vp, _vp, _vp, _vp],
+    "ngcf_layer_mean": [C.POINTER(_vp), C.c_int, C.c_int, _vp, _i64, _i64, _vp, _i64, _vp],
+    "ngcf_layer_mean_sets": [C.POINTER(_vp), C.c_int, C.c_int, C.POINTER(_vp), C.POINTER(_i64), C.POINTER(_i64),
+                             C.POINTER(_vp), C.c_int, _i64, _vp],
+    "ngcf_rowgrad_expand": [_vp, _i64, _vp, _i64, C.c_int, _f32, _vp, _i64, _vp],
     "ngcf_softmax_loss_workspace": [_i64, C.c_int, C.c_int, C.POINTER(_sz)],
     "ngcf_softmax_loss": [_vp, _vp, _vp, _i64, C.c_int, _vp, _vp, _f32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _sz, _vp],
     "ngcf_laplacian_entries": [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp],

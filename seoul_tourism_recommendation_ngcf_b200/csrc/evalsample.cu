@@ -6,7 +6,8 @@
 //   * ngcf_laplacian_entries — the non-zeros of L = D^-1/2 A D^-1/2 from the rating pairs (matrix.py:41-62),
 //                           section 8(f) #2.
 //   * ngcf_hard_negatives  — dynamic hard-negative sampling inside a training step: per batch row, M free items
-//                           scored against the user with the current layer outputs, the hardest one kept.
+//                           scored against the user with the current layer outputs, the hardest one kept
+//                           (ngcf_hard_negatives_mean: the same on LightGCN's layer-mean rows).
 // All are small latency/HBM-bound integer + dot-product kernels; no tensor cores.
 #include <limits.h>
 
@@ -195,6 +196,7 @@ struct HardNegArgs {
     int64_t* chosen;
     int64_t* cand;
     float* score;
+    float inv_n;                                         // kMean: 1 / n (last, so the other fields keep their offsets)
 };
 
 // One warp per batch row.  The user's final row (gather_row's formula: E_0 raw, E_k / max(||E_k||, 1e-12)) stays in
@@ -202,29 +204,49 @@ struct HardNegArgs {
 // l draws j = l and l + 32), and scored HN_GROUP at a time against the candidates' final rows, whose layer blocks are
 // normalised on the fly.  Only the B*M candidate rows of E_0..E_K are read.
 // kSigned: the pick is the largest signed score instead (the hard negative of a softmax loss).
-template <bool kSigned>
+// kMean: the final rows are LightGCN's layer mean (E_0 + ... + E_K) * inv_n, summed in ngcf_layer_mean's order, instead
+// of the normalised concat; every layer then has the width dim[0].  The user's mean row is kept in ur[0].
+template <bool kSigned, bool kMean>
 __global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegArgs a) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * HN_WARPS + warp;
     if (row >= a.batch) return;
     const int64_t usr = a.u_id[row];
     float ur[NGCF_MAX_LAYERS + 1][HN_Q];
+    if constexpr (kMean) {
+        const int d = a.dim[0];
+        float acc[HN_Q] = {};
 #pragma unroll
-    for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
-        if (k < a.n) {
-            const int d = a.dim[k];
-            const float* src = a.layer[k] + usr * (int64_t)d;
-            float ss = 0.f;
+        for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+            if (k < a.n) {
+                const float* src = a.layer[k] + usr * (int64_t)d;
 #pragma unroll
-            for (int q = 0; q < HN_Q; ++q) {
-                const int c = lane + 32 * q;
-                ur[k][q] = c < d ? src[c] : 0.f;
-                ss = fmaf(ur[k][q], ur[k][q], ss);
+                for (int q = 0; q < HN_Q; ++q) {
+                    const int c = lane + 32 * q;
+                    if (c < d) acc[q] += src[c];
+                }
             }
-            if (k > 0) {
-                const float scale = 1.f / fmaxf(sqrtf(warp_sum(ss)), 1e-12f);   // F.normalize, NGCF.py:144
+        }
 #pragma unroll
-                for (int q = 0; q < HN_Q; ++q) ur[k][q] *= scale;
+        for (int q = 0; q < HN_Q; ++q) ur[0][q] = acc[q] * a.inv_n;
+    } else {
+#pragma unroll
+        for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+            if (k < a.n) {
+                const int d = a.dim[k];
+                const float* src = a.layer[k] + usr * (int64_t)d;
+                float ss = 0.f;
+#pragma unroll
+                for (int q = 0; q < HN_Q; ++q) {
+                    const int c = lane + 32 * q;
+                    ur[k][q] = c < d ? src[c] : 0.f;
+                    ss = fmaf(ur[k][q], ur[k][q], ss);
+                }
+                if (k > 0) {
+                    const float scale = 1.f / fmaxf(sqrtf(warp_sum(ss)), 1e-12f);   // F.normalize, NGCF.py:144
+#pragma unroll
+                    for (int q = 0; q < HN_Q; ++q) ur[k][q] *= scale;
+                }
             }
         }
     }
@@ -254,30 +276,56 @@ __global__ void __launch_bounds__(HN_WARPS * 32) hard_negatives_kernel(HardNegAr
             it[g] = __shfl_sync(FULL_MASK, j < 32 ? item[0] : item[1], j & 31);
         }
         float sc[HN_GROUP] = {};
+        if constexpr (kMean) {
+            const int d = a.dim[0];
+            float acc[HN_GROUP][HN_Q] = {};
 #pragma unroll
-        for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
-            if (k < a.n) {
-                const int d = a.dim[k];
-                float v[HN_GROUP][HN_Q];
+            for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+                if (k < a.n) {
 #pragma unroll
-                for (int g = 0; g < HN_GROUP; ++g) {
-                    const float* src = a.layer[k] + (a.n_user + it[g]) * (int64_t)d;
+                    for (int g = 0; g < HN_GROUP; ++g) {
+                        const float* src = a.layer[k] + (a.n_user + it[g]) * (int64_t)d;
 #pragma unroll
-                    for (int q = 0; q < HN_Q; ++q) {
-                        const int c = lane + 32 * q;
-                        v[g][q] = c < d ? src[c] : 0.f;
+                        for (int q = 0; q < HN_Q; ++q) {
+                            const int c = lane + 32 * q;
+                            if (c < d) acc[g][q] += src[c];
+                        }
                     }
                 }
+            }
 #pragma unroll
-                for (int g = 0; g < HN_GROUP; ++g) {
-                    float dot = 0.f, ss = 0.f;
+            for (int g = 0; g < HN_GROUP; ++g) {
+                float dot = 0.f;
 #pragma unroll
-                    for (int q = 0; q < HN_Q; ++q) {
-                        dot = fmaf(ur[k][q], v[g][q], dot);
-                        ss = fmaf(v[g][q], v[g][q], ss);
+                for (int q = 0; q < HN_Q; ++q) dot = fmaf(ur[0][q], acc[g][q] * a.inv_n, dot);
+                sc[g] = warp_sum(dot);
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k <= NGCF_MAX_LAYERS; ++k) {
+                if (k < a.n) {
+                    const int d = a.dim[k];
+                    float v[HN_GROUP][HN_Q];
+#pragma unroll
+                    for (int g = 0; g < HN_GROUP; ++g) {
+                        const float* src = a.layer[k] + (a.n_user + it[g]) * (int64_t)d;
+#pragma unroll
+                        for (int q = 0; q < HN_Q; ++q) {
+                            const int c = lane + 32 * q;
+                            v[g][q] = c < d ? src[c] : 0.f;
+                        }
                     }
-                    dot = warp_sum(dot);
-                    sc[g] += k > 0 ? dot / fmaxf(sqrtf(warp_sum(ss)), 1e-12f) : dot;
+#pragma unroll
+                    for (int g = 0; g < HN_GROUP; ++g) {
+                        float dot = 0.f, ss = 0.f;
+#pragma unroll
+                        for (int q = 0; q < HN_Q; ++q) {
+                            dot = fmaf(ur[k][q], v[g][q], dot);
+                            ss = fmaf(v[g][q], v[g][q], ss);
+                        }
+                        dot = warp_sum(dot);
+                        sc[g] += k > 0 ? dot / fmaxf(sqrtf(warp_sum(ss)), 1e-12f) : dot;
+                    }
                 }
             }
         }
@@ -384,8 +432,8 @@ extern "C" int ngcf_sample_negatives(const int32_t* pos_ptr, const int32_t* pos_
     return NGCF_OK;
 }
 
-static int hard_negatives(bool is_signed, const float* const* layers_host, const int* dims_host, int n_layers_plus1,
-                          int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+static int hard_negatives(bool is_signed, bool mean, const float* const* layers_host, const int* dims_host,
+                          int n_layers_plus1, int64_t n_user, const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
                           const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed, const uint64_t* seed_dev,
                           int64_t* chosen, int64_t* cand, float* score, void* stream) {
     NGCF_REQUIRE(layers_host && dims_host, "hard_negatives: null layer array");
@@ -395,6 +443,8 @@ static int hard_negatives(bool is_signed, const float* const* layers_host, const
     for (int k = 0; k < n_layers_plus1; ++k) {
         NGCF_REQUIRE(layers_host[k] && dims_host[k] > 0 && dims_host[k] <= NGCF_MAX_WIDTH, "hard_negatives: bad block %d",
                      k);
+        NGCF_REQUIRE(!mean || dims_host[k] == dims_host[0], "hard_negatives: layer %d is %d wide, layer 0 %d", k,
+                     dims_host[k], dims_host[0]);
         a.layer[k] = layers_host[k];
         a.dim[k] = dims_host[k];
     }
@@ -404,15 +454,19 @@ static int hard_negatives(bool is_signed, const float* const* layers_host, const
     NGCF_REQUIRE(M >= 1 && M <= HN_MAX_M, "hard_negatives: M %d outside [1, %d]", M, HN_MAX_M);
     NGCF_REQUIRE(batch >= 0, "hard_negatives: batch %lld", (long long)batch);
     NGCF_REQUIRE(batch == 0 || (u_id && excl_ptr && chosen), "hard_negatives: null pointer");
-    a.n = n_layers_plus1; a.n_user = n_user; a.u_id = u_id; a.batch = batch; a.excl_ptr = excl_ptr;
+    a.n = n_layers_plus1; a.inv_n = 1.0f / (float)n_layers_plus1; a.n_user = n_user; a.u_id = u_id; a.batch = batch; a.excl_ptr = excl_ptr;
     a.excl_idx = excl_idx; a.n_items = (int)n_items; a.M = M; a.seed = seed; a.seed_dev = seed_dev;
     a.chosen = chosen; a.cand = cand; a.score = score;
     if (batch == 0) return NGCF_OK;
     const unsigned grid = (unsigned)ceil_div64(batch, HN_WARPS);
-    if (is_signed)
-        hard_negatives_kernel<true><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    if (mean && is_signed)
+        hard_negatives_kernel<true, true><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    else if (mean)
+        hard_negatives_kernel<false, true><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+    else if (is_signed)
+        hard_negatives_kernel<true, false><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
     else
-        hard_negatives_kernel<false><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
+        hard_negatives_kernel<false, false><<<grid, HN_WARPS * 32, 0, as_stream(stream)>>>(a);
     NGCF_LAUNCH_OK("hard_negatives_kernel");
     return NGCF_OK;
 }
@@ -422,7 +476,7 @@ extern "C" int ngcf_hard_negatives(const float* const* layers_host, const int* d
                                    const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
                                    const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
                                    void* stream) {
-    return hard_negatives(false, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
+    return hard_negatives(false, false, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
                           n_items, M, seed, seed_dev, chosen, cand, score, stream);
 }
 
@@ -431,6 +485,19 @@ extern "C" int ngcf_hard_negatives_signed(const float* const* layers_host, const
                                           const int32_t* excl_idx, int64_t n_items, int M, uint64_t seed,
                                           const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
                                           void* stream) {
-    return hard_negatives(true, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
+    return hard_negatives(true, false, layers_host, dims_host, n_layers_plus1, n_user, u_id, batch, excl_ptr, excl_idx,
                           n_items, M, seed, seed_dev, chosen, cand, score, stream);
+}
+
+extern "C" int ngcf_hard_negatives_mean(const float* const* layers_host, int d, int n_layers_plus1, int64_t n_user,
+                                        const int64_t* u_id, int64_t batch, const int64_t* excl_ptr,
+                                        const int32_t* excl_idx, int64_t n_items, int M, int signed_pick, uint64_t seed,
+                                        const uint64_t* seed_dev, int64_t* chosen, int64_t* cand, float* score,
+                                        void* stream) {
+    NGCF_REQUIRE(n_layers_plus1 >= 1 && n_layers_plus1 <= NGCF_MAX_LAYERS + 1, "hard_negatives: %d blocks",
+                 n_layers_plus1);
+    int dims[NGCF_MAX_LAYERS + 1];
+    for (int k = 0; k < n_layers_plus1; ++k) dims[k] = d;
+    return hard_negatives(signed_pick != 0, true, layers_host, dims, n_layers_plus1, n_user, u_id, batch, excl_ptr,
+                          excl_idx, n_items, M, seed, seed_dev, chosen, cand, score, stream);
 }
