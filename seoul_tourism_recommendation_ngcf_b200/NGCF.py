@@ -17,21 +17,50 @@ import torch.nn as nn
 import torch.distributed as dist
 
 from . import _lib
-from .plan import LaplacianPlan, node_dropout_bits, node_dropout_compact, spmm
+from .plan import LaplacianPlan, NodeDropout, spmm
 from .sampler import HardNegatives
 from .sharded import RowShards, all_gather_rows
 
 LEAKY_SLOPE = 0.2   # NGCF.py:140
 
 
-def _stream() -> int:
-    return _lib.current_stream()
-
-
 class _Ctx:
-    """Per-forward state shared by the autograd node and the module (layer activations, plan, masks)."""
-    __slots__ = ("plan", "E", "S", "dims", "vals_f", "vals_b", "mess_mult", "mess_p", "seed", "seed_dev", "masked", "drop_p", "bits_f", "bits_b", "comp_f", "comp_b", "mess_bits",
-                 "rows", "offsets", "W1", "W2", "fresh_key", "node_mode", "last_partial", "fm_stream", "hneg")
+    """Per-forward state shared by an autograd node and its module (NGCF or LightGCN): plan, layer outputs, RNG key,
+    node dropout, batch rows.  LightGCN leaves the NGCF-only fields (dims, S, W1, W2, vals_*, mess_*, last_partial,
+    fm_stream) unset."""
+    __slots__ = ("plan", "E", "seed", "seed_dev", "drop_p", "dropout", "rows", "offsets", "fresh_key", "hneg",
+                 "dims", "S", "W1", "W2", "vals_f", "vals_b", "mess_mult", "mess_p", "mess_bits", "last_partial",
+                 "fm_stream")
+
+    @property
+    def node_mode(self) -> str:
+        return self.dropout.mode
+
+
+class _RowGrads:
+    """A backward's output-row gradients summed per distinct row (ngcf_rowgrad_scatter): row r's sum is gsum[slot[r]],
+    slot[r] = -1 for rows without one.  ``reset()`` puts those slots back to -1 at the end of the backward."""
+
+    def __init__(self, mod, st: _Ctx, gouts, n_sets: int, width: int, n_rows: int):
+        dev = st.E[0].device
+        g = [(go.contiguous() if go is not None else torch.zeros(st.rows[j].numel(), width, device=dev))
+             for j, go in enumerate(gouts)]
+        batch = [r.numel() for r in st.rows[:n_sets]]
+        self.n_sets, self.rows, self.offs = n_sets, _lib.ptr_array(st.rows[:n_sets]), _lib.i64_array(st.offsets[:n_sets])
+        self.batch = _lib.i64_array(batch)
+        self.slot = mod._slot_map(n_rows, dev)
+        self.gsum = torch.empty(max(sum(batch), 1), width, dtype=torch.float32, device=dev)
+        _lib.check(_lib.load().ngcf_rowgrad_scatter(self.rows, self.offs, _lib.ptr_array(g), self.batch, n_sets, width,
+                                                    self.slot.data_ptr(), self.gsum.data_ptr(), _lib.current_stream()),
+                   "rowgrad_scatter")
+
+    def reset(self):
+        _lib.check(_lib.load().ngcf_rowgrad_reset(self.rows, self.offs, self.batch, self.n_sets, self.slot.data_ptr(),
+                                                  _lib.current_stream()), "rowgrad_reset")
+
+
+def _index(t, dev) -> torch.Tensor:
+    return t.to(device=dev, dtype=torch.int64).contiguous()
 
 
 def _capturing() -> bool:
@@ -69,30 +98,9 @@ class _Propagate(torch.autograd.Function):
             X0 = X0.clone()
         st.E, st.S, st.W1, st.W2 = [X0], [], list(W1), list(W2)
         side = st.plan.fwd
-        st.bits_f = st.bits_b = st.comp_f = st.comp_b = None
-        st.node_mode = mod._node_mode
         st.last_partial = None
-        if st.drop_p > 0:
-            # this step's node-dropout decisions for all K layers, drawn once instead of a hash evaluation per entry in
-            # each of the 2K products; a symmetric L serves both directions from one pass.  "compact" (default) also
-            # deletes the dropped entries like NGCF.sparse_dropout does, so layer k gathers (1-p)^(k+1) of the rows
-            shared = st.plan.side(True, False) is side
-            # compacted survivor lists are read by the streaming SpMM (widths that are multiples of 4); the reference's
-            # own width 65 runs the row-per-warp kernel from per-step decision bytes instead
-            # (every width, the last one too: the batch-row gradient rows of the final backward product are D_total wide)
-            node_mode = mod._node_mode if all(d % 4 == 0 for d in st.dims) or mod._node_mode == "inkernel" else "bits"
-            st.node_mode = node_mode
-            if node_mode == "compact":
-                # L's and (symmetric L) L^T's survivor lists in one pass: L^T's half on a second stream, beside the
-                # forward or behind its last layer, measured slower on one B200 (0.518 / 0.509-0.513 vs 0.502-0.510 ms
-                # per step: two more launches and the entries read twice cost more than the overlap hides)
-                st.comp_f, ct = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=True, as_Lt=shared)
-                if shared:
-                    st.comp_b = ct
-            elif node_mode == "bits":
-                st.bits_f, bt = node_dropout_bits(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=True, as_Lt=shared)
-                if shared:
-                    st.bits_b = bt
+        # the reference's own width 65 runs the row-per-warp kernel from per-step decision bytes (NodeDropout)
+        st.dropout = NodeDropout(st.plan, mod._node_mode, st.drop_p, st.seed, st.seed_dev, K, r0, st.dims)
         # message dropout (NGCF.py:142): optionally this step's decisions for every layer, one bit per element, drawn
         # by a full-GPU pass instead of inside the dense kernels (measured slower at Gowalla shape: off by default)
         self_uses_mess_bits = mod._mess_bits
@@ -101,7 +109,8 @@ class _Propagate(torch.autograd.Function):
             if self_uses_mess_bits and st.mess_mult is None and st.mess_p[k] > 0 and st.dims[k + 1] % 4 == 0:
                 bits = torch.empty(nloc * ((st.dims[k + 1] + 31) // 32), dtype=torch.int32, device=dev)
                 _lib.check(lib.ngcf_mess_dropout_bits(nv, st.dims[k + 1], float(st.mess_p[k]), st.seed,
-                                                      _lib.ptr(st.seed_dev), k, r0, bits.data_ptr(), _stream()),
+                                                      _lib.ptr(st.seed_dev), k, r0, bits.data_ptr(),
+                                                      _lib.current_stream()),
                            "mess_dropout_bits")
                 st.mess_bits[k] = bits
         # [W1^T ; W2^T] and 2 b1 + b2 of every layer: one launch (NGCF.py:131-136 applies w1_list[i] twice)
@@ -109,14 +118,13 @@ class _Propagate(torch.autograd.Function):
         biases = [torch.empty(st.dims[k + 1], dtype=torch.float32, device=dev) for k in range(K)]
         _lib.check(lib.ngcf_pack_weights_all(_lib.ptr_array(W1), _lib.ptr_array(b1), _lib.ptr_array(W2), _lib.ptr_array(b2),
                                              _lib.int_array(st.dims[:K]), _lib.int_array(st.dims[1:]), K,
-                                             _lib.ptr_array(wcats), _lib.ptr_array(biases), _stream()), "pack_weights_all")
+                                             _lib.ptr_array(wcats), _lib.ptr_array(biases), _lib.current_stream()),
+                   "pack_weights_all")
         _join_feature_mix(st)                                          # the first product reads the mixed user rows
         for k in range(K):
             d_in, d_out = st.dims[k], st.dims[k + 1]
             vals = st.vals_f[k] if st.vals_f is not None else None
-            S = spmm(side, vals, st.E[k], d_in, drop_p=st.drop_p, seed=st.seed, seed_dev=st.seed_dev, layer=k,
-                     row_offset=r0, keep_bits=st.bits_f,
-                     compact=st.comp_f[k] if st.comp_f is not None else None)               # NGCF.py:124-130
+            S = spmm(side, vals, st.E[k], d_in, **st.dropout.args(k))                           # NGCF.py:124-130
             wcat, bias = wcats[k], biases[k]
             xkey = None
             if sh is None:
@@ -134,7 +142,7 @@ class _Propagate(torch.autograd.Function):
             _lib.check(lib.ngcf_dense_fwd(S.data_ptr(), E_loc.data_ptr(), nv, d_in, d_out, wcat.data_ptr(),
                                           bias.data_ptr(), LEAKY_SLOPE, _lib.ptr(mm[r0:r0 + nloc] if mm is not None else None),
                                           _lib.ptr(st.mess_bits[k]), float(st.mess_p[k]), st.seed, _lib.ptr(st.seed_dev), k, r0, En.data_ptr(),
-                                          _stream()),
+                                          _lib.current_stream()),
                        "dense_fwd")                                                          # NGCF.py:131-142
             if xkey is not None and k == K - 1:
                 # nothing downstream gathers from the LAST layer's output: other ranks need it for the <= 3 B batch rows only
@@ -155,13 +163,13 @@ class _Propagate(torch.autograd.Function):
             _lib.check(pick(layers, dims, K + 1, mod.n_user, st.rows[0].data_ptr(),
                             st.rows[0].numel(), train.ptr.data_ptr(), _lib.ptr(train.idx),
                             mod.n_item, hn.n_candidates, st.seed, _lib.ptr(st.seed_dev),
-                            chosen.data_ptr(), _lib.ptr(cand), _lib.ptr(score), _stream()),
+                            chosen.data_ptr(), _lib.ptr(cand), _lib.ptr(score), _lib.current_stream()),
                        "hard_negatives")
         outs =[torch.empty(st.rows[j].numel(), D, dtype=torch.float32, device=dev) for j in range(n_sets)]
         _lib.check(lib.ngcf_gather_concat_sets(layers, dims, K + 1, _lib.ptr_array(st.rows[:n_sets]),
                                                _lib.i64_array(st.offsets[:n_sets]),
                                                _lib.i64_array([r.numel() for r in st.rows[:n_sets]]), _lib.ptr_array(outs),
-                                               n_sets, D, _stream()), "gather_concat_sets")       # NGCF.py:144-155
+                                               n_sets, D, _lib.current_stream()), "gather_concat_sets")   # NGCF.py:144-155
         ctx.st, ctx.mod, ctx.n_sets = st, mod, n_sets
         return tuple(outs)
 
@@ -176,18 +184,12 @@ class _Propagate(torch.autograd.Function):
         N = mod.n_user + mod.n_item
         r0, nloc, nv, N_all = (sh.r0, sh.rows, sh.valid, sh.N_pad) if sh is not None else (0, N, N, N)
         D = sum(dims)
-        g = [(go.contiguous() if go is not None else torch.zeros(st.rows[j].numel(), D, device=dev))
-             for j, go in enumerate(gouts)]
-        batch = [r.numel() for r in st.rows[:n_sets]]
-        rows_h, offs_h = _lib.ptr_array(st.rows[:n_sets]), _lib.i64_array(st.offsets[:n_sets])
-        g_h, batch_h = _lib.ptr_array(g), _lib.i64_array(batch)
-        slot = mod._slot_map(N_all, dev)
-        gsum = torch.empty(sum(batch), D, dtype=torch.float32, device=dev)
-        _lib.check(lib.ngcf_rowgrad_scatter(rows_h, offs_h, g_h, batch_h, n_sets, D, slot.data_ptr(),
-                                            gsum.data_ptr(), _stream()), "rowgrad_scatter")
+        rg = _RowGrads(mod, st, gouts, n_sets, D, N_all)
+        slot, gsum = rg.slot, rg.gsum
         # F.normalize's backward (NGCF.py:144) for the <= 3B rows that carry an output-row gradient, once, in place
-        _lib.check(lib.ngcf_rowgrad_normalize(rows_h, offs_h, batch_h, n_sets, _lib.ptr_array(st.E), _lib.int_array(dims),
-                                              K + 1, slot.data_ptr(), gsum.data_ptr(), D, _stream()), "rowgrad_normalize")
+        _lib.check(lib.ngcf_rowgrad_normalize(rg.rows, rg.offs, rg.batch, n_sets, _lib.ptr_array(st.E),
+                                              _lib.int_array(dims), K + 1, slot.data_ptr(), gsum.data_ptr(), D,
+                                              _lib.current_stream()), "rowgrad_normalize")
         slot_loc = slot[r0:r0 + nloc]
         sizes = [dims[k + 1] * dims[k] for k in range(K)]
         n_flat = 2 * sum(sizes) + 2 * sum(dims[1:])
@@ -210,10 +212,7 @@ class _Propagate(torch.autograd.Function):
         # explicit (COO-order) masks need the separately sorted L^T; in-kernel device-RNG dropout is keyed on the
         # entry's coordinates, so a symmetric L keeps sharing its forward arrays (transposed=1 swaps the key)
         side = st.plan.side(True, st.vals_b is not None)
-        if st.drop_p > 0 and st.node_mode == "compact" and st.comp_b is None:
-            _, st.comp_b = node_dropout_compact(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=False, as_Lt=True)
-        if st.drop_p > 0 and st.node_mode == "bits" and st.bits_b is None:
-            _, st.bits_b = node_dropout_bits(side, st.drop_p, st.seed, st.seed_dev, K, r0, as_L=False, as_Lt=True)
+        st.dropout.draw_transposed()
         gE_next = None
         col_off = D
         # the weight-gradient kernels need gM only: beside the transposed product (and the gS exchange queued behind the
@@ -257,7 +256,7 @@ class _Propagate(torch.autograd.Function):
                                           _lib.ptr(st.seed_dev), k, r0, 1, gS.data_ptr(),
                                           gEl.data_ptr(),
                                           gW1[k].data_ptr(), gb1[k].data_ptr(), gW2[k].data_ptr(), gb2[k].data_ptr(),
-                                          gM_scratch.data_ptr(), _stream()), "dense_bwd")
+                                          gM_scratch.data_ptr(), _lib.current_stream()), "dense_bwd")
             if peer:                                                  # L^T gS needs every rank's rows of gS
                 mod._xchg.push(("gS", d_in), r0, nloc)
             elif sh is not None:
@@ -268,17 +267,15 @@ class _Propagate(torch.autograd.Function):
             vals = st.vals_b[k] if st.vals_b is not None else None
             last = (k == 0)
             gE_next = spmm(side, vals, gS_all, d_in, addend=gEl, slot=slot_loc if last else None,
-                           gsum=gsum if last else None, drop_p=st.drop_p, seed=st.seed, seed_dev=st.seed_dev, layer=k,
-                           transposed=True, row_offset=r0, keep_bits=st.bits_b,
-                           compact=st.comp_b[k] if st.comp_b is not None else None)   # gE_k = gEl + L^T gS (+ row grads)
+                           gsum=gsum if last else None,
+                           **st.dropout.args(k, transposed=True))              # gE_k = gEl + L^T gS (+ row grads)
             if mod._trace is not None:                                # debugging aid: per-layer backward tensors
                 mod._trace.append(dict(k=k, gS=gS.clone(), gEl=gEl.clone(), gE=gE_next.clone()))
         if overlap:                                                   # join: the weight gradients are complete
             _lib.check(lib.ngcf_set_wgrad_stream(None), "set_wgrad_stream")
             if lib.ngcf_wgrad_stream_forked():                        # (FFMA layers never fork: nothing to wait for)
                 torch.cuda.current_stream().wait_stream(mod._side_stream)
-        _lib.check(lib.ngcf_rowgrad_reset(rows_h, offs_h, batch_h, n_sets, slot.data_ptr(), _stream()),
-                   "rowgrad_reset")
+        rg.reset()
         if sh is not None:
             if mod._xchg is not None and dims[0] % 4 == 0:
                 mod._xchg.push(("gE0", dims[0]), r0, nloc)             # tables are replicated: full gradient everywhere
@@ -311,10 +308,128 @@ def draw_seed(generator=None) -> int:
 
 class _TableModel(nn.Module):
     """What NGCF and LightGCN share: E_0 of a forward is the live packed [N, d] table behind ``user_embedding`` and
-    ``item_embedding`` (no copy), one execution plan per ``lap_list`` element, the row-gradient slot map, and the rule
-    that refuses to use a forward's E_0 once the table changed under it.  Subclasses set n_user, n_item, emb_size,
-    lap_list, _plans, _table, _slot, _shard, _snapshot and _mix_count, and name themselves in _NAME."""
+    ``item_embedding`` (no copy), one execution plan per ``lap_list`` element, the row-gradient slot map, the rule
+    that refuses to use a forward's E_0 once the table changed under it, and the forward's steps either side of the
+    propagation: batch rows, feature mix, RNG key, and ``all_users_emb`` / ``all_items_emb`` built on first read.
+    Subclasses set n_user, n_item, emb_size, n_layer, lap_list and rng, name themselves in _NAME and supply
+    ``_readout``."""
     _STALE_ADVICE = "Run the forward again."
+
+    def __init__(self):
+        super().__init__()
+        self._plans = {}
+        self._table = None
+        self._slot = None
+        self._winner = None      # feature mix: per-user scratch of ngcf_feature_mix
+        self._last = None        # _Ctx of the last forward
+        self._all_E = None
+        self._shard = None       # sharded.RowShards once NGCF.shard() was called
+        self._snapshot = False
+        self._mix_count = 0
+        self._seed_dev = None    # device uint64 added to the RNG key (set by graph.GraphedStep)
+
+    def _feature_tables(self, num_dict: dict):
+        """The five feature tables in the reference's registration order (NGCF.py:39-45), which fixes the state_dict
+        order; each nn.Embedding draws its initial values from the CPU generator.  The reference needs
+        embed_size % 5 == 0 (its concat is 5*(emb//5) wide, NGCF.py:110-114); here the last table of the concat order
+        (dow) absorbs the remainder, which is the same thing whenever emb % 5 == 0."""
+        w = self.emb_size // 5
+        self.feat_widths = [w, w, w, w, self.emb_size - 4 * w]          # age, sex, month, day, dow
+        self.month_emb = nn.Embedding(int(num_dict['month']), w)
+        self.day_emb = nn.Embedding(int(num_dict['day']), w)
+        self.sex_emb = nn.Embedding(int(num_dict['sex']), w)
+        self.age_emb = nn.Embedding(int(num_dict['age']), w)
+        self.dow_emb = nn.Embedding(int(num_dict['dayofweek']), self.feat_widths[4])
+
+    def _cuda_device(self) -> torch.device:
+        dev = self.user_embedding.weight.device
+        if dev.type != "cuda":
+            raise RuntimeError(f"{self._NAME} (B200) runs on a CUDA device only; there is no CPU fallback. "
+                               "Move the module with .to('cuda').")
+        return dev
+
+    def _batch(self, dev, u_id, pos_item, neg_item) -> _Ctx:
+        """A forward's _Ctx with its row sets: users, positives and, unless ``neg_item`` is empty, negatives (st.rows,
+        their offsets into the packed table in st.offsets).  With ``neg_item`` a HardNegatives the negatives are the
+        buffer its device pass fills, and st.hneg holds that pass's operands."""
+        st = _Ctx()
+        u_id, pos_item = _index(u_id, dev), _index(pos_item, dev)
+        hneg = neg_item if isinstance(neg_item, HardNegatives) else None
+        if hneg is not None:
+            if self._shard is not None:
+                raise ValueError("HardNegatives: not available on a row-sharded model (the candidates' rows of the "
+                                 "last layer are spread over the ranks)")
+            if hneg.train.n_rows != self.n_user or hneg.train.n_items != self.n_item:
+                raise ValueError(f"HardNegatives: train has {hneg.train.n_rows} rows over {hneg.train.n_items} items; "
+                                 f"the model has {self.n_user} users and {self.n_item} items")
+            neg_item = torch.empty(u_id.numel(), dtype=torch.int64, device=dev)   # written by the hard-negative pass
+        else:
+            neg_item = _index(neg_item, dev) if len(neg_item) > 0 else None   # NGCF.py:154
+        st.rows = [u_id, pos_item] + ([neg_item] if neg_item is not None else [])
+        st.offsets = [0, self.n_user] + ([self.n_user] if neg_item is not None else [])
+        st.hneg = None
+        if hneg is not None:
+            M = hneg.n_candidates
+            st.hneg = (hneg, hneg._on(dev), neg_item,
+                       torch.empty(u_id.numel(), M, dtype=torch.int64, device=dev) if hneg.debug else None,
+                       torch.empty(u_id.numel(), M, dtype=torch.float32, device=dev) if hneg.debug else None)
+            hneg.chosen, hneg.cand, hneg.score = st.hneg[2:]
+        return st
+
+    def _feature_mix(self, table, u_id, feats):
+        """The feature mix of the batch users' rows of ``table`` (NGCF.py:103-115) on the current stream; ``feats`` are
+        the age, sex, month, day and dow indices."""
+        dev = table.device
+        if self._winner is None or self._winner.device != dev or self._winner.numel() != self.n_user:
+            self._winner = torch.full((self.n_user,), -1, dtype=torch.int32, device=dev)
+        tabs = [self.age_emb.weight, self.sex_emb.weight, self.month_emb.weight, self.day_emb.weight, self.dow_emb.weight]
+        feats = [_index(t, dev) for t in feats]
+        _lib.check(_lib.load().ngcf_feature_mix(table.data_ptr(), self.n_user, self.emb_size, _lib.ptr_array(tabs),
+                                                _lib.int_array(self.feat_widths), _lib.ptr_array(feats),
+                                                u_id.data_ptr(), u_id.numel(), float(self.emb_ratio),
+                                                self._winner.data_ptr(), _lib.current_stream()), "feature_mix")
+        self._mix_count += 1
+
+    def _draw_seed(self, st: _Ctx, mess_dropout: bool = False):
+        """The forward's RNG key from torch's CPU generator (reproducible under torch.manual_seed), drawn only when a
+        device-RNG stream is live and only after the rng="reference" mask draws, whose RNG stream it must not shift.
+        The hard-negative draws take the same key: with dropout on, a forward with HardNegatives and one without
+        draw the same key from the generator and so the same dropout masks."""
+        need = st.drop_p > 0 or mess_dropout or st.hneg is not None
+        if not need:
+            st.seed = 0
+        elif self.rng == "reference":
+            if self._seed_gen is None:
+                self._seed_gen = torch.Generator().manual_seed(torch.initial_seed() & (2 ** 63 - 1))
+            st.seed = draw_seed(self._seed_gen)
+        else:
+            st.seed = draw_seed()
+        # CUDA-graph mode (graph.GraphedStep): the launches are frozen, so the per-step key comes from a device counter
+        st.seed_dev = self._seed_dev if need else None
+
+    def _finish(self, st: _Ctx, outs):
+        """Keeps the forward's state for the backward and all_users_emb; returns the (users, positives, negatives)
+        rows, negatives ``torch.empty(0)`` when the batch has none (NGCF.py:153)."""
+        self._last, self._all_E = st, None
+        return outs[0], outs[1], (outs[2] if len(outs) > 2 else torch.empty(0))
+
+    # ---- attributes the reference sets in forward (NGCF.py:147-149), materialised on first read ---------
+    @_lib.on_device
+    def _materialize(self):
+        if self._last is None:
+            raise AttributeError("all_users_emb / all_items_emb exist after the first forward")
+        if self._all_E is None:
+            self._check_fresh(self._last, "all_users_emb / all_items_emb")
+            self._all_E = self._readout(self._last)
+        return self._all_E
+
+    @property
+    def all_users_emb(self):
+        return self._materialize()[:self.n_user, :]
+
+    @property
+    def all_items_emb(self):
+        return self._materialize()[self.n_user:, :]
 
     def _packed_table(self) -> torch.Tensor:
         """[N, d] view over user_embedding.weight and item_embedding.weight laid out back to back, so that
@@ -346,6 +461,9 @@ class _TableModel(nn.Module):
         if p is None or p.src is not L or p.coo_val.device != dev:
             p = LaplacianPlan(L, dev, shard=self._shard)
             self._plans[year_idx] = p
+        N = self.n_user + self.n_item
+        if p.N != N:
+            raise ValueError(f"{self._NAME}: the Laplacian is {p.N}x{p.N} but n_user + n_item = {N}")
         return p
 
     def _fresh_key(self):
@@ -399,26 +517,11 @@ class NGCF(_TableModel):
         if max([self.emb_size] + self.weight_size) > 128 or self.n_layer > 8:
             raise ValueError("embedding/layer widths up to 128 and up to 8 layers are supported")
 
-        # Feature tables in the reference's registration order (NGCF.py:39-45).  The reference needs
-        # embed_size % 5 == 0 (its concat is 5*(emb//5) wide, NGCF.py:110-114); here the last table of the
-        # concat order (dow) absorbs the remainder, which is the same thing whenever emb % 5 == 0.
-        w = self.emb_size // 5
-        self.feat_widths = [w, w, w, w, self.emb_size - 4 * w]          # age, sex, month, day, dow
-        self.month_emb = nn.Embedding(int(num_dict['month']), w)
-        self.day_emb = nn.Embedding(int(num_dict['day']), w)
-        self.sex_emb = nn.Embedding(int(num_dict['sex']), w)
-        self.age_emb = nn.Embedding(int(num_dict['age']), w)
-        self.dow_emb = nn.Embedding(int(num_dict['dayofweek']), self.feat_widths[4])
+        self._feature_tables(num_dict)
         self.item_embedding = nn.Embedding(self.n_item, self.emb_size)
         self.user_embedding = nn.Embedding(self.n_user, self.emb_size)
         self.lap_list = lap_list
         self.set_layers()
-        self._plans = {}
-        self._table = None
-        self._slot = None
-        self._winner = None
-        self._last = None
-        self._all_E = None
         self._mess_bits = os.environ.get("NGCF_B200_MESS_BITS", "0") == "1"   # precompute message-dropout bits per step
         self._node_mode = "compact"   # device-RNG node dropout: "compact" (survivors only), "bits", or "inkernel"
         # E_0 of a forward is the LIVE packed table, not a copy (the reference's torch.cat at NGCF.py:120 copies 2 x 18 MB
@@ -426,11 +529,8 @@ class NGCF(_TableModel):
         # under a pending backward / under all_users_emb: that is detected and refused (_check_fresh).  snapshot=True (or
         # NGCF_B200_SNAPSHOT=1) copies the table per forward instead and lifts the restriction.
         self._snapshot = bool(snapshot) or os.environ.get("NGCF_B200_SNAPSHOT", "0") == "1"
-        self._mix_count = 0
         self._seed_gen = None    # rng="reference": private generator for the device-RNG key (message dropout), so the
                                  # CPU generator is consumed by the node masks only, exactly like the reference's stream
-        self._seed_dev = None    # device uint64 added to the RNG key (set by graph.GraphedStep)
-        self._shard = None       # sharded.RowShards once shard() was called
         self._group = None
         self._xchg = None        # sharded.PeerExchange (peer-memory exchange) when available
         self._side_stream = None     # weight gradients beside the transposed product (_Propagate.backward)
@@ -526,49 +626,19 @@ class NGCF(_TableModel):
     # ---- forward ---------------------------------------------------------------------------------------
     @_lib.on_device
     def forward(self, year, u_id, age, sex, month, day, dow, pos_item, neg_item, node_flag):
-        lib = _lib.load()
-        dev = self.user_embedding.weight.device
-        if dev.type != "cuda":
-            raise RuntimeError("NGCF (B200) runs on a CUDA device only; there is no CPU fallback. "
-                               "Move the module with .to('cuda').")
-        K, N = self.n_layer, self.n_user + self.n_item
+        dev = self._cuda_device()
+        K = self.n_layer
         if (self._side_stream is None or self._side_stream.device != dev) and not _capturing():
             # second streams of the capture-time overlaps, handed out of torch's pool BEFORE any capture begins
             self._side_stream, self._side_stream3 = (torch.cuda.Stream(device=dev) for _ in range(2))
-
-        def ix(t):
-            return t.to(device=dev, dtype=torch.int64).contiguous()
-
-        u_id, pos_item = ix(u_id), ix(pos_item)
-        feats_idx = [ix(age), ix(sex), ix(month), ix(day), ix(dow)]          # concat order, NGCF.py:110
-        hneg = neg_item if isinstance(neg_item, HardNegatives) else None
-        if hneg is not None:
-            if self._shard is not None:
-                raise ValueError("HardNegatives: not available on a row-sharded model (the candidates' rows of the "
-                                 "last layer are spread over the ranks)")
-            if hneg.train.n_rows != self.n_user or hneg.train.n_items != self.n_item:
-                raise ValueError(f"HardNegatives: train has {hneg.train.n_rows} rows over {hneg.train.n_items} items; "
-                                 f"the model has {self.n_user} users and {self.n_item} items")
-            has_neg = True
-            neg_item = torch.empty(u_id.numel(), dtype=torch.int64, device=dev)   # written by ngcf_hard_negatives
-        else:
-            has_neg = len(neg_item) > 0                                      # NGCF.py:154
-            neg_item = ix(neg_item) if has_neg else None
+        st = self._batch(dev, u_id, pos_item, neg_item)
         year_idx = int(year.min()) % 18                                      # == year.unique()[0] % 18, NGCF.py:117
 
         table = self._packed_table()
-        if self._winner is None or self._winner.device != dev or self._winner.numel() != self.n_user:
-            self._winner = torch.full((self.n_user,), -1, dtype=torch.int32, device=dev)
-        tabs = [self.age_emb.weight, self.sex_emb.weight, self.month_emb.weight, self.day_emb.weight, self.dow_emb.weight]
-        def mix():
-            _lib.check(lib.ngcf_feature_mix(table.data_ptr(), self.n_user, self.emb_size, _lib.ptr_array(tabs),
-                                            _lib.int_array(self.feat_widths), _lib.ptr_array(feats_idx), u_id.data_ptr(),
-                                            u_id.numel(), float(self.emb_ratio), self._winner.data_ptr(), _stream()),
-                       "feature_mix")                                        # NGCF.py:103-115
-
+        feats = (age, sex, month, day, dow)                                  # concat order, NGCF.py:110
         # the feature mix (two small launches that rewrite <= B user rows) on a second stream beside the node-dropout
         # compaction, which does not touch the table; joined before the first product (0.502 -> 0.499 ms per step)
-        fm_stream = None
+        st.fm_stream = None
         if self._shard is None and _capturing() and bool(node_flag) and \
                 (self.node_dropout or 0) > 0 and self.rng == "device":
             main = torch.cuda.current_stream()
@@ -576,29 +646,23 @@ class NGCF(_TableModel):
                 self._side_stream3 = torch.cuda.Stream(device=dev)
             self._side_stream3.wait_stream(main)
             with torch.cuda.stream(self._side_stream3):
-                mix()
-            fm_stream = self._side_stream3
+                self._feature_mix(table, st.rows[0], feats)
+            st.fm_stream = self._side_stream3
         else:
-            mix()
+            self._feature_mix(table, st.rows[0], feats)
 
-        self._mix_count += 1
-        st = _Ctx()
-        st.fm_stream = fm_stream
         st.fresh_key = self._fresh_key()
         st.plan = plan = self._plan(year_idx, dev)
         if self._shard is not None and "edge_keep" in (self._inject or {}):
             raise ValueError("explicit edge masks are not supported in row-sharded mode")
-        if plan.N != N:
-            raise ValueError(f"Laplacian is {plan.N}x{plan.N} but n_user+n_item = {N}")
         st.dims = [self.emb_size] + self.weight_size
         inj = self._inject or {}
         # node dropout: active whenever node_flag is set, in eval mode too (NGCF.py:124-126)
-        st.masked = bool(node_flag) and (self.node_dropout is not None) and \
-            (self.node_dropout > 0 or "edge_keep" in inj)
+        masked = bool(node_flag) and (self.node_dropout is not None) and (self.node_dropout > 0 or "edge_keep" in inj)
         st.vals_f = st.vals_b = None
         st.drop_p = 0.0
         masks = None
-        if st.masked:
+        if masked:
             if "edge_keep" in inj:
                 masks = [m.to(device=dev, dtype=torch.uint8).contiguous() for m in inj["edge_keep"]]
             elif self.rng == "reference":
@@ -612,65 +676,24 @@ class NGCF(_TableModel):
             st.mess_mult = [m.to(device=dev, dtype=torch.float32).contiguous() for m in inj["mess_mult"]]
         elif self.training and self.mess_dropout is not None:
             st.mess_p = [float(p) for p in self.mess_dropout[:K]]
-        # per-forward RNG key from torch's CPU generator (reproducible under torch.manual_seed); drawn only when
-        # a device-RNG stream is live and only after the reference-mode mask draws, whose RNG stream it must not shift
-        # (the hard-negative draws take the same seed: with dropout on, a forward with HardNegatives and one without draw
-        # the same key from the generator and so the same dropout masks)
-        need_seed = st.drop_p > 0 or any(p > 0 for p in st.mess_p) or hneg is not None
-        if not need_seed:
-            st.seed = 0
-        elif self.rng == "reference":
-            if self._seed_gen is None:
-                self._seed_gen = torch.Generator().manual_seed(torch.initial_seed() & (2 ** 63 - 1))
-            st.seed = draw_seed(self._seed_gen)
-        else:
-            st.seed = draw_seed()
-        # CUDA-graph mode (graph.GraphedStep): the launches are frozen, so the per-step key comes from a device counter
-        st.seed_dev = self._seed_dev if need_seed else None
+        self._draw_seed(st, mess_dropout=any(p > 0 for p in st.mess_p))
         if masks is not None:
             st.vals_f = [plan.entries(plan.fwd, masks[k]) for k in range(K)]
             st.vals_b = [plan.entries(plan.bwd, masks[k]) for k in range(K)]
-        st.rows = [u_id, pos_item] + ([neg_item] if has_neg else [])
-        st.offsets = [0, self.n_user] + ([self.n_user] if has_neg else [])
-        st.hneg = None
-        if hneg is not None:
-            M = hneg.n_candidates
-            st.hneg = (hneg, hneg._on(dev), neg_item,
-                       torch.empty(u_id.numel(), M, dtype=torch.int64, device=dev) if hneg.debug else None,
-                       torch.empty(u_id.numel(), M, dtype=torch.float32, device=dev) if hneg.debug else None)
-            hneg.chosen, hneg.cand, hneg.score = st.hneg[2:]
 
         wb = [l.weight for l in self.w1_list] + [l.bias for l in self.w1_list] + \
              [l.weight for l in self.w2_list] + [l.bias for l in self.w2_list]
         outs = _Propagate.apply(self, st, len(st.rows), self.user_embedding.weight, self.item_embedding.weight, *wb)
-        self._last, self._all_E = st, None
-        u_embeddings, pos_i_embeddings = outs[0], outs[1]
-        neg_i_embeddings = outs[2] if has_neg else torch.empty(0)           # NGCF.py:153
-        return u_embeddings, pos_i_embeddings, neg_i_embeddings
+        return self._finish(st, outs)
 
-    # ---- attributes the reference sets in forward (NGCF.py:147-149), materialised on first read ---------
-    @_lib.on_device
-    def _materialize(self):
-        if self._last is None:
-            raise AttributeError("all_users_emb / all_items_emb exist after the first forward (NGCF.py:148-149)")
-        if self._all_E is None:
-            self._check_fresh(self._last, "all_users_emb / all_items_emb")
-            if self._last.last_partial is not None:                   # row-sharded: the last layer travelled for the batch
-                sh = self._shard                                       # rows only; complete it now (COLLECTIVE: every rank
-                self._xchg.push(self._last.last_partial, sh.r0, sh.rows)    # must read the attribute)
-                self._last.last_partial = None
-            st, lib = self._last, _lib.load()
-            N, D = self.n_user + self.n_item, sum(st.dims)
-            out = torch.empty(N, D, dtype=torch.float32, device=st.E[0].device)
-            _lib.check(lib.ngcf_gather_concat(_lib.ptr_array(st.E), _lib.int_array(st.dims), self.n_layer + 1, None, 0,
-                                              N, out.data_ptr(), D, _stream()), "gather_concat")
-            self._all_E = out
-        return self._all_E
-
-    @property
-    def all_users_emb(self):
-        return self._materialize()[:self.n_user, :]
-
-    @property
-    def all_items_emb(self):
-        return self._materialize()[self.n_user:, :]
+    def _readout(self, st: _Ctx) -> torch.Tensor:
+        """[N, sum(dims)]: the concatenated layer outputs of every row (NGCF.py:144-149)."""
+        if st.last_partial is not None:                       # row-sharded: the last layer travelled for the batch
+            sh = self._shard                                   # rows only; complete it now (COLLECTIVE: every rank
+            self._xchg.push(st.last_partial, sh.r0, sh.rows)   # must read the attribute)
+            st.last_partial = None
+        N, D = self.n_user + self.n_item, sum(st.dims)
+        out = torch.empty(N, D, dtype=torch.float32, device=st.E[0].device)
+        _lib.check(_lib.load().ngcf_gather_concat(_lib.ptr_array(st.E), _lib.int_array(st.dims), self.n_layer + 1, None,
+                                                  0, N, out.data_ptr(), D, _lib.current_stream()), "gather_concat")
+        return out

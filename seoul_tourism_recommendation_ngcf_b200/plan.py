@@ -21,10 +21,6 @@ import torch
 from . import _lib
 
 
-def _stream() -> int:
-    return _lib.current_stream()
-
-
 def greedy_tiles(rowptr: np.ndarray, max_rows: int, max_ent: int) -> np.ndarray:
     """Cuts rows [0, n) into consecutive tiles of at most ``max_rows`` rows and ``max_ent`` entries (a single
     row longer than ``max_ent`` gets a tile of its own).  Returns int32 [n_tiles, 4] = (r0, r1, e0, e1)."""
@@ -56,7 +52,8 @@ def device_tiles(rowptr: torch.Tensor, max_rows: int, max_ent: int) -> torch.Ten
     for capacity in (guess, cap):
         tiles = torch.empty(capacity, 4, dtype=torch.int32, device=dev)
         _lib.check(lib.ngcf_build_tiles(rowptr.data_ptr(), n, int(max_rows), int(max_ent), nxt.data_ptr(),
-                                        tiles.data_ptr(), capacity, count.data_ptr(), _stream()), "build_tiles")
+                                        tiles.data_ptr(), capacity, count.data_ptr(), _lib.current_stream()),
+                   "build_tiles")
         if int(count) <= capacity:
             return tiles[:int(count)].contiguous()
     raise RuntimeError("tile builder overflow")
@@ -210,7 +207,7 @@ class CsrSide:
             kl = torch.empty(max(self.nnz, 1), dtype=torch.int32, device=dev)
             kt = torch.empty(max(self.nnz, 1), dtype=torch.int32, device=dev)
             _lib.check(lib.ngcf_entry_keys(C.byref(self.descriptor(None)), int(row_offset), kl.data_ptr(), kt.data_ptr(),
-                                           _stream()), "entry_keys")
+                                           _lib.current_stream()), "entry_keys")
             self.key_l, self.key_t, self.key_row_offset = kl, kt, int(row_offset)
             self._struct_cache.clear()
 
@@ -274,7 +271,7 @@ class LaplacianPlan:
             perm = torch.empty(max(nnz, 1), dtype=torch.int32, device=device)
             _lib.check(lib.ngcf_coo_to_csr(row.data_ptr(), col.data_ptr(), nnz, n_rows, n_cols, 0,
                                            rowptr.data_ptr(), colidx.data_ptr(), perm.data_ptr(), ws.data_ptr(),
-                                           need.value, _stream()), "coo_to_csr")
+                                           need.value, _lib.current_stream()), "coo_to_csr")
             # perm indexes this side's entry list; compose with `pos` so it addresses the ORIGINAL COO order
             perm = pos[perm[:nnz].to(torch.int64)].to(torch.int32) if nnz else perm
             side = CsrSide(rowptr, colidx, perm, n_rows, nnz)
@@ -329,7 +326,8 @@ class LaplacianPlan:
             return out
         out = torch.zeros(side.nnz + 2, 2, dtype=torch.int32, device=self.coo_val.device)
         _lib.check(lib.ngcf_edge_entries(side.colidx.data_ptr(), self.coo_val.data_ptr(), side.perm.data_ptr(),
-                                         _lib.ptr(keep_mask), out.data_ptr(), side.nnz, _stream()), "edge_entries")
+                                         _lib.ptr(keep_mask), out.data_ptr(), side.nnz, _lib.current_stream()),
+                   "edge_entries")
         return out
 
 
@@ -343,7 +341,7 @@ def node_dropout_bits(side: CsrSide, drop_p: float, seed: int, seed_dev, n_layer
     bt = torch.empty(side.nnz, dtype=torch.uint8, device=dev) if as_Lt else None
     _lib.check(lib.ngcf_node_dropout_bits(C.byref(side.descriptor(None)), float(drop_p), int(seed) & (2 ** 64 - 1),
                                           _lib.ptr(seed_dev), int(n_layers), int(row_offset), _lib.ptr(bl), _lib.ptr(bt),
-                                          _stream()), "node_dropout_bits")
+                                          _lib.current_stream()), "node_dropout_bits")
     return bl, bt
 
 
@@ -378,7 +376,7 @@ def node_dropout_compact(side: CsrSide, drop_p: float, seed: int, seed_dev, n_la
     et, tt = arrs(ct)
     _lib.check(lib.ngcf_node_dropout_compact(C.byref(side.descriptor(None)), float(drop_p), int(seed) & (2 ** 64 - 1),
                                              _lib.ptr(seed_dev), int(n_layers), int(row_offset), el, tl, et, tt,
-                                             _stream()), "node_dropout_compact")
+                                             _lib.current_stream()), "node_dropout_compact")
     return cl, ct
 
 
@@ -403,5 +401,55 @@ def spmm(side: CsrSide, ent, X, d: int, out=None, addend=None, slot=None, gsum=N
                              int(row_offset), _lib.ptr(keep_bits),
                              _lib.ptr(compact[0]) if compact is not None else None,
                              _lib.ptr(compact[1]) if compact is not None else None,
-                             out.data_ptr(), out.stride(0), _stream()), "spmm")
+                             out.data_ptr(), out.stride(0), _lib.current_stream()), "spmm")
     return out
+
+
+def node_dropout_mode(mode: str, widths) -> str:
+    """The node-dropout mode a step runs for the requested ``mode``: survivor lists ("compact") are read by the
+    streaming SpMM, which needs every width to be a multiple of 4 (the last one too: the batch-row gradient rows of the
+    final backward product are D_total wide); other widths take per-step decision bytes ("bits")."""
+    return "bits" if mode == "compact" and any(d % 4 for d in widths) else mode
+
+
+class NodeDropout:
+    """One step's device-RNG node dropout for the K products over L and the K transposed products over L^T.
+
+    ``mode`` "compact" deletes the dropped entries like NGCF.sparse_dropout does (per-step survivor lists, so layer k
+    gathers (1-p)^(k+1) of the rows); "bits" draws per-step decision bytes; "inkernel" hashes every entry inside each
+    product; ``node_dropout_mode`` turns "compact" into "bits" for widths the survivor lists cannot serve.  The
+    decisions of all K layers are drawn once, on construction, and a symmetric L serves L^T from the same pass;
+    otherwise ``draw_transposed()`` draws L^T's where the backward calls it.  (L^T's half on a second stream, beside
+    the forward or behind its last layer, measured slower on one B200: 0.518 / 0.509-0.513 vs 0.502-0.510 ms per step,
+    two more launches and the entries read twice cost more than the overlap hides.)  ``args(layer, transposed)`` are
+    the dropout arguments of one ``spmm`` call."""
+
+    def __init__(self, plan: LaplacianPlan, mode: str, drop_p: float, seed: int, seed_dev, n_layers: int,
+                 row_offset: int, widths):
+        mode = node_dropout_mode(mode, widths)
+        self.plan, self.mode, self.drop_p, self.seed, self.seed_dev = plan, mode, drop_p, seed, seed_dev
+        self.n_layers, self.row_offset = n_layers, row_offset
+        self.fwd = self.bwd = None          # per-layer (ent, cnt) pairs ("compact") or one uint8 array ("bits")
+        if self._drawn():
+            shared = plan.side(True, False) is plan.fwd
+            self.fwd, bwd = self._draw(plan.fwd, as_L=True, as_Lt=shared)
+            if shared:
+                self.bwd = bwd
+
+    def _drawn(self) -> bool:
+        return self.drop_p > 0 and self.mode in ("compact", "bits")
+
+    def _draw(self, side: CsrSide, as_L: bool, as_Lt: bool):
+        draw = node_dropout_compact if self.mode == "compact" else node_dropout_bits
+        return draw(side, self.drop_p, self.seed, self.seed_dev, self.n_layers, self.row_offset, as_L=as_L, as_Lt=as_Lt)
+
+    def draw_transposed(self):
+        """L^T's decisions, unless the forward's pass drew them with L's."""
+        if self._drawn() and self.bwd is None:
+            _, self.bwd = self._draw(self.plan.side(True, False), as_L=False, as_Lt=True)
+
+    def args(self, layer: int, transposed: bool = False) -> dict:
+        lists = self.bwd if transposed else self.fwd
+        return dict(drop_p=self.drop_p, seed=self.seed, seed_dev=self.seed_dev, layer=layer, transposed=transposed,
+                    row_offset=self.row_offset, keep_bits=lists if self.mode == "bits" else None,
+                    compact=lists[layer] if self.mode == "compact" and lists is not None else None)

@@ -83,11 +83,9 @@ def products(m):
 
     def run():
         for k in range(K):
-            spmm(fwd, None, st.E[k], EMB, drop_p=st.drop_p, seed=st.seed, seed_dev=st.seed_dev, layer=k,
-                 compact=st.comp_f[k])
+            spmm(fwd, None, st.E[k], EMB, **st.dropout.args(k))
         for k in range(K - 1, -1, -1):
-            spmm(bwd, None, st.E[k + 1], EMB, slot=slot, gsum=gsum, drop_p=st.drop_p, seed=st.seed,
-                 seed_dev=st.seed_dev, layer=k, transposed=True, compact=st.comp_b[k])
+            spmm(bwd, None, st.E[k + 1], EMB, slot=slot, gsum=gsum, **st.dropout.args(k, transposed=True))
     return run
 
 
