@@ -432,6 +432,32 @@ int ngcf_softmax_loss(const float* u, const float* p, const float* n, int64_t ba
                       float* loss /*[1]*/, float* gu, float* gp, float* gn, void* workspace, size_t workspace_bytes,
                       void* stream);
 
+/* ---- XSimGCL (xsimgcl.py): layer noise, cosine InfoNCE over distinct ids, view-2 row gradients --------------------
+ * ngcf_perturb_rows, in place on rows r < n_rows of E ([n_rows, ld], 1 <= d <= NGCF_MAX_WIDTH, ld >= d):
+ *   u_c = (hash64(seed + *seed_dev, r, c, layer, 'NOIS').x >> 8) * 2^-24            (uniform on [0, 1), c < d)
+ *   E[r, c] += eps * sign(E[r, c]) * u_c / max(|u|, 1e-12)                         (sign(0) = 0)
+ * One warp per row.  eps >= 0, 0 <= layer <= NGCF_MAX_LAYERS, n_rows < 2^31; seed_dev optional, as for dropout. */
+int ngcf_perturb_rows(float* E, int64_t n_rows, int d, int64_t ld, float eps, uint64_t seed, const uint64_t* seed_dev,
+                      int layer, void* stream);
+/* ngcf_infonce: x1, x2 [batch, D] fp32, ids [batch].  Row i is valid iff ids[i] occurs in no earlier row (torch.unique
+ * semantics at a fixed shape); U = the number of valid rows, found on the device.  With z = x / max(|x|, 1e-12) per row:
+ *   loss[0] = (1/U) sum_{valid i} [ logsumexp_{valid j} (z1_i . z2_j / temperature) - z1_i . z2_i / temperature ]
+ * and, when g1 / g2 are given, its gradients with respect to x1 and x2 (zero on the rows that are not valid).  The
+ * products run on the softmax loss's tensor-core path; no atomics: two calls give the same bits.  1 <= batch <= 4096,
+ * 1 <= D <= 1152, temperature > 0.  workspace: ngcf_infonce_workspace bytes (a short one: NGCF_ERR_WORKSPACE).
+ * Allocates nothing, never synchronises (capturable). */
+int ngcf_infonce_workspace(int64_t batch, int D, size_t* bytes_host);
+int ngcf_infonce(const float* x1, const float* x2, int64_t batch, int D, const int64_t* ids, float temperature,
+                 float* loss /*[1]*/, float* g1, float* g2, void* workspace, size_t workspace_bytes, void* stream);
+/* ngcf_rowgrad_add: for each of the n_sets (<= 2) row sets (rows rows_host[j][b] + offsets_host[j], gradient rows
+ * g_host[j] [batch_host[j], d]):  dst[t, :] += g_host[j][b, :]  with t = slot[row] (a slot map that ngcf_rowgrad_scatter
+ * built over these rows), or t = row when slot is NULL (dst a dense [N, ld_dst] matrix).  Rows sharing a destination
+ * are added with atomics, in no fixed order: the result is exact when at most one of them is non-zero, as with
+ * ngcf_infonce's gradients.  1 <= d <= NGCF_MAX_WIDTH, ld_dst >= d. */
+int ngcf_rowgrad_add(const int64_t* const* rows_host, const int64_t* offsets_host, const float* const* g_host,
+                     const int64_t* batch_host, int n_sets, int d, const int32_t* slot, float* dst, int64_t ld_dst,
+                     void* stream);
+
 /* ---- Laplacian builder on the device: matrix.py:41-62 restricted to the non-zeros (SURVEY.md section 8(f) #2) ----------
  * From n_pairs DISTINCT (user, item, rating != 0) pairs: deg[N] = number of non-zeros per row of A = [[0,R],[R^T,0]]
  * (matrix.py:55), then the 2*n_pairs entries of L = D^-1/2 A D^-1/2 (matrix.py:56-62): entry e -> (user, n_user+item),

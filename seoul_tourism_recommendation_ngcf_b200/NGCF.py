@@ -390,12 +390,12 @@ class _TableModel(nn.Module):
                                                 self._winner.data_ptr(), _lib.current_stream()), "feature_mix")
         self._mix_count += 1
 
-    def _draw_seed(self, st: _Ctx, mess_dropout: bool = False):
+    def _draw_seed(self, st: _Ctx, mess_dropout: bool = False, noise: bool = False):
         """The forward's RNG key from torch's CPU generator (reproducible under torch.manual_seed), drawn only when a
-        device-RNG stream is live and only after the rng="reference" mask draws, whose RNG stream it must not shift.
-        The hard-negative draws take the same key: with dropout on, a forward with HardNegatives and one without
-        draw the same key from the generator and so the same dropout masks."""
-        need = st.drop_p > 0 or mess_dropout or st.hneg is not None
+        device-RNG stream is live (dropout, hard negatives, XSimGCL's layer noise) and only after the rng="reference"
+        mask draws, whose RNG stream it must not shift.  The hard-negative draws take the same key: with dropout on, a
+        forward with HardNegatives and one without draw the same key from the generator and so the same dropout masks."""
+        need = st.drop_p > 0 or mess_dropout or noise or st.hneg is not None
         if not need:
             st.seed = 0
         elif self.rng == "reference":

@@ -85,6 +85,11 @@ SIGNATURES = {
     "ngcf_rowgrad_expand": [_vp, _i64, _vp, _i64, C.c_int, _f32, _vp, _i64, _vp],
     "ngcf_softmax_loss_workspace": [_i64, C.c_int, C.c_int, C.POINTER(_sz)],
     "ngcf_softmax_loss": [_vp, _vp, _vp, _i64, C.c_int, _vp, _vp, _f32, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _sz, _vp],
+    "ngcf_perturb_rows": [_vp, _i64, C.c_int, _i64, _f32, _u64, _vp, C.c_int, _vp],
+    "ngcf_infonce_workspace": [_i64, C.c_int, C.POINTER(_sz)],
+    "ngcf_infonce": [_vp, _vp, _i64, C.c_int, _vp, _f32, _vp, _vp, _vp, _vp, _sz, _vp],
+    "ngcf_rowgrad_add": [C.POINTER(_vp), C.POINTER(_i64), C.POINTER(_vp), C.POINTER(_i64), C.c_int, C.c_int, _vp, _vp,
+                         _i64, _vp],
     "ngcf_laplacian_entries": [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp],
     "ngcf_plgraph_entries": [_i64, _i64, _i64, C.c_double, _u64, _i64, _i64, _vp, _vp, _i64, _vp],
     "ngcf_build_tiles": [_vp, _i64, C.c_int, C.c_int, _vp, _vp, _i64, _vp, _vp],

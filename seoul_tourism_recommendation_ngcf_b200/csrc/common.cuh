@@ -137,6 +137,7 @@ __device__ __forceinline__ uint2 ngcf_hash64(uint64_t seed, uint32_t a, uint32_t
 }
 #define NGCF_STREAM_NODE 0x4e4f4445u   // 'NODE'
 #define NGCF_STREAM_MESS 0x4d455353u   // 'MESS'
+#define NGCF_STREAM_NOISE 0x4e4f4953u  // 'NOIS': XSimGCL's layer noise (ngcf_perturb_rows)
 __device__ __forceinline__ uint32_t ngcf_threshold16(float p) { return (uint32_t)(p * 65536.0f); }   // keep iff u16 >= it
 
 // Per-step randomness: `seed` is a host value baked into the launch, `seed_dev` an optional device counter

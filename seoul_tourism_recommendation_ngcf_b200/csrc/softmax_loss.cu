@@ -17,8 +17,11 @@
 //   4. images of G, G^T, C^T and U^T, then gU = G·C and [gP; gN] = G^T·U, the same main loop, tiled over D in
 //      128-column blocks; the epilogue adds (2 wd / bs) x and stores each output row once.
 // Forward only (no gradient buffers): steps 1-3 without G.
+// softmax_run is shared with the cosine InfoNCE of xsimgcl.cu, which adds a validity mask (rows and columns outside it
+// take no part: no loss term, masked as a column, zero gradient) and divides by the number of valid rows.
 #include <math.h>
 
+#include "softmax_core.cuh"
 #include "tc_gemm.cuh"
 
 namespace {
@@ -40,6 +43,7 @@ struct LossGemmArgs {
     float inv_tau;
     const int64_t* pos_ids;    // NULL: no masking
     const int64_t* neg_ids;
+    const uint8_t* valid;      // NULL: every column < B takes part
     float* S;                  // [B][ld]
     float2* part;              // [B][n_b_tiles]: (max, sum of exp) of the row's unmasked logits in the tile
     int D;
@@ -108,6 +112,7 @@ __global__ void __launch_bounds__(ST_THREADS, 1) softmax_gemm_kernel(LossGemmArg
                         const int q = q0 + jj;
                         bool masked = q >= a.B;
                         if (!masked && a.pos_ids && (neg || q != r)) masked = ids[q] == my_id;
+                        if (!masked && a.valid) masked = !a.valid[q];
                         v[jj] = masked ? -INFINITY : v[jj] * a.inv_tau;
                         cm = fmaxf(cm, v[jj]);
                     }
@@ -153,15 +158,24 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
     return s;
 }
 
-// one block per row i: LSE_i from the per-tile partials (in tile order), the row's loss term, and (kGrad) G in place of S
+// one block per row i: LSE_i from the per-tile partials (in tile order), the row's loss term, and (kGrad) G in place of S;
+// a row outside `valid` has no loss term and a zero row of G
 template <bool kGrad>
 __global__ void __launch_bounds__(SL_ROW_THREADS) softmax_row_kernel(float* __restrict__ S, const float2* __restrict__ part,
                                                                      int n_tiles, int ld, const float* __restrict__ u,
                                                                      const float* __restrict__ p,
                                                                      const float* __restrict__ n, int D, float wd,
-                                                                     float g_scale, double* __restrict__ row_loss) {
+                                                                     float g_scale, const uint8_t* __restrict__ valid,
+                                                                     double* __restrict__ row_loss) {
     __shared__ float red[SL_ROW_THREADS / 32];
     const int64_t i = blockIdx.x;
+    float* srow = S + i * ld;
+    if (valid && !valid[i]) {
+        if (threadIdx.x == 0) row_loss[i] = 0.0;
+        if (kGrad)
+            for (int j = threadIdx.x * 4; j < ld; j += SL_ROW_THREADS * 4) st_f4(srow + j, make_float4(0.f, 0.f, 0.f, 0.f));
+        return;
+    }
     float m = -INFINITY;
     for (int t = 0; t < n_tiles; ++t) m = fmaxf(m, part[i * n_tiles + t].x);
     float sum = 0.f;
@@ -171,7 +185,6 @@ __global__ void __launch_bounds__(SL_ROW_THREADS) softmax_row_kernel(float* __re
     }
     // LSE = m + lsum, kept apart: at |s| ~ 1e4 an fp32 LSE would round by 1e-3, and that error would enter every P
     const float lsum = logf(sum);                                         // the row's own positive keeps sum >= 1
-    float* srow = S + i * ld;
     const float s_ii = srow[i];
     float su = 0.f, sp = 0.f, sn = 0.f;
     for (int c = threadIdx.x; c < D; c += SL_ROW_THREADS) {
@@ -197,19 +210,38 @@ __global__ void __launch_bounds__(SL_ROW_THREADS) softmax_row_kernel(float* __re
     }
 }
 
-// loss = sum_i row_loss[i] / bs: strided partial sums and a tree, both in a fixed order, in double
-__global__ void __launch_bounds__(SL_ROW_THREADS) softmax_sum_kernel(const double* __restrict__ row_loss, int64_t B,
-                                                                     double bs, float* __restrict__ loss) {
-    __shared__ double red[SL_ROW_THREADS];
-    double s = 0.0;
-    for (int64_t i = threadIdx.x; i < B; i += SL_ROW_THREADS) s += row_loss[i];
-    red[threadIdx.x] = s;
+// fixed-order sum of v over the block (strided partials, then a tree), in double; thread 0 gets it
+__device__ __forceinline__ double block_sum_fixed(double v, double* red) {
+    red[threadIdx.x] = v;
     __syncthreads();
     for (int w = SL_ROW_THREADS / 2; w > 0; w >>= 1) {
         if (threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
         __syncthreads();
     }
-    if (threadIdx.x == 0) *loss = (float)(red[0] / bs);
+    return red[0];
+}
+
+// loss = sum_i row_loss[i] / bs, in a fixed order in double.  With `valid`, bs = the number of valid rows, and 1 / bs
+// goes to *inv_count as well.
+__global__ void __launch_bounds__(SL_ROW_THREADS) softmax_sum_kernel(const double* __restrict__ row_loss, int64_t B,
+                                                                     double bs, const uint8_t* __restrict__ valid,
+                                                                     float* __restrict__ loss,
+                                                                     float* __restrict__ inv_count) {
+    __shared__ double red[SL_ROW_THREADS];
+    double s = 0.0, c = 0.0;
+    for (int64_t i = threadIdx.x; i < B; i += SL_ROW_THREADS) {
+        s += row_loss[i];
+        if (valid) c += valid[i];
+    }
+    const double total = block_sum_fixed(s, red);
+    if (valid) {
+        __syncthreads();
+        bs = block_sum_fixed(c, red);
+    }
+    if (threadIdx.x == 0) {
+        *loss = (float)(total / bs);
+        if (valid) *inv_count = (float)(1.0 / bs);
+    }
 }
 
 // workspace layout; every region starts on a 1024-byte boundary (the operand images are read by bulk copies into
@@ -262,6 +294,8 @@ int launch_gemm(LossGemmArgs a, int a_tiles, cudaStream_t st) {
 
 }  // namespace
 
+size_t softmax_run_bytes(int64_t batch, bool has_n, int D) { return loss_layout(batch, has_n, D).total - 1024; }
+
 extern "C" int ngcf_softmax_loss_workspace(int64_t batch, int n_cols, int D, size_t* bytes_host) {
     NGCF_REQUIRE(bytes_host, "softmax_loss_workspace: null pointer");
     NGCF_REQUIRE(batch >= 1 && batch <= SL_MAX_B, "softmax_loss_workspace: batch %lld not in [1, %d]", (long long)batch,
@@ -283,7 +317,6 @@ extern "C" int ngcf_softmax_loss(const float* u, const float* p, const float* n,
     NGCF_REQUIRE(weight_decay >= 0.f && isfinite(weight_decay), "softmax_loss: weight_decay %g is not >= 0", weight_decay);
     NGCF_REQUIRE(batch_size > 0.f && isfinite(batch_size), "softmax_loss: batch_size %g is not > 0", batch_size);
     NGCF_REQUIRE(!gn || n, "softmax_loss: gn given without n");
-    const bool grad = gu != nullptr;
     NGCF_REQUIRE((gu && gp && (gn || !n)) || (!gu && !gp && !gn),
                  "softmax_loss: give every gradient buffer (gu, gp, and gn with n) or none");
     NGCF_REQUIRE(pos_ids || !neg_ids, "softmax_loss: neg_ids given without pos_ids");
@@ -295,8 +328,20 @@ extern "C" int ngcf_softmax_loss(const float* u, const float* p, const float* n,
                        L.total);
         return NGCF_ERR_WORKSPACE;
     }
-    cudaStream_t st = as_stream(stream);
-    uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~(uintptr_t)1023);
+    SoftmaxRun r{};
+    r.u = u; r.p = p; r.n = n; r.batch = batch; r.D = D; r.pos_ids = pos_ids; r.neg_ids = neg_ids;
+    r.temperature = temperature; r.weight_decay = weight_decay; r.batch_size = batch_size;
+    r.loss = loss; r.gu = gu; r.gp = gp; r.gn = gn;
+    return softmax_run(r, reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~(uintptr_t)1023),
+                       as_stream(stream));
+}
+
+int softmax_run(const SoftmaxRun& r, uint8_t* ws, cudaStream_t st) {
+    const float *u = r.u, *p = r.p, *n = r.n;
+    const int64_t batch = r.batch;
+    const int D = r.D;
+    const bool grad = r.gu != nullptr;
+    const LossLayout L = loss_layout(batch, n != nullptr, D);
     float* S = reinterpret_cast<float*>(ws + L.S);
     float2* part = reinterpret_cast<float2*>(ws + L.part);
     double* row_loss = reinterpret_cast<double*>(ws + L.row_loss);
@@ -310,20 +355,24 @@ extern "C" int ngcf_softmax_loss(const float* u, const float* p, const float* n,
     LossGemmArgs a{};
     a.B = batch; a.Bp = L.Bp; a.D = D;
     a.Aimg = ws + L.U; a.Bimg = ws + L.C; a.KB = L.KBd; a.n_b_tiles = L.n_col_tiles;
-    a.ld = L.n_cols_pad; a.inv_tau = 1.f / temperature; a.pos_ids = pos_ids; a.neg_ids = neg_ids; a.S = S; a.part = part;
+    a.ld = L.n_cols_pad; a.inv_tau = 1.f / r.temperature; a.pos_ids = r.pos_ids; a.neg_ids = r.neg_ids;
+    a.valid = r.valid; a.S = S; a.part = part;
     rc = launch_gemm<SL_LOGITS>(a, bt, st);
     if (rc != NGCF_OK) return rc;
 
     // 3. LSE, the row terms and G; the loss
-    const float g_scale = 1.f / (temperature * batch_size);
+    const float g_scale = 1.f / (r.temperature * r.batch_size);
     if (grad)
         softmax_row_kernel<true><<<(unsigned)batch, SL_ROW_THREADS, 0, st>>>(S, part, L.n_col_tiles, L.n_cols_pad, u, p, n,
-                                                                             D, weight_decay, g_scale, row_loss);
+                                                                             D, r.weight_decay, g_scale, r.valid,
+                                                                             row_loss);
     else
         softmax_row_kernel<false><<<(unsigned)batch, SL_ROW_THREADS, 0, st>>>(S, part, L.n_col_tiles, L.n_cols_pad, u, p,
-                                                                              n, D, weight_decay, g_scale, row_loss);
+                                                                              n, D, r.weight_decay, g_scale, r.valid,
+                                                                              row_loss);
     NGCF_LAUNCH_OK("softmax_row_kernel");
-    softmax_sum_kernel<<<1, SL_ROW_THREADS, 0, st>>>(row_loss, batch, (double)batch_size, loss);
+    softmax_sum_kernel<<<1, SL_ROW_THREADS, 0, st>>>(row_loss, batch, (double)r.batch_size, r.valid, r.loss,
+                                                     r.inv_count);
     NGCF_LAUNCH_OK("softmax_sum_kernel");
     if (!grad) return NGCF_OK;
 
@@ -334,13 +383,13 @@ extern "C" int ngcf_softmax_loss(const float* u, const float* p, const float* n,
     if (rc == NGCF_OK && n) rc = gemm_pack<true>(true, n, D, (int)batch, D, KBb, KBb, KBc, ws + L.CT, st);
     if (rc == NGCF_OK) rc = gemm_pack<true>(true, u, D, (int)batch, D, KBb, 0, KBb, ws + L.UT, st);
     if (rc != NGCF_OK) return rc;
-    a.reg = 2.f * weight_decay / batch_size;
+    a.reg = 2.f * r.weight_decay / r.batch_size;
     a.n_b_tiles = L.Dt;
     a.Aimg = ws + L.G; a.Bimg = ws + L.CT; a.KB = KBc;
-    a.x0 = u; a.out0 = gu;
+    a.x0 = u; a.out0 = r.gu;
     rc = launch_gemm<SL_GRAD_U>(a, bt, st);
     if (rc != NGCF_OK) return rc;
     a.Aimg = ws + L.GT; a.Bimg = ws + L.UT; a.KB = KBb;
-    a.x0 = p; a.x1 = n; a.out0 = gp; a.out1 = gn;
+    a.x0 = p; a.x1 = n; a.out0 = r.gp; a.out1 = r.gn;
     return launch_gemm<SL_GRAD_C>(a, L.n_col_tiles, st);
 }

@@ -110,6 +110,8 @@ class Experiment(nn.Module):
                         loss = self.criterion(u, p, n, pos_item.to(dev, torch.int64), neg_ids)
                     else:
                         loss = self.criterion(u, p, n)
+                    if getattr(self.model, "cl_loss", None) is not None:    # XSimGCL's contrastive term
+                        loss = loss + self.model.cl_loss
                     loss.backward()
                     self.optimizer.step()
                 total_loss += loss.detach()

@@ -63,6 +63,8 @@ class GraphedStep:
             loss = self.criterion(u, p, n, rows[1], rows[2] if len(rows) > 2 else None)
         else:
             loss = self.criterion(u, p, n)
+        if getattr(m, "cl_loss", None) is not None:                   # XSimGCL's contrastive term
+            loss = loss + m.cl_loss
         loss.backward()
         if self.optimizer is not None and with_optimizer:
             self.optimizer.step()         # (a replay overwrites every gradient buffer, so nothing needs zeroing)
